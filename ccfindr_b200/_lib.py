@@ -12,6 +12,7 @@ c_ip = C.POINTER(C.c_int)
 c_i32p = C.POINTER(C.c_int32)
 c_i64p = C.POINTER(C.c_int64)
 c_fp = C.POINTER(C.c_float)
+c_u8p = C.POINTER(C.c_uint8)
 
 
 class VbnmfCfg(C.Structure):
@@ -36,6 +37,8 @@ SIGNATURES = {
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "vbnmf_create_from_mtx": (C.c_int, [C.POINTER(C.c_void_p), C.c_char_p, C.c_int, c_i64p]),
     "vbnmf_get_csc": (C.c_int, [C.c_void_p, c_i64p, c_i32p, c_dp]),
+    "vbnmf_qc_stats": (C.c_int, [C.c_void_p, c_dp, c_dp, c_dp, c_i64p, c_i64p]),
+    "vbnmf_create_subset": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, c_u8p, c_u8p, c_dp]),
     "vbnmf_destroy": (None, [C.c_void_p]),
     "vbnmf_last_error": (C.c_char_p, [C.c_void_p]),
     "vbnmf_set_precision": (C.c_int, [C.c_void_p, C.c_int]),

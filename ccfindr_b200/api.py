@@ -12,6 +12,11 @@ ships as source in r-shim/).  What runs where:
                                            nmf_updateR + likelihood on the GPU (Engine.ml_run)
     cluster_id()     R/utils.R:903-909     first-maximum argmax per cell (GPU: Engine.cluster_id)
     optimal_rank()   R/utils2.R:59-95      host post-processing of measure (smoothing spline)
+    filter_cells(), filter_genes(), calc_vmr(), normalize_count()
+                     R/utils.R:78-95,134-218,318-327  thresholds, marker matching and the median
+                                           here; the per-cell / per-gene sums and the subset /
+                                           scale of the matrix on the GPU (Engine.qc_stats,
+                                           Engine.subset)
 
 There is no CPU fallback: every factorization needs libvbnmf.so and a CUDA device.
 """
@@ -61,6 +66,103 @@ def remove_zeros(object):
     out = scNMFSet(mat[gi][:, ci], rowData=[object.rowData[i] for i in gi],
                    colData=[object.colData[j] for j in ci])
     return out
+
+
+# ---- cell / gene QC (R/utils.R:78-95,134-218,318-327): statistics and subsetting on the GPU -------
+def vmr_from_sums(gene_sum, gene_sumsq, m):
+    """Variance-to-mean ratio per gene over all m cells, zeros included: var is R's var
+    (denominator m - 1), mean = S1 / m; a gene with mean 0 gets NaN (R's 0 / 0)."""
+    s1 = np.asarray(gene_sum, dtype=np.float64)
+    s2 = np.asarray(gene_sumsq, dtype=np.float64)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        mean = s1 / m
+        var = (s2 - s1 * s1 / m) / (m - 1)
+        return np.where(mean == 0, np.nan, var / mean)
+
+
+def cell_mask(cell_sum, umi_min=0, umi_max=np.inf):
+    """filter_cells: cells with umi_min <= total count <= umi_max."""
+    cell_sum = np.asarray(cell_sum)
+    return (cell_sum >= umi_min) & (cell_sum <= umi_max)
+
+
+def marker_mask(rowData, markers):
+    """Genes of which some field of rowData (the id or symbol of genes.tsv) is in markers."""
+    if markers is None:
+        return np.zeros(len(rowData), dtype=bool)
+    mset = {markers} if isinstance(markers, str) else set(markers)
+    return np.array([any(f in mset for f in (g if isinstance(g, (tuple, list)) else (g,)))
+                     for g in rowData], dtype=bool)
+
+
+def gene_mask(vmr, gene_cells, rowData, markers=None, vmr_min=0, min_cells_expressed=0,
+              max_cells_expressed=np.inf):
+    """filter_genes: vmr > vmr_min (NaN fails) with min <= cells expressed <= max, or a marker."""
+    gene_cells = np.asarray(gene_cells)
+    keep = (np.asarray(vmr) > vmr_min) & (gene_cells >= min_cells_expressed) \
+        & (gene_cells <= max_cells_expressed)
+    return keep | marker_mask(rowData, markers)
+
+
+def normalize_scale(cell_sum):
+    """normalize_count: the factor median(cell_sum) / cell_sum[j] of every cell, in fp64 (the
+    median of an even number of cells is the mean of the two middle values, as R's)."""
+    cell_sum = np.asarray(cell_sum, dtype=np.float64)
+    if (cell_sum == 0).any():
+        raise ValueError("Input matrix contains empty columns")
+    return np.median(cell_sum) / cell_sum
+
+
+def _qc_subset(object, device, select):
+    """Statistics of object.counts on the GPU, select(stats) -> (keep_rows, keep_cols, col_scale),
+    the subset built on the GPU and returned as a new scNMFSet (counts, rowData, colData)."""
+    with Engine(object.counts, device=device) as eng:
+        rows, cols, scale = select(eng.qc_stats())
+        with eng.subset(rows, cols, scale) as sub:
+            mat = sub.csc()
+    return scNMFSet(mat, rowData=[g for g, k in zip(object.rowData, rows) if k],
+                    colData=[c for c, k in zip(object.colData, cols) if k])
+
+
+def calc_vmr(object, device=0):
+    """calc_vmr (R/utils.R:134-218): variance-to-mean ratio of every gene over all cells (sums on
+    the GPU).  NaN for a gene without counts."""
+    with Engine(object.counts, device=device) as eng:
+        st = eng.qc_stats()
+    return vmr_from_sums(st["gene_sum"], st["gene_sumsq"], object.ncol())
+
+
+def filter_cells(object, umi_min=0, umi_max=np.inf, device=0):
+    """filter_cells (R/utils.R:78-95): a new scNMFSet with the cells whose total count lies in
+    [umi_min, umi_max].  The defaults keep every cell (they are not the reference's defaults,
+    which are not restated here).  Totals and the subset are computed on the GPU."""
+    def select(st):
+        return np.ones(object.nrow(), dtype=bool), cell_mask(st["cell_sum"], umi_min, umi_max), None
+    return _qc_subset(object, device, select)
+
+
+def filter_genes(object, markers=None, vmr_min=0, min_cells_expressed=0,
+                 max_cells_expressed=np.inf, device=0):
+    """filter_genes (R/utils.R:134-218, without rescue.genes): a new scNMFSet with the genes whose
+    VMR exceeds vmr_min and which have a non-zero count in between min_cells_expressed and
+    max_cells_expressed cells, plus every gene with a field of its rowData in `markers`.
+    Statistics and the subset are computed on the GPU."""
+    def select(st):
+        vmr = vmr_from_sums(st["gene_sum"], st["gene_sumsq"], object.ncol())
+        rows = gene_mask(vmr, st["gene_cells"], object.rowData, markers, vmr_min,
+                         min_cells_expressed, max_cells_expressed)
+        return rows, np.ones(object.ncol(), dtype=bool), None
+    return _qc_subset(object, device, select)
+
+
+def normalize_count(object, device=0):
+    """normalize_count (R/utils.R:318-327): a new scNMFSet with every cell's counts scaled by
+    median(cell totals) / its total.  The factors are computed in fp64 on the host from totals
+    summed on the GPU; the scaled matrix is built on the GPU.  An empty cell raises ValueError."""
+    def select(st):
+        return (np.ones(object.nrow(), dtype=bool), np.ones(object.ncol(), dtype=bool),
+                normalize_scale(st["cell_sum"]))
+    return _qc_subset(object, device, select)
 
 
 def read_10x(dir, count="matrix.mtx", genes="genes.tsv", barcodes="barcodes.tsv",

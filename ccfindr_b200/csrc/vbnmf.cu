@@ -39,6 +39,7 @@
 #include "kernels_common.cuh"
 #include "svd_init.cuh"
 #include "mtx_ingest.cuh"
+#include "qc.cuh"
 #include "rp_ranks.h"
 #include "rp_table.h"
 
@@ -1339,6 +1340,26 @@ int init_svd2_t(H *h, int r, const double hyper[4], uint64_t seed, int64_t cell_
 
 }  // namespace
 
+// ---- cell / gene QC (qc.cuh) ---------------------------------------------------------------------
+namespace {
+
+// the kept entries of src into h's CSC (h->d_colptr already holds the new column pointers)
+template <typename OT>
+void launch_subset_compact(H *h, const H *src, const int32_t *d_cols, const int32_t *d_rowmap,
+                           const double *d_scale, OT *out_val, unsigned *d_bad) {
+    const int grid = h->num_sms * 8;
+    if (src->val_float)
+        vb::qc_subset_compact_kernel<float, OT><<<grid, vb::kBlock, 0, h->stream>>>(
+            h->m, d_cols, src->d_colptr, src->d_rowidx, (const float *)src->d_val, d_rowmap,
+            d_scale, h->d_colptr, h->d_rowidx, out_val, d_bad);
+    else
+        vb::qc_subset_compact_kernel<double, OT><<<grid, vb::kBlock, 0, h->stream>>>(
+            h->m, d_cols, src->d_colptr, src->d_rowidx, (const double *)src->d_val, d_rowmap,
+            d_scale, h->d_colptr, h->d_rowidx, out_val, d_bad);
+}
+
+}  // namespace
+
 extern "C" {
 
 const char *vbnmf_last_error(const vbnmf_handle *h) {
@@ -1662,6 +1683,158 @@ int vbnmf_get_csc(vbnmf_handle *h, int64_t *colptr, int32_t *rowidx, double *val
             CK(copy_sync(h, values, h->d_val, (size_t)h->nnz * 8, cudaMemcpyDeviceToHost));
         }
     }
+    return 0;
+}
+
+int vbnmf_qc_stats(vbnmf_handle *h, double *cell_sum, double *gene_sum, double *gene_sumsq,
+                   int64_t *gene_cells, int64_t *cell_genes) {
+    if (!h) return VBNMF_ERR_ARG;
+    if (h->nranks > 1)
+        return fail(h, VBNMF_ERR_STATE, "vbnmf_qc_stats: the handle holds one shard of the cells "
+                                        "(vbnmf_attach_comm); its gene statistics would be partial");
+    CK(cudaSetDevice(h->device));
+    const int64_t n = h->n, m = h->m;
+    if (cell_sum || gene_sum || gene_sumsq) {
+        double *d = nullptr;  // [cell_sum m | gene_sum n | gene_sumsq n]
+        CK(vmalloc(h, &d, (size_t)(m + 2 * n) * 8));
+        auto body = [&]() -> int {
+            CK(cudaMemsetAsync(d + m, 0, (size_t)2 * n * 8, h->stream));
+            const int grid = h->num_sms * 8;
+            if (h->val_float)
+                vb::qc_stats_kernel<float><<<grid, vb::kBlock, 0, h->stream>>>(
+                    m, h->d_colptr, h->d_rowidx, (const float *)h->d_val, d, d + m, d + m + n);
+            else
+                vb::qc_stats_kernel<double><<<grid, vb::kBlock, 0, h->stream>>>(
+                    m, h->d_colptr, h->d_rowidx, (const double *)h->d_val, d, d + m, d + m + n);
+            CK(cudaGetLastError());
+            if (cell_sum) CK(cudaMemcpyAsync(cell_sum, d, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+            if (gene_sum) CK(cudaMemcpyAsync(gene_sum, d + m, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+            if (gene_sumsq)
+                CK(cudaMemcpyAsync(gene_sumsq, d + m + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            return 0;
+        };
+        const int rc = body();
+        vfree(h->stream, d);
+        if (rc) return rc;
+    }
+    // entries with a non-zero value: the counts scan_matrix keeps on the device
+    static_assert(sizeof(unsigned long long) == sizeof(int64_t), "d_cnt is copied as int64");
+    if (gene_cells) CK(cudaMemcpyAsync(gene_cells, h->d_cnt, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (cell_genes) CK(cudaMemcpyAsync(cell_genes, h->d_cnt + n, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *keep_rows,
+                        const uint8_t *keep_cols, const double *col_scale) {
+    if (!out) return VBNMF_ERR_ARG;
+    *out = nullptr;
+    H *h = new H();
+    auto bail = [&](int rc) {
+        g_create_error = h->err;
+        vbnmf_destroy(h);
+        return rc;
+    };
+    StageTimer tm("vbnmf_create_subset(total)");
+    if (!src || !keep_rows || !keep_cols)
+        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: bad arguments"));
+    // the gene statistics and the empty-gene test of one shard are partial: refused, not guessed
+    if (src->nranks > 1)
+        return bail(fail(h, VBNMF_ERR_STATE, "vbnmf_create_subset: the source holds one shard of "
+                                             "the cells (vbnmf_attach_comm)"));
+    const int64_t n0 = src->n, m0 = src->m;
+    int64_t n = 0, m = 0;
+    for (int64_t i = 0; i < n0; i++) n += keep_rows[i] != 0;
+    for (int64_t j = 0; j < m0; j++) m += keep_cols[j] != 0;
+    if (n == 0 || m == 0)
+        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: no rows or no columns selected"));
+    h->n = n; h->m = m;
+    int rc = init_common(h, src->device);
+    if (rc) return bail(rc);
+    bool as_float = true;
+    auto body = [&]() -> int {
+        uint8_t *d_mask = nullptr;  // [rows n0 | columns m0]
+        double *d_scale = nullptr;
+        int32_t *d_rowmap = nullptr, *d_cols = nullptr, *d_nsel = nullptr;
+        int64_t *d_ptr = nullptr;
+        unsigned *d_bad = nullptr;
+        void *d_tmp = nullptr;
+        struct Free {
+            cudaStream_t s; void **p[8];
+            ~Free() { for (void **q : p) if (q) vfree(s, *q); }
+        } fr{h->stream, {(void **)&d_mask, (void **)&d_scale, (void **)&d_rowmap, (void **)&d_cols,
+                         (void **)&d_nsel, (void **)&d_ptr, (void **)&d_bad, &d_tmp}};
+        // src's arrays are read on this handle's stream: src's own work on them must be complete
+        CK(cudaStreamSynchronize(src->stream));
+        cudaStream_t s = h->stream;
+        CK(vmalloc(h, &d_mask, (size_t)(n0 + m0)));
+        CK(cudaMemcpyAsync(d_mask, keep_rows, (size_t)n0, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(d_mask + n0, keep_cols, (size_t)m0, cudaMemcpyHostToDevice, s));
+        if (col_scale) {
+            CK(vmalloc(h, &d_scale, (size_t)m0 * 8));
+            CK(cudaMemcpyAsync(d_scale, col_scale, (size_t)m0 * 8, cudaMemcpyHostToDevice, s));
+        }
+        CK(vmalloc(h, &d_rowmap, (size_t)n0 * 4));
+        CK(vmalloc(h, &d_cols, (size_t)m * 4));
+        CK(vmalloc(h, &d_nsel, 4));
+        CK(vmalloc(h, &d_ptr, (size_t)(m + 1) * 8));
+        cub::CountingInputIterator<int32_t> iota(0);
+        size_t tb1 = 0, tb2 = 0, tb3 = 0;
+        CK(cub::DeviceScan::ExclusiveSum(nullptr, tb1, d_rowmap, d_rowmap, n0, s));
+        CK(cub::DeviceSelect::Flagged(nullptr, tb2, iota, d_mask + n0, d_cols, d_nsel, m0, s));
+        CK(cub::DeviceScan::ExclusiveSum(nullptr, tb3, d_ptr, d_ptr, m + 1, s));
+        CK(vmalloc(h, &d_tmp, std::max(tb1, std::max(tb2, tb3))));
+        // kept rows renumbered in order (exclusive scan of the row mask), dropped rows -> -1
+        vb::qc_mask_kernel<<<cdiv(n0, vb::kBlock), vb::kBlock, 0, s>>>(n0, d_mask, d_rowmap);
+        CK(cub::DeviceScan::ExclusiveSum(d_tmp, tb1, d_rowmap, d_rowmap, n0, s));
+        vb::qc_rowmap_kernel<<<cdiv(n0, vb::kBlock), vb::kBlock, 0, s>>>(n0, d_mask, d_rowmap);
+        // kept columns in order; per kept column its kept entries; the scan gives the new colptr
+        CK(cub::DeviceSelect::Flagged(d_tmp, tb2, iota, d_mask + n0, d_cols, d_nsel, m0, s));
+        vb::qc_subset_count_kernel<<<h->num_sms * 8, vb::kBlock, 0, s>>>(
+            m, d_cols, src->d_colptr, src->d_rowidx, d_rowmap, d_ptr);
+        CK(cudaMemsetAsync(d_ptr + m, 0, 8, s));
+        CK(cub::DeviceScan::ExclusiveSum(d_tmp, tb3, d_ptr, d_ptr, m + 1, s));
+        int64_t nnz = 0;
+        CK(cudaMemcpyAsync(&nnz, d_ptr + m, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        if (nnz == 0) return fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: the selection holds no entries");
+        h->nnz = h->nnz_global = nnz;
+        // allocation order of the other create paths: the arena first, then the CSC arrays
+        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
+        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
+        CK(cudaMemcpyAsync(h->d_colptr, d_ptr, (size_t)(m + 1) * 8, cudaMemcpyDeviceToDevice, s));
+        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
+        CK(vmalloc(h, &d_bad, 4));
+        CK(cudaMemsetAsync(d_bad, 0, 4, s));
+        // values as fp32 when every kept (scaled) value is exact in fp32, else fp64 (vbnmf_create)
+        float *dv = nullptr;
+        CK(vmalloc(h, &dv, (size_t)nnz * 4));
+        h->d_val = dv;
+        launch_subset_compact<float>(h, src, d_cols, d_rowmap, d_scale, dv, d_bad);
+        unsigned bad = 0;
+        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        if (bad) {
+            vfree(s, dv);
+            h->d_val = nullptr;
+            double *dd = nullptr;
+            CK(vmalloc(h, &dd, (size_t)nnz * 8));
+            h->d_val = dd;
+            launch_subset_compact<double>(h, src, d_cols, d_rowmap, d_scale, dd, d_bad);
+            as_float = false;
+        }
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        return 0;
+    };
+    if ((rc = body())) return bail(rc);
+    h->val_float = as_float;
+    rc = as_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
+    if (rc) return bail(rc);
+    *out = h;
     return 0;
 }
 

@@ -108,6 +108,59 @@ class Engine:
                                         rowidx.ctypes.data_as(_lib.c_i32p), _dp(values)))
         return sp.csc_matrix((values, rowidx, colptr), shape=(self.n, self.m))
 
+    # -- cell / gene QC ------------------------------------------------------------------------
+    def qc_stats(self):
+        """Per-cell and per-gene statistics of the resident matrix, computed on the device (the
+        inputs of filter_cells / filter_genes / calc_vmr, R/utils.R:78-95,134-218): cell_sum (m),
+        gene_sum and gene_sumsq (n) as fp64 sums of x and x^2, gene_cells (n) and cell_genes (m)
+        as numbers of entries with a non-zero value.  Exact for integer counts."""
+        out = dict(cell_sum=np.zeros(self.m), gene_sum=np.zeros(self.n), gene_sumsq=np.zeros(self.n),
+                   gene_cells=np.zeros(self.n, dtype=np.int64),
+                   cell_genes=np.zeros(self.m, dtype=np.int64))
+        self._ck(self.lib.vbnmf_qc_stats(self.handle, _dp(out["cell_sum"]), _dp(out["gene_sum"]),
+                                         _dp(out["gene_sumsq"]),
+                                         out["gene_cells"].ctypes.data_as(_lib.c_i64p),
+                                         out["cell_genes"].ctypes.data_as(_lib.c_i64p)))
+        return out
+
+    def subset(self, keep_rows, keep_cols, col_scale=None):
+        """A new Engine on the same device holding the genes where keep_rows is true and the cells
+        where keep_cols is true (order kept), each entry of cell j multiplied by col_scale[j] when
+        given (normalize_count, R/utils.R:318-327).  Built from this engine's device arrays: only
+        the masks and the scales cross the bus.  This engine is left as it was."""
+        keep_rows = np.asarray(keep_rows)
+        keep_cols = np.asarray(keep_cols)
+        if keep_rows.dtype != np.bool_ or keep_cols.dtype != np.bool_:
+            raise ValueError("keep_rows and keep_cols must be boolean arrays")
+        if keep_rows.shape != (self.n,):
+            raise ValueError("keep_rows must have one entry per gene (%d)" % self.n)
+        if keep_cols.shape != (self.m,):
+            raise ValueError("keep_cols must have one entry per cell (%d)" % self.m)
+        scale = None
+        if col_scale is not None:
+            scale = np.ascontiguousarray(col_scale, dtype=np.float64)
+            if scale.shape != (self.m,):
+                raise ValueError("col_scale must have one entry per cell (%d)" % self.m)
+            if not np.isfinite(scale).all():
+                raise ValueError("col_scale must be finite")
+        rows = np.ascontiguousarray(keep_rows, dtype=np.uint8)
+        cols = np.ascontiguousarray(keep_cols, dtype=np.uint8)
+        out = Engine.__new__(Engine)
+        out.lib = self.lib
+        out.handle = C.c_void_p()
+        out._keep = None
+        rc = self.lib.vbnmf_create_subset(C.byref(out.handle), self.handle,
+                                          rows.ctypes.data_as(_lib.c_u8p),
+                                          cols.ctypes.data_as(_lib.c_u8p), _dp(scale))
+        if rc != 0:
+            msg = self.lib.vbnmf_last_error(None)
+            out.handle = C.c_void_p()
+            raise _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
+        info = out.info()
+        out.n, out.m, out.nnz = int(info["n"]), int(info["m"]), int(info["nnz"])
+        out.r = 0
+        return out
+
     # -- lifetime ------------------------------------------------------------------------------
     def close(self):
         if getattr(self, "handle", None) and self.handle.value:

@@ -16,6 +16,11 @@
  *   nmf_updateR() + likelihood() loop, R/factorize.R:189-212           mlnmf_run, mlnmf_run2 (both criteria)
  *   vb_init(): 'random', 'svd2', R/bayesian.R:111-115,150-159          vbnmf_init_random, vbnmf_init_svd2
  *   read_10x(): readMM + as(., 'dgCMatrix'), R/utils.R:34               vbnmf_create_from_mtx
+ *   filter_cells(): colSums(counts), R/utils.R:78-95                   vbnmf_qc_stats +
+ *                                                                      vbnmf_create_subset
+ *   filter_genes(): rowSums, VMR, cells expressed, R/utils.R:134-218   vbnmf_qc_stats +
+ *                                                                      vbnmf_create_subset
+ *   normalize_count(): counts scaled per cell, R/utils.R:318-327       vbnmf_create_subset (col_scale)
  *   Rmpi task farm over restarts, R/bayesian.R:263                     one handle per process/GPU;
  *                                                                      cells sharded: vbnmf_attach_comm
  *
@@ -100,6 +105,25 @@ VBNMF_API int vbnmf_create_from_mtx(vbnmf_handle **out, const char *path, int de
 /* The CSC arrays of a handle copied to the host: colptr (m+1), rowidx (nnz), values (nnz); any may
  * be NULL.  (After vbnmf_create_from_mtx the front end needs them for the row/column filters.) */
 VBNMF_API int vbnmf_get_csc(vbnmf_handle *h, int64_t *colptr, int32_t *rowidx, double *values);
+
+/* QC statistics of the matrix a handle holds (filter_cells / filter_genes / calc_vmr,
+ * R/utils.R:78-95,134-218).  Any pointer may be NULL.  cell_sum (m), gene_sum, gene_sumsq (n):
+ * fp64 sums of x and x^2; gene_cells (n), cell_genes (m): entries with a non-zero value.
+ * The sums are exact for integer counts (any summation order gives the same bits).  A handle with
+ * a communicator of more than one rank attached is refused (VBNMF_ERR_STATE). */
+VBNMF_API int vbnmf_qc_stats(vbnmf_handle *h, double *cell_sum, double *gene_sum,
+                             double *gene_sumsq, int64_t *gene_cells, int64_t *cell_genes);
+
+/* A new handle on src's device holding the rows i with keep_rows[i] != 0 and the columns j with
+ * keep_cols[j] != 0 of src's matrix (order kept, rows renumbered), each kept entry of column j
+ * multiplied by col_scale[j] when col_scale != NULL (normalize_count, R/utils.R:318-327).
+ * Built from src's device arrays; src is not modified and stays valid.  keep_rows has src's n
+ * entries, keep_cols and col_scale its m.  Stored entries are kept as stored (explicit zeros
+ * included); the values are held as by vbnmf_create (fp32 when every one is exact in fp32), so
+ * the handle equals vbnmf_create on the same CSC.  No rows, columns or entries selected:
+ * VBNMF_ERR_ARG; src with more than one rank attached: VBNMF_ERR_STATE. */
+VBNMF_API int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *keep_rows,
+                                  const uint8_t *keep_cols, const double *col_scale);
 
 VBNMF_API void vbnmf_destroy(vbnmf_handle *h);
 VBNMF_API const char *vbnmf_last_error(const vbnmf_handle *h); /* h may be NULL: error of the last create */
