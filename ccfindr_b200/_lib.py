@@ -39,6 +39,7 @@ SIGNATURES = {
     "vbnmf_get_csc": (C.c_int, [C.c_void_p, c_i64p, c_i32p, c_dp]),
     "vbnmf_qc_stats": (C.c_int, [C.c_void_p, c_dp, c_dp, c_dp, c_i64p, c_i64p]),
     "vbnmf_create_subset": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, c_u8p, c_u8p, c_dp]),
+    "vbnmf_create_shuffled": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_uint64]),
     "vbnmf_destroy": (None, [C.c_void_p]),
     "vbnmf_last_error": (C.c_char_p, [C.c_void_p]),
     "vbnmf_set_precision": (C.c_int, [C.c_void_p, C.c_int]),

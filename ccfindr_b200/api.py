@@ -9,7 +9,9 @@ ships as source in r-shim/).  What runs where:
                                            (src/vbnmf_update.cpp) and hyper_update (:2-53): in
                                            libvbnmf.so on the GPU (Engine.run)
     factorize()      R/factorize.R:139-276 loops and measures here; the it-loop (:189-212) with
-                                           nmf_updateR + likelihood on the GPU (Engine.ml_run)
+                                           nmf_updateR + likelihood on the GPU (Engine.ml_run);
+                                           with device_shuffle=True the null matrices of
+                                           randomize (:172-173) on the GPU too (Engine.shuffle)
     cluster_id()     R/utils.R:903-909     first-maximum argmax per cell (GPU: Engine.cluster_id)
     optimal_rank()   R/utils2.R:59-95      host post-processing of measure (smoothing spline)
     filter_cells(), filter_genes(), calc_vmr(), normalize_count()
@@ -584,13 +586,23 @@ def _vb_iterate(eng, irun, mat, ranks, ga, gb, initializer, Itmax, hyper_update,
 
 def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, progress_bar=True,
               Itmax=10000, ncnn_step=40, criterion="likelihood", linkage="average", Tol=1e-5,
-              store_connectivity=False, seed=1, device=0):
+              store_connectivity=False, seed=1, device=0, device_shuffle=False):
     """Maximum likelihood factorization (R/factorize.R:139-276); the it-loop (:189-212) runs on the
     GPU with either stopping criterion.  The consensus measures never form the m(m-1)/2
     connectivity vector of the reference (:51-78): dispersion and the cophenetic correlation are
-    computed from the groups of cells that share their labels over the runs."""
+    computed from the groups of cells that share their labels over the runs.
+
+    `randomize=True` fits every rank on `nsmpl` null matrices, each column of the counts shuffled
+    over the genes (:172-173).  By default the shuffle is a NumPy permutation of the dense column
+    (Philox stream keyed by `seed`) and every null matrix is uploaded anew.
+    `device_shuffle=True` (needs `randomize=True`): the counts are uploaded once and each null
+    matrix is drawn on the GPU from the resident copy (Engine.shuffle; no dense matrix, no upload):
+    sample `ismpl` of rank `r` is Engine.shuffle(seed * 100003 + 1000 * r + 37 * ismpl), closed
+    after its `nrun` restarts.  Same distribution, different draw than the default."""
     if criterion not in ("likelihood", "connectivity"):
         raise ValueError("Unknown stopping criterion.")        # :212
+    if device_shuffle and not randomize:
+        raise ValueError("device_shuffle applies to randomize=True")
     mat0 = object.counts
     _check_no_empty(mat0)
     nrow, ncol = mat0.shape
@@ -601,6 +613,7 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
     rste, dste, cste = np.full(nrank, np.nan), np.full(nrank, np.nan), np.full(nrank, np.nan)
     g = np.random.Generator(np.random.Philox(key=[int(seed), 77]))
     eng = Engine(mat0, device=device)
+    sample = eng
     labels_last = None
     try:
         for irank, rank in enumerate(ranks):
@@ -609,19 +622,23 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
             rdat, ddat, cdat = [], [], []
             for ismpl in range(1, nsmpl + 1):
                 mat = mat0
-                if randomize:                                    # :172-173 column-wise shuffle
+                if randomize and not device_shuffle:             # :172-173 column-wise shuffle
                     dense = np.asarray(mat0.todense())
                     for j in range(ncol):
                         dense[:, j] = g.permutation(dense[:, j])
                     mat = sp.csc_matrix(dense)
                     eng.close()
                     eng = Engine(mat, device=device)
+                if device_shuffle:                               # :172-173 on the GPU
+                    sample = eng.shuffle(seed * 100003 + 1000 * rank + 37 * ismpl)
+                else:
+                    sample = eng
                 rmax, labels = -np.inf, []
                 for irun in range(1, nrun + 1):
                     w0, h0 = synth.uniform_init(nrow, ncol, rank,
                                                 seed * 100003 + 1000 * rank + 37 * ismpl + irun)
-                    res = eng.ml_run(w0, h0, Itmax=Itmax, Tol=Tol, criterion=criterion,
-                                     ncnn_step=ncnn_step)
+                    res = sample.ml_run(w0, h0, Itmax=Itmax, Tol=Tol, criterion=criterion,
+                                        ncnn_step=ncnn_step)
                     lk0 = res["lik"]
                     labels.append(np.argmax(res["h"], axis=0) + 1)  # connectivity(), :51-60
                     disp = dispersion_from_labels(labels)
@@ -630,6 +647,8 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
                             res["niter"], lk0, disp))
                     if (irun == 1 or lk0 > rmax) and not np.isnan(lk0):  # :219-223
                         rmax, wmax, hmax = lk0, res["w"], res["h"]
+                if sample is not eng:
+                    sample.close()
                 coph = _cophenet(labels, ncol, linkage)
                 labels_last = labels
                 if verbose >= 1:
@@ -650,6 +669,7 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
                 cste[irank] = np.std(cdat, ddof=1) / den
             rave[irank], dave[irank], coav[irank] = np.mean(rdat), np.mean(ddat), np.mean(cdat)
     finally:
+        sample.close()
         eng.close()
     object.ranks = ranks
     object.basis, object.coeff = wdat, hdat

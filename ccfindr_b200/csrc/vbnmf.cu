@@ -40,6 +40,7 @@
 #include "svd_init.cuh"
 #include "mtx_ingest.cuh"
 #include "qc.cuh"
+#include "shuffle.cuh"
 #include "rp_ranks.h"
 #include "rp_table.h"
 
@@ -1360,6 +1361,31 @@ void launch_subset_compact(H *h, const H *src, const int32_t *d_cols, const int3
 
 }  // namespace
 
+// ---- column shuffle (shuffle.cuh) ---------------------------------------------------------------
+namespace {
+
+// the shuffled CSC of src into h's arrays (h->d_colptr already holds src's column pointers)
+template <typename VT>
+int launch_shuffle(H *h, const H *src, uint64_t seed, unsigned *d_bad) {
+    const int64_t per_warp = vb::shuffle_words(h->n) * 2 * 4;
+    const int warps = (int)std::min<int64_t>(vb::kShuffleWarps, vb::kShuffleSmemMax / per_warp);
+    const int smem = (int)(warps * per_warp);
+    auto kern = vb::shuffle_columns_kernel<VT>;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem));
+    const int grid = (int)std::min<int64_t>((int64_t)h->num_sms * std::max(per_sm, 1),
+                                            cdiv(h->m, warps));
+    kern<<<grid, warps * 32, smem, h->stream>>>(h->n, h->m, seed, src->d_colptr,
+                                                (const VT *)src->d_val, h->d_rowidx, (VT *)h->d_val,
+                                                d_bad);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+}  // namespace
+
 extern "C" {
 
 const char *vbnmf_last_error(const vbnmf_handle *h) {
@@ -1833,6 +1859,73 @@ int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *ke
     if ((rc = body())) return bail(rc);
     h->val_float = as_float;
     rc = as_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
+    if (rc) return bail(rc);
+    *out = h;
+    return 0;
+}
+
+int vbnmf_create_shuffled(vbnmf_handle **out, vbnmf_handle *src, uint64_t seed) {
+    if (!out) return VBNMF_ERR_ARG;
+    *out = nullptr;
+    H *h = new H();
+    auto bail = [&](int rc) {
+        g_create_error = h->err;
+        vbnmf_destroy(h);
+        return rc;
+    };
+    StageTimer tm("vbnmf_create_shuffled(total)");
+    if (!src) return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: bad arguments"));
+    // the draw is keyed by the column index: a shard would need its global column offset
+    if (src->nranks > 1)
+        return bail(fail(h, VBNMF_ERR_STATE, "vbnmf_create_shuffled: the source holds one shard of "
+                                             "the cells (vbnmf_attach_comm)"));
+    if (src->n > vb::kShuffleMaxRows)
+        return bail(fail(h, VBNMF_ERR_ARG,
+                         "vbnmf_create_shuffled: n = " + std::to_string(src->n) + " rows; at most " +
+                             std::to_string(vb::kShuffleMaxRows) +
+                             " (a column's row bitmap must fit one CTA's shared memory)"));
+    const int64_t n = src->n, m = src->m, nnz = src->nnz;
+    h->n = n; h->m = m; h->nnz = nnz;
+    int rc = init_common(h, src->device);
+    if (rc) return bail(rc);
+    h->val_float = src->val_float;
+    auto body = [&]() -> int {
+        unsigned *d_bad = nullptr;
+        struct Free {
+            cudaStream_t s; unsigned **p;
+            ~Free() { vfree(s, *p); }
+        } fr{h->stream, &d_bad};
+        int optin = 0;
+        CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+        if (optin < vb::shuffle_words(n) * 2 * 4)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: the row bitmap of a column does "
+                                          "not fit this device's shared memory");
+        // src's arrays are read on this handle's stream: src's own work on them must be complete
+        CK(cudaStreamSynchronize(src->stream));
+        cudaStream_t s = h->stream;
+        // allocation order of the other create paths: the arena first, then the CSC arrays
+        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
+        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
+        CK(cudaMemcpyAsync(h->d_colptr, src->d_colptr, (size_t)(m + 1) * 8,
+                           cudaMemcpyDeviceToDevice, s));
+        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
+        CK(vmalloc(h, &h->d_val, (size_t)nnz * (h->val_float ? 4 : 8)));
+        CK(vmalloc(h, &d_bad, 4));
+        CK(cudaMemsetAsync(d_bad, 0, 4, s));
+        const int lrc = h->val_float ? launch_shuffle<float>(h, src, seed, d_bad)
+                                     : launch_shuffle<double>(h, src, seed, d_bad);
+        if (lrc) return lrc;
+        unsigned bad = 0;
+        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        if (bad)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: a column holds more entries than "
+                                          "there are rows (repeated entries)");
+        return 0;
+    };
+    if ((rc = body())) return bail(rc);
+    rc = h->val_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
     if (rc) return bail(rc);
     *out = h;
     return 0;

@@ -108,7 +108,7 @@ class Engine:
                                         rowidx.ctypes.data_as(_lib.c_i32p), _dp(values)))
         return sp.csc_matrix((values, rowidx, colptr), shape=(self.n, self.m))
 
-    # -- cell / gene QC ------------------------------------------------------------------------
+    # -- cell / gene QC, column shuffle -------------------------------------------------------
     def qc_stats(self):
         """Per-cell and per-gene statistics of the resident matrix, computed on the device (the
         inputs of filter_cells / filter_genes / calc_vmr, R/utils.R:78-95,134-218): cell_sum (m),
@@ -145,13 +145,27 @@ class Engine:
                 raise ValueError("col_scale must be finite")
         rows = np.ascontiguousarray(keep_rows, dtype=np.uint8)
         cols = np.ascontiguousarray(keep_cols, dtype=np.uint8)
+        return self._derived(lambda out: self.lib.vbnmf_create_subset(
+            out, self.handle, rows.ctypes.data_as(_lib.c_u8p), cols.ctypes.data_as(_lib.c_u8p),
+            _dp(scale)))
+
+    def shuffle(self, seed):
+        """A new Engine on the same device holding this engine's matrix with every column shuffled
+        over the genes: the null matrix of factorize(randomize=TRUE) (R/factorize.R:172-173).
+        colptr and each column's values are kept and only the rows are drawn, from a counter RNG
+        keyed by (seed, column); synth.shuffle_columns_reference is the CPU restatement.  Built
+        from this engine's device arrays: nothing crosses the bus.  This engine is left as it
+        was."""
+        return self._derived(lambda out: self.lib.vbnmf_create_shuffled(
+            out, self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF))
+
+    def _derived(self, create):
+        """An Engine around the handle create(out) makes from this engine's handle."""
         out = Engine.__new__(Engine)
         out.lib = self.lib
         out.handle = C.c_void_p()
         out._keep = None
-        rc = self.lib.vbnmf_create_subset(C.byref(out.handle), self.handle,
-                                          rows.ctypes.data_as(_lib.c_u8p),
-                                          cols.ctypes.data_as(_lib.c_u8p), _dp(scale))
+        rc = create(C.byref(out.handle))
         if rc != 0:
             msg = self.lib.vbnmf_last_error(None)
             out.handle = C.c_void_p()

@@ -216,3 +216,67 @@ def device_random_init_reference(nrow, ncol, rank, hyper, seed, cell_offset=0):
             ident = (1 << 62) | ((j + cell_offset) << 6) | k
             h[k, j] = hyper["bh"] / hyper["ah"] * _Stream(seed, ident).gamma(hyper["ah"])
     return w, h
+
+
+# ---- CPU restatement of the on-device column shuffle (csrc/shuffle.cuh) ----------------------
+_GOLDEN = np.uint64(0x9E3779B97F4A7C15)
+
+
+def _mix64_np(z):
+    z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+    z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    return z ^ (z >> np.uint64(31))
+
+
+def _umulhi(u, n):
+    """(u * n) >> 64 for a uint64 array u and 0 < n < 2^31, computed on the 32-bit halves of u
+    (exact: hi * n + (lo * n >> 32) < 2^64)."""
+    n = np.uint64(n)
+    hi, lo = u >> np.uint64(32), u & np.uint64(0xFFFFFFFF)
+    return (hi * n + ((lo * n) >> np.uint64(32))) >> np.uint64(32)
+
+
+def _shuffle_draws(seed, j, count):
+    """u_0 .. u_{count-1} of column j: the first `count` next() of VbStream(seed, 3 << 62 | j)."""
+    s0 = np.uint64(_Stream(seed, (3 << 62) | int(j)).s)
+    with np.errstate(over="ignore"):
+        return _mix64_np(s0 + np.arange(1, count + 1, dtype=np.uint64) * _GOLDEN)
+
+
+def shuffle_rows(seed, j, n, k):
+    """s_0 .. s_{k-1}: the first k distinct rows umulhi(u_t, n) among the draws of column j."""
+    if k > n:
+        raise ValueError("a column holds more entries than there are rows")
+    if k == 0:
+        return np.zeros(0, dtype=np.int64)
+    # expected draws for k distinct of n: n (H_n - H_{n-k}) <= k + k^2 / (n - k); the batch is
+    # doubled until it holds k distinct rows (for k close to n the k^2 term is capped)
+    nb = k + min(k * k // max(n - k, 1), 8 * k) + 64
+    while True:
+        with np.errstate(over="ignore"):
+            r = _umulhi(_shuffle_draws(seed, j, nb), n)
+        _, first = np.unique(r, return_index=True)
+        if len(first) >= k:
+            return r[np.sort(first)[:k]].astype(np.int64)
+        nb *= 2
+
+
+def shuffle_columns_reference(csc, seed):
+    """What Engine.shuffle(seed) holds: each column of `csc` shuffled over the rows
+    (factorize(randomize=TRUE), R/factorize.R:172-173).  indptr is kept; the t-th stored entry of
+    column j (stored zeros included, ascending source row) goes to row
+    shuffle_rows(seed, j, n, k)[t], and every column is sorted by row."""
+    X = sp.csc_matrix(csc)
+    if not X.has_sorted_indices:
+        X = X.copy()
+        X.sort_indices()
+    n, m = X.shape
+    rows = np.empty(X.nnz, dtype=np.int32)
+    vals = np.empty(X.nnz, dtype=np.float64)
+    for j in range(m):
+        b, e = int(X.indptr[j]), int(X.indptr[j + 1])
+        s = shuffle_rows(seed, j, n, e - b)
+        o = np.argsort(s)
+        rows[b:e] = s[o]
+        vals[b:e] = X.data[b:e][o]
+    return sp.csc_matrix((vals, rows, X.indptr.copy()), shape=(n, m))

@@ -21,6 +21,8 @@
  *   filter_genes(): rowSums, VMR, cells expressed, R/utils.R:134-218   vbnmf_qc_stats +
  *                                                                      vbnmf_create_subset
  *   normalize_count(): counts scaled per cell, R/utils.R:318-327       vbnmf_create_subset (col_scale)
+ *   factorize(randomize = TRUE): each column of the counts shuffled    vbnmf_create_shuffled
+ *     over the genes, R/factorize.R:172-173
  *   Rmpi task farm over restarts, R/bayesian.R:263                     one handle per process/GPU;
  *                                                                      cells sharded: vbnmf_attach_comm
  *
@@ -124,6 +126,20 @@ VBNMF_API int vbnmf_qc_stats(vbnmf_handle *h, double *cell_sum, double *gene_sum
  * VBNMF_ERR_ARG; src with more than one rank attached: VBNMF_ERR_STATE. */
 VBNMF_API int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *keep_rows,
                                   const uint8_t *keep_cols, const double *col_scale);
+
+/* A new handle on src's device holding src's matrix with each column shuffled over the genes: the
+ * null matrix of factorize(randomize = TRUE) (R/factorize.R:172-173).  colptr, nnz and each
+ * column's values (stored zeros included) are kept; only the rows are drawn.  Column j with k
+ * entries: u_t = the (t+1)-th next() of the counter stream (seed, 3 << 62 | j) of
+ * vbnmf_init_random, row of draw t = (u_t * n) >> 64, s_0 .. s_{k-1} = the first k distinct rows
+ * drawn; the t-th stored entry goes to row s_t, and the column is stored sorted by row (csrc/
+ * shuffle.cuh, restated in ccfindr_b200/synth.py:shuffle_columns_reference).  Built from src's
+ * device arrays after src's stream has finished; src is not modified.  The values keep src's
+ * format, so the handle equals vbnmf_create on the same CSC.  A gene left without entries is
+ * accepted here and refused when a factorization is set up (VBNMF_ERR_EMPTY).  n above 929,792
+ * rows (one column's row bitmap must fit one CTA's 227 KB of shared memory) or a column with more
+ * entries than rows: VBNMF_ERR_ARG; src with more than one rank attached: VBNMF_ERR_STATE. */
+VBNMF_API int vbnmf_create_shuffled(vbnmf_handle **out, vbnmf_handle *src, uint64_t seed);
 
 VBNMF_API void vbnmf_destroy(vbnmf_handle *h);
 VBNMF_API const char *vbnmf_last_error(const vbnmf_handle *h); /* h may be NULL: error of the last create */
