@@ -27,7 +27,9 @@ class VbnmfError(RuntimeError):
         self.code = code
 
 
+ERR_ARG = 1
 ERR_HYPER = 2
+ERR_MEMORY = 7
 
 # name -> (restype, argtypes); every symbol declared in include/vbnmf.h
 SIGNATURES = {
@@ -40,6 +42,8 @@ SIGNATURES = {
     "vbnmf_qc_stats": (C.c_int, [C.c_void_p, c_dp, c_dp, c_dp, c_i64p, c_i64p]),
     "vbnmf_create_subset": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, c_u8p, c_u8p, c_dp]),
     "vbnmf_create_shuffled": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_uint64]),
+    "vbnmf_consensus": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, c_i32p, C.c_int64, c_i64p,
+                                  c_i64p, c_i64p, C.c_int64, c_i64p]),
     "vbnmf_destroy": (None, [C.c_void_p]),
     "vbnmf_last_error": (C.c_char_p, [C.c_void_p]),
     "vbnmf_set_precision": (C.c_int, [C.c_void_p, C.c_int]),

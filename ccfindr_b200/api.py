@@ -11,7 +11,9 @@ ships as source in r-shim/).  What runs where:
     factorize()      R/factorize.R:139-276 loops and measures here; the it-loop (:189-212) with
                                            nmf_updateR + likelihood on the GPU (Engine.ml_run);
                                            with device_shuffle=True the null matrices of
-                                           randomize (:172-173) on the GPU too (Engine.shuffle)
+                                           randomize (:172-173) on the GPU too (Engine.shuffle);
+                                           with device_consensus=True dispersion and the
+                                           cophenetic correlation (:51-78) too (engine.consensus)
     cluster_id()     R/utils.R:903-909     first-maximum argmax per cell (GPU: Engine.cluster_id)
     optimal_rank()   R/utils2.R:59-95      host post-processing of measure (smoothing spline)
     filter_cells(), filter_genes(), calc_vmr(), normalize_count()
@@ -28,7 +30,7 @@ import numpy as np
 import scipy.sparse as sp
 
 from . import synth
-from ._lib import ERR_HYPER, VbnmfError
+from ._lib import ERR_HYPER, ERR_MEMORY, VbnmfError
 from .engine import EPS, Engine
 
 
@@ -301,7 +303,7 @@ def vb_factorize(object, ranks=2, nrun=1, verbose=2, progress_bar=True, initiali
                  Itmax=10000, hyper_update=(True,) * 4, gamma_a=1, gamma_b=1, Tol=1e-5,
                  hyper_update_n0=10, hyper_update_dn=1, connectivity=True, fudge=None, ncores=1,
                  useC=True, unif_stop=True, seed=1, device=0, inits=None, precision=0,
-                 parallel=False, device_init=False, shard_cells=False):
+                 parallel=False, device_init=False, shard_cells=False, device_consensus=False):
     """Bayesian NMF inference of a count matrix (R/bayesian.R:229-301).
 
     Arguments as in the reference (dots replaced by underscores).  Extras: `seed` keys the NumPy
@@ -322,6 +324,8 @@ def vb_factorize(object, ranks=2, nrun=1, verbose=2, progress_bar=True, initiali
     once per iteration (SURVEY.md 8e), and the coeff / dcoeff columns are gathered at the end, so
     every rank returns the same full object.  For matrices that do not fit one GPU, or to cut the
     time of one large factorization.
+    `device_consensus=True`: the dispersion printed with `connectivity` is computed on the GPU from
+    exact integer moments of the label runs (consensus_from_labels) instead of on the host.
     """
     if fudge is None:
         fudge = EPS                                             # :238
@@ -340,7 +344,7 @@ def vb_factorize(object, ranks=2, nrun=1, verbose=2, progress_bar=True, initiali
     if device_init:
         initializer += "_device"
     common = (ga, gb, initializer, Itmax, hyper_update, Tol, hyper_update_n0, hyper_update_dn,
-              connectivity, fudge)
+              connectivity, fudge, device_consensus)
     vb = []
     if parallel and shard_cells:
         raise ValueError("parallel (independent jobs per GPU) and shard_cells (one job on all GPUs) "
@@ -514,7 +518,8 @@ def _vb_parallel(mat, ranks, nrun, common, unif_stop, verbose, seed, inits, devi
 
 
 def _vb_iterate(eng, irun, mat, ranks, ga, gb, initializer, Itmax, hyper_update, Tol, n0, dn,
-                connectivity, fudge, unif_stop, nrun, verbose, seed, inits, previous, cols=None):
+                connectivity, fudge, device_consensus, unif_stop, nrun, verbose, seed, inits,
+                previous, cols=None):
     """R/bayesian.R:303-390 for one run; the it-loop runs on the GPU.  cols = (c0, c1): the engine
     holds the cells [c0, c1) of `mat` and the calls are collective over the shards."""
     nrow, ncol = mat.shape
@@ -560,7 +565,11 @@ def _vb_iterate(eng, irun, mat, ranks, ga, gb, initializer, Itmax, hyper_update,
         if connectivity:                                        # :353-357 (only printed)
             out["labels"][irank] = eng.cluster_id()
             runs = [p["labels"][irank] for p in previous if p["labels"][irank] is not None]
-            disp = dispersion_from_labels(runs + [out["labels"][irank]])
+            if device_consensus:
+                disp = consensus_from_labels(runs + [out["labels"][irank]], tree=False,
+                                             device=eng.device)[0]
+            else:
+                disp = dispersion_from_labels(runs + [out["labels"][irank]])
         if verbose >= 2:
             msg = "Rank = %d: Nsteps = %d, log(evidence) = %s, hyper = (%s,%s,%s,%s)" % (
                 rank, it, lk0, hyper["aw"], hyper["bw"], hyper["ah"], hyper["bh"])
@@ -586,7 +595,8 @@ def _vb_iterate(eng, irun, mat, ranks, ga, gb, initializer, Itmax, hyper_update,
 
 def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, progress_bar=True,
               Itmax=10000, ncnn_step=40, criterion="likelihood", linkage="average", Tol=1e-5,
-              store_connectivity=False, seed=1, device=0, device_shuffle=False):
+              store_connectivity=False, seed=1, device=0, device_shuffle=False,
+              device_consensus=False):
     """Maximum likelihood factorization (R/factorize.R:139-276); the it-loop (:189-212) runs on the
     GPU with either stopping criterion.  The consensus measures never form the m(m-1)/2
     connectivity vector of the reference (:51-78): dispersion and the cophenetic correlation are
@@ -598,11 +608,18 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
     `device_shuffle=True` (needs `randomize=True`): the counts are uploaded once and each null
     matrix is drawn on the GPU from the resident copy (Engine.shuffle; no dense matrix, no upload):
     sample `ismpl` of rank `r` is Engine.shuffle(seed * 100003 + 1000 * r + 37 * ismpl), closed
-    after its `nrun` restarts.  Same distribution, different draw than the default."""
+    after its `nrun` restarts.  Same distribution, different draw than the default.
+    `device_consensus=True` (average linkage only): dispersion and the cophenetic correlation are
+    computed on the GPU (consensus_from_labels) from exact integer moments and the merge list of
+    the average-linkage tree, with no cap on the number of label groups below what device memory
+    holds.  Equal distances are merged in a defined order (smallest group indices first), so the
+    cophenetic value can differ from the default's, which breaks such ties differently."""
     if criterion not in ("likelihood", "connectivity"):
         raise ValueError("Unknown stopping criterion.")        # :212
     if device_shuffle and not randomize:
         raise ValueError("device_shuffle applies to randomize=True")
+    if device_consensus and linkage != "average":
+        raise ValueError("device_consensus supports linkage='average' only")
     mat0 = object.counts
     _check_no_empty(mat0)
     nrow, ncol = mat0.shape
@@ -641,7 +658,10 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
                                         ncnn_step=ncnn_step)
                     lk0 = res["lik"]
                     labels.append(np.argmax(res["h"], axis=0) + 1)  # connectivity(), :51-60
-                    disp = dispersion_from_labels(labels)
+                    if device_consensus:
+                        disp = consensus_from_labels(labels, tree=False, device=device)[0]
+                    else:
+                        disp = dispersion_from_labels(labels)
                     if verbose >= 2:
                         print("Nsteps = %d , likelihood = %s , dispersion = %s\n" % (
                             res["niter"], lk0, disp))
@@ -649,7 +669,10 @@ def factorize(object, ranks=2, nrun=20, randomize=False, nsmpl=1, verbose=2, pro
                         rmax, wmax, hmax = lk0, res["w"], res["h"]
                 if sample is not eng:
                     sample.close()
-                coph = _cophenet(labels, ncol, linkage)
+                if device_consensus:
+                    coph = consensus_from_labels(labels, device=device)[1]
+                else:
+                    coph = _cophenet(labels, ncol, linkage)
                 labels_last = labels
                 if verbose >= 1:
                     print("Sample# %d : Max(likelihood) = %s , dispersion = %s , cophenetic = %s"
@@ -777,6 +800,64 @@ def cophenet_from_labels(label_runs, method="average", max_groups=6000):
 
 def _cophenet(labels, nc, method="average"):
     return cophenet_from_labels(labels, method)
+
+
+# ---- consensus measures from integer moments and the merge list (vbnmf_consensus) -------------
+def dispersion_from_moments(s1, s2, m, nrun):
+    """dispersion (R/factorize.R:62-67) from S1 = sum a and S2 = sum a^2 over the m(m-1)/2 cell
+    pairs, a = runs in which both cells share a label: sum (a/nrun - 1/2)^2 = con4 / (4 nrun^2)
+    with the integer con4 = 4 S2 - 4 nrun S1 + nrun^2 m(m-1)/2."""
+    s1, s2, m, nrun = int(s1), int(s2), int(m), int(nrun)
+    con4 = 4 * s2 - 4 * nrun * s1 + nrun * nrun * (m * (m - 1) // 2)
+    return 1.0 / m + 8.0 * (con4 / (4.0 * nrun * nrun)) / m ** 2
+
+
+def cophenet_from_merges(s1, s2, m, nrun, merges):
+    """cophenet (R/factorize.R:69-78) under average linkage from S1, S2 and the merge list
+    ((G-1) x 5: a, b, IP_ab, N_a, N_b; vbnmf_consensus).  A merge joins N_a N_b cell pairs at
+    height h = 1 - IP_ab / (nrun N_a N_b), which is also their mean distance, so
+    sum d c = sum c^2 and every moment of the correlation is a sum over the merges or an integer.
+    NaN when m < 3 or either variance is not positive, as cophenet_from_labels."""
+    s1, s2, m, nrun = int(s1), int(s2), int(m), int(nrun)
+    if m < 3:
+        return np.nan
+    P = m * (m - 1) // 2
+    mg = np.asarray(merges, dtype=np.int64).reshape(-1, 5)
+    p = (mg[:, 3] * mg[:, 4]).astype(np.float64)
+    h = 1.0 - mg[:, 2].astype(np.float64) / (np.int64(nrun) * mg[:, 3] * mg[:, 4]).astype(np.float64)
+    hp = h * p
+    sc = float(np.cumsum(hp)[-1]) if len(hp) else 0.0          # sequential sums, merge order
+    sc2 = float(np.cumsum(h * hp)[-1]) if len(hp) else 0.0
+    sd = (nrun * P - s1) / nrun
+    sd2 = (nrun * nrun * P - 2 * nrun * s1 + s2) / (nrun * nrun)
+    cov = sc2 - sd * sc / P
+    vd = sd2 - sd * sd / P
+    vc = sc2 - sc * sc / P
+    if vd <= 0 or vc <= 0:
+        return np.nan
+    return float(cov / np.sqrt(vd * vc))
+
+
+def consensus_from_labels(label_runs, tree=True, device=0, max_groups=0):
+    """(dispersion, cophenetic) of label runs (1-based, as factorize makes them) computed on the
+    GPU (engine.consensus): the moments always, the average-linkage tree when tree=True (else the
+    cophenetic value is None).  More label groups than max_groups or device memory allow: a
+    warning and a NaN cophenetic value, as cophenet_from_labels past its cap."""
+    from . import engine
+    L = np.stack([np.asarray(v) for v in label_runs]).astype(np.int64) - 1
+    nrun, m = L.shape
+    try:
+        res = engine.consensus(L, device=device, tree=tree, max_groups=max_groups)
+    except VbnmfError as e:
+        if e.code != ERR_MEMORY:
+            raise
+        warnings.warn("cophenetic correlation not computed: %d label groups (%s)" % (e.ngroups, e))
+        res = engine.consensus(L, device=device, tree=False)
+        return dispersion_from_moments(res["s1"], res["s2"], m, nrun), np.nan
+    disp = dispersion_from_moments(res["s1"], res["s2"], m, nrun)
+    if not tree:
+        return disp, None
+    return disp, cophenet_from_merges(res["s1"], res["s2"], m, nrun, res["merges"])
 
 
 def cluster_id(object, rank=2):

@@ -41,6 +41,7 @@
 #include "mtx_ingest.cuh"
 #include "qc.cuh"
 #include "shuffle.cuh"
+#include "consensus.cuh"
 #include "rp_ranks.h"
 #include "rp_table.h"
 
@@ -1386,6 +1387,180 @@ int launch_shuffle(H *h, const H *src, uint64_t seed, unsigned *d_bad) {
 
 }  // namespace
 
+// ---- consensus measures (consensus.cuh) ---------------------------------------------------------
+namespace {
+
+// device buffers freed (stream-ordered) when the scope ends
+struct ScopedBufs {
+    cudaStream_t s;
+    std::vector<void *> p;
+    ~ScopedBufs() { for (void *q : p) vfree(s, q); }
+    template <typename T>
+    cudaError_t get(H *h, T **x, size_t bytes) {
+        *x = nullptr;
+        const cudaError_t e = vmalloc(h, x, bytes);
+        if (e == cudaSuccess) p.push_back((void *)*x);
+        return e;
+    }
+};
+
+inline int64_t choose2(unsigned long long x) { return (int64_t)(x * (x - 1) / 2); }
+
+// S1 = sum over runs t of sum_c C(n^t_c, 2) (the tables of the pairs (t, t) are diagonal);
+// S2 = S1 + 2 sum_{t < u} sum_{c, c'} C(M^tu_cc', 2).  Pairs go in batches whose tables fit 256 MB.
+int consensus_moments(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, int64_t moments[2]) {
+    const int KK = K * K;
+    const int64_t npairs = (int64_t)nrun * (nrun + 1) / 2;
+    std::vector<int32_t> pt, pu;
+    for (int t = 0; t < nrun; t++)
+        for (int u = t; u < nrun; u++) { pt.push_back(t); pu.push_back(u); }
+    const int64_t batch = std::max<int64_t>(1, std::min<int64_t>({npairs, 65535,
+                                                                 (256ll << 20) / ((int64_t)KK * 8)}));
+    ScopedBufs B{h->stream, {}};
+    int32_t *d_pt = nullptr, *d_pu = nullptr;
+    unsigned long long *d_tab = nullptr;
+    CK(B.get(h, &d_pt, (size_t)npairs * 4));
+    CK(B.get(h, &d_pu, (size_t)npairs * 4));
+    CK(B.get(h, &d_tab, (size_t)batch * KK * 8));
+    CK(cudaMemcpyAsync(d_pt, pt.data(), (size_t)npairs * 4, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d_pu, pu.data(), (size_t)npairs * 4, cudaMemcpyHostToDevice, h->stream));
+    const int smem = KK * 4;
+    CK(cudaFuncSetAttribute(vb::pair_contingency_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            std::max(smem, 1)));
+    std::vector<unsigned long long> tab((size_t)batch * KK);
+    int64_t s1 = 0, cross = 0;
+    for (int64_t p0 = 0; p0 < npairs; p0 += batch) {
+        const int64_t np = std::min(batch, npairs - p0);
+        CK(cudaMemsetAsync(d_tab, 0, (size_t)np * KK * 8, h->stream));
+        const int gx = (int)std::max<int64_t>(1, std::min<int64_t>(cdiv(m, vb::kBlock),
+                                                                   cdiv(4 * h->num_sms, np)));
+        vb::pair_contingency_kernel<<<dim3(gx, (unsigned)np), vb::kBlock, smem, h->stream>>>(
+            m, nrun, K, d_lab, d_pt + p0, d_pu + p0, d_tab);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        CK(copy_sync(h, tab.data(), d_tab, (size_t)np * KK * 8, cudaMemcpyDeviceToHost));
+        for (int64_t p = 0; p < np; p++) {
+            int64_t sum = 0;
+            for (int i = 0; i < KK; i++) sum += choose2(tab[(size_t)(p * KK + i)]);
+            (pt[(size_t)(p0 + p)] == pu[(size_t)(p0 + p)] ? s1 : cross) += sum;
+        }
+    }
+    moments[0] = s1;
+    moments[1] = s1 + 2 * cross;
+    return 0;
+}
+
+// Groups of cells with equal label tuples, in lexicographic order of (L[0], L[1], ...): their
+// count G, sizes (G) and tuples (G x W words, 4 labels per word).  d_size / d_tup are allocated
+// here and owned by the caller.
+int consensus_groups(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, int W, int64_t *G_out,
+                     int64_t **d_size, uint32_t **d_tup) {
+    cudaStream_t s = h->stream;
+    ScopedBufs B{s, {}};
+    uint32_t *d_k0, *d_k1;
+    int32_t *d_p0, *d_p1, *d_flag, *d_gid;
+    CK(B.get(h, &d_k0, (size_t)m * 4));
+    CK(B.get(h, &d_k1, (size_t)m * 4));
+    CK(B.get(h, &d_p0, (size_t)m * 4));
+    CK(B.get(h, &d_p1, (size_t)m * 4));
+    int bits = 1;
+    while ((1 << bits) < K) bits++;
+    cub::DoubleBuffer<uint32_t> keys(d_k0, d_k1);
+    cub::DoubleBuffer<int32_t> vals(d_p0, d_p1);
+    size_t sort_bytes = 0, scan_bytes = 0;
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)m, 0, bits, s));
+    CK(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, d_p0, d_p1, (int)m, s));
+    void *d_tmp = nullptr;
+    CK(B.get(h, &d_tmp, std::max(sort_bytes, scan_bytes)));
+    std::vector<int32_t> iota((size_t)m);
+    std::iota(iota.begin(), iota.end(), 0);
+    CK(cudaMemcpyAsync(vals.Current(), iota.data(), (size_t)m * 4, cudaMemcpyHostToDevice, s));
+    const int gm = cdiv(m, vb::kBlock);
+    for (int t = nrun - 1; t >= 0; t--) {  // LSD: cub's radix sort is stable
+        vb::group_gather_key_kernel<<<gm, vb::kBlock, 0, s>>>(m, d_lab + (int64_t)t * m,
+                                                             vals.Current(), keys.Current());
+        CK(cub::DeviceRadixSort::SortPairs(d_tmp, sort_bytes, keys, vals, (int)m, 0, bits, s));
+        h->launches += 2;
+    }
+    const int32_t *d_perm = vals.Current();
+    d_flag = (int32_t *)d_k0;  // the key buffers are free now
+    d_gid = (int32_t *)d_k1;
+    vb::group_flag_kernel<<<gm, vb::kBlock, 0, s>>>(m, nrun, d_lab, d_perm, d_flag);
+    CK(cub::DeviceScan::InclusiveSum(d_tmp, scan_bytes, d_flag, d_gid, (int)m, s));
+    int32_t G32 = 0;
+    CK(copy_sync(h, &G32, d_gid + m - 1, 4, cudaMemcpyDeviceToHost));
+    const int64_t G = G32;
+    int64_t *d_start;
+    CK(B.get(h, &d_start, (size_t)G * 8));
+    CK(vmalloc(h, d_size, (size_t)G * 8));
+    CK(vmalloc(h, d_tup, (size_t)G * W * 4));
+    vb::group_start_kernel<<<gm, vb::kBlock, 0, s>>>(m, nrun, W, d_lab, d_perm, d_flag, d_gid,
+                                                     d_start, *d_tup);
+    vb::group_size_kernel<<<cdiv(G, vb::kBlock), vb::kBlock, 0, s>>>(G, m, d_start, *d_size);
+    h->launches += 4;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(s));
+    *G_out = G;
+    return 0;
+}
+
+// bytes the pool can still hand out: the driver's free memory plus what the pool keeps cached
+size_t device_bytes_available(H *h) {
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return 0;
+    cudaMemPool_t mp;
+    uint64_t reserved = 0, used = 0;
+    if (cudaDeviceGetDefaultMemPool(&mp, h->device) == cudaSuccess &&
+        cudaMemPoolGetAttribute(mp, cudaMemPoolAttrReservedMemCurrent, &reserved) == cudaSuccess &&
+        cudaMemPoolGetAttribute(mp, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess &&
+        reserved > used)
+        free_b += (size_t)(reserved - used);
+    return free_b;
+}
+
+// the packed IP triangle, the row cache and the merge loop; merges (G - 1) x 5 on the host
+int consensus_tree(H *h, int64_t G, int nrun, int W, const int64_t *d_size0, const uint32_t *d_tup,
+                   int64_t *merges, int64_t *rescans) {
+    cudaStream_t s = h->stream;
+    ScopedBufs B{s, {}};
+    vb::MergeArgs A;
+    A.G = G;
+    A.nrun = nrun;
+    const int64_t ntri = G * (G - 1) / 2;
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, vb::merge_loop_kernel, vb::kMergeBlock, 0));
+    const int grid = h->num_sms * std::max(per_sm, 1);
+    CK(B.get(h, &A.ip, (size_t)ntri * 8));
+    CK(B.get(h, &A.size, (size_t)G * 8));
+    CK(B.get(h, &A.bq, (size_t)G * 8));
+    CK(B.get(h, &A.bb, (size_t)G * 4));
+    CK(B.get(h, &A.merges, (size_t)(G - 1) * 5 * 8));
+    CK(B.get(h, &A.resc, (size_t)G * 4));
+    CK(B.get(h, &A.nresc, 16));
+    CK(B.get(h, &A.part_q, (size_t)grid * 8));
+    CK(B.get(h, &A.part_a, (size_t)grid * 8));
+    CK(B.get(h, &A.rescans, 8));
+    CK(cudaMemcpyAsync(A.size, d_size0, (size_t)G * 8, cudaMemcpyDeviceToDevice, s));
+    CK(cudaMemsetAsync(A.rescans, 0, 8, s));
+    const int pad = 4 * W - nrun;
+    const dim3 fill_grid(cdiv(G, 64), (unsigned)std::min<int64_t>(cdiv(G, 4), 65535));
+    vb::ip_fill_kernel<<<fill_grid, vb::kBlock, 0, s>>>(G, W, pad, d_tup, A.size, A.ip);
+    vb::row_best_kernel<<<(int)std::min<int64_t>(G, 1 << 20), vb::kMergeBlock, 0, s>>>(
+        G, nrun, A.ip, A.size, A.bq, A.bb);
+    h->launches += 2;
+    CK(cudaGetLastError());
+    void *args[] = {&A};
+    CK(cudaLaunchCooperativeKernel((void *)vb::merge_loop_kernel, grid, vb::kMergeBlock, args, 0, s));
+    h->launches += 1;
+    CK(cudaMemcpyAsync(merges, A.merges, (size_t)(G - 1) * 5 * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(rescans, A.rescans, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+}  // namespace
+
 extern "C" {
 
 const char *vbnmf_last_error(const vbnmf_handle *h) {
@@ -1929,6 +2104,76 @@ int vbnmf_create_shuffled(vbnmf_handle **out, vbnmf_handle *src, uint64_t seed) 
     if (rc) return bail(rc);
     *out = h;
     return 0;
+}
+
+int vbnmf_consensus(int device, int64_t m, int nrun, int nlabels, const int32_t *labels,
+                    int64_t max_groups, int64_t moments[2], int64_t *ngroups, int64_t *merges,
+                    int64_t merge_cap, int64_t *rescans) {
+    H *h = new H();
+    auto done = [&](int rc) {
+        g_create_error = h->err;
+        vbnmf_destroy(h);
+        return rc;
+    };
+    auto arg = [&](const std::string &msg) { return done(fail(h, VBNMF_ERR_ARG, "vbnmf_consensus: " + msg)); };
+    if (ngroups) *ngroups = 0;
+    if (rescans) *rescans = 0;
+    if (!labels || !moments || (merges && (!ngroups || !rescans)))
+        return arg("labels and moments are required, ngroups and rescans with merges");
+    if (nrun < 1 || m < 1 || m > INT32_MAX) return arg("needs nrun >= 1 and 1 <= m < 2^31");
+    if (nlabels < 1 || nlabels > vb::kConsensusMaxLabels)
+        return arg("nlabels = " + std::to_string(nlabels) + "; 1 ... " +
+                   std::to_string(vb::kConsensusMaxLabels) +
+                   " (a K x K table of counters must fit one CTA's shared memory)");
+    const unsigned __int128 half = (unsigned __int128)((m + 1) / 2);
+    if ((unsigned __int128)nrun * half * half >= ((unsigned __int128)1 << 53))
+        return arg("nrun * ceil(m / 2)^2 must be below 2^53 (exact IP values and their fp64 ratios)");
+    for (int64_t i = 0; i < (int64_t)nrun * m; i++)
+        if (labels[i] < 0 || labels[i] >= nlabels)
+            return arg("label " + std::to_string(labels[i]) + " outside 0 ... nlabels - 1");
+    int rc = init_common(h, device);
+    if (rc) return done(rc);
+    StageTimer tm("vbnmf_consensus(total)");
+    const int W = (nrun + 3) / 4;
+    int64_t *d_size = nullptr;
+    uint32_t *d_tup = nullptr;
+    auto body = [&]() -> int {
+        int32_t *d_lab = nullptr;
+        CK(vmalloc(h, &d_lab, (size_t)nrun * m * 4));
+        struct Free {
+            cudaStream_t s; int32_t *p;
+            ~Free() { vfree(s, p); }
+        } fr{h->stream, d_lab};
+        CK(cudaMemcpyAsync(d_lab, labels, (size_t)nrun * m * 4, cudaMemcpyHostToDevice, h->stream));
+        int r = consensus_moments(h, m, nrun, nlabels, d_lab, moments);
+        if (r || !merges) return r;
+        int64_t G = 0;
+        if ((r = consensus_groups(h, m, nrun, nlabels, d_lab, W, &G, &d_size, &d_tup))) return r;
+        *ngroups = G;
+        if (merge_cap < G - 1)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_consensus: merge_cap = " + std::to_string(merge_cap) +
+                                              " below G - 1 = " + std::to_string(G - 1));
+        return 0;
+    };
+    rc = body();
+    if (!rc && merges && *ngroups > 1) {
+        const int64_t G = *ngroups;
+        // the triangle, the row cache, the merge list and the sizes; 256 MB left for the rest
+        const double need = 8.0 * G * (G - 1) / 2 + 64.0 * G + (256 << 20);
+        if (max_groups > 0 && G > max_groups)
+            rc = fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) +
+                                               " groups above max_groups = " + std::to_string(max_groups));
+        else if (cudaStreamSynchronize(h->stream) != cudaSuccess ||
+                 need > (double)device_bytes_available(h))
+            rc = fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) + " groups need " +
+                                               std::to_string((int64_t)(need / 1e9)) +
+                                               " GB of device memory for the IP triangle");
+        else
+            rc = consensus_tree(h, G, nrun, W, d_size, d_tup, merges, rescans);
+    }
+    vfree(h->stream, d_size);
+    vfree(h->stream, d_tup);
+    return done(rc);
 }
 
 int vbnmf_set_precision(vbnmf_handle *h, int precision) {

@@ -35,6 +35,7 @@ class Engine:
         self.lib = _lib.load()
         self.handle = C.c_void_p()
         self._keep = None
+        self.device = int(device)
         if _device_csc is not None:
             n, m, nnz, d_colptr, d_rowidx, d_val, keep = _device_csc
             self._keep = keep  # borrowed device arrays must outlive the handle
@@ -88,6 +89,7 @@ class Engine:
         self.lib = _lib.load()
         self.handle = C.c_void_p()
         self._keep = None
+        self.device = int(device)
         dims = (C.c_int64 * 3)()
         rc = self.lib.vbnmf_create_from_mtx(C.byref(self.handle), str(path).encode(), int(device), dims)
         if rc != 0:
@@ -165,6 +167,7 @@ class Engine:
         out.lib = self.lib
         out.handle = C.c_void_p()
         out._keep = None
+        out.device = self.device
         rc = create(C.byref(out.handle))
         if rc != 0:
             msg = self.lib.vbnmf_last_error(None)
@@ -360,6 +363,40 @@ def set_host_threads(n):
 
 def trim_pool(device=0):
     _lib.check(_lib.load().vbnmf_trim_pool(int(device)))
+
+
+def consensus(labels, device=0, tree=True, max_groups=0):
+    """Consensus measures of restarts on the device (vbnmf_consensus, R/factorize.R:51-78).
+    labels: nrun x m integers 0 ... K-1 (one row per run).  Returns dict(s1, s2) -- the sums of a
+    and a^2 over cell pairs, a = runs in which both cells share a label -- and with tree=True also
+    ngroups (G), merges ((G-1) x 5 int64: a, b, IP_ab, N_a, N_b of every average-linkage merge)
+    and rescans.  More groups than max_groups (0: what device memory allows) raise VbnmfError with
+    code ERR_MEMORY and the number of groups in its `ngroups`."""
+    L = np.ascontiguousarray(np.atleast_2d(labels), dtype=np.int32)
+    nrun, m = L.shape
+    K = int(L.max()) + 1 if L.size else 1
+    mom = np.zeros(2, dtype=np.int64)
+    ng, resc = C.c_int64(0), C.c_int64(0)
+    merges = None
+    cap = 0
+    if tree:
+        cap = min(m, K ** nrun) - 1                              # G <= min(m, K^nrun)
+        merges = np.zeros((max(cap, 1), 5), dtype=np.int64)
+    lib = _lib.load()
+    rc = lib.vbnmf_consensus(int(device), m, nrun, K, L.ctypes.data_as(_lib.c_i32p), int(max_groups),
+                             mom.ctypes.data_as(_lib.c_i64p), C.byref(ng),
+                             None if merges is None else merges.ctypes.data_as(_lib.c_i64p), cap,
+                             C.byref(resc))
+    if rc != 0:
+        msg = lib.vbnmf_last_error(None)
+        err = _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
+        err.ngroups = ng.value
+        raise err
+    out = dict(s1=int(mom[0]), s2=int(mom[1]))
+    if tree:
+        G = ng.value
+        out.update(ngroups=G, merges=merges[:max(G - 1, 0)].copy(), rescans=resc.value)
+    return out
 
 
 class Comm:

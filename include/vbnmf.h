@@ -23,6 +23,8 @@
  *   normalize_count(): counts scaled per cell, R/utils.R:318-327       vbnmf_create_subset (col_scale)
  *   factorize(randomize = TRUE): each column of the counts shuffled    vbnmf_create_shuffled
  *     over the genes, R/factorize.R:172-173
+ *   factorize(): dispersion() and cophenet() of the consensus          vbnmf_consensus
+ *     connectivity, R/factorize.R:51-78,214-216,226 (average linkage)
  *   Rmpi task farm over restarts, R/bayesian.R:263                     one handle per process/GPU;
  *                                                                      cells sharded: vbnmf_attach_comm
  *
@@ -74,7 +76,8 @@ enum {
     VBNMF_ERR_CUDA = 3,
     VBNMF_ERR_STATE = 4,
     VBNMF_ERR_NCCL = 5,
-    VBNMF_ERR_EMPTY = 6  /* 'Input matrix contains empty rows/columns', R/bayesian.R:244-247 */
+    VBNMF_ERR_EMPTY = 6, /* 'Input matrix contains empty rows/columns', R/bayesian.R:244-247 */
+    VBNMF_ERR_MEMORY = 7 /* vbnmf_consensus: more label groups than max_groups or device memory allow */
 };
 
 /* Upload a CSC count matrix from HOST memory and build the device-side layouts.
@@ -140,6 +143,32 @@ VBNMF_API int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const u
  * rows (one column's row bitmap must fit one CTA's 227 KB of shared memory) or a column with more
  * entries than rows: VBNMF_ERR_ARG; src with more than one rank attached: VBNMF_ERR_STATE. */
 VBNMF_API int vbnmf_create_shuffled(vbnmf_handle **out, vbnmf_handle *src, uint64_t seed);
+
+/* Consensus measures of factorize() (R/factorize.R:51-78,214-216,226) from the labels of nrun
+ * restarts, without the m(m-1)/2 connectivity vector.  Handle-free: runs on `device` and releases
+ * everything it allocated before returning.  labels: HOST memory, run-major (nrun x m), values
+ * 0 ... nlabels - 1.  Let a_xy = number of runs in which cells x and y share a label.
+ *   moments[0] = S1 = sum_{x<y} a_xy = sum_t sum_c C(n^t_c, 2),
+ *   moments[1] = S2 = sum_{x<y} a_xy^2 = S1 + 2 sum_{t<u} sum_{c,c'} C(M^tu_cc', 2)
+ *   (exact; M^tu = K x K contingency table of runs t and u); dispersion follows from S1, S2.
+ * merges == NULL: moments only.  Otherwise also the average-linkage tree of 1 - a / nrun:
+ *   groups = the distinct columns of labels in the order of (L[0], L[1], ...); *ngroups = G;
+ *   IP_ab = n_a n_b #{t: T_at = T_bt} for groups a < b;
+ *   G - 1 greedy steps: among active a < b take the largest q_ab = IP_ab / (nrun N_a N_b) (both
+ *   exact int64 values converted to fp64, IEEE division), ties to the smallest a, then the
+ *   smallest b; record (a, b, IP_ab, N_a, N_b) as row s of merges ((G - 1) x 5, row-major);
+ *   IP_ak += IP_bk for every active k, N_a += N_b, retire b.  (The Lance-Williams update of
+ *   average linkage is exact on the integers IP.)  *rescans = rows rescanned by the row cache of
+ *   the merge loop.
+ * The tree needs 8 G (G - 1) / 2 bytes of device memory for the IP triangle.  G above max_groups
+ * (0: no limit) or above what device memory allows: VBNMF_ERR_MEMORY, with G in *ngroups.
+ * VBNMF_ERR_ARG: nrun < 1, m < 1 or m >= 2^31; nlabels outside 1 ... 240 (a K x K table of
+ * counters must fit one CTA's shared memory); a label outside 0 ... nlabels - 1;
+ * nrun * ceil(m / 2)^2 >= 2^53; merge_cap < G - 1 (G still in *ngroups).
+ * Error text: vbnmf_last_error(NULL). */
+VBNMF_API int vbnmf_consensus(int device, int64_t m, int nrun, int nlabels, const int32_t *labels,
+                              int64_t max_groups, int64_t moments[2], int64_t *ngroups,
+                              int64_t *merges, int64_t merge_cap, int64_t *rescans);
 
 VBNMF_API void vbnmf_destroy(vbnmf_handle *h);
 VBNMF_API const char *vbnmf_last_error(const vbnmf_handle *h); /* h may be NULL: error of the last create */
