@@ -69,6 +69,7 @@ SIGNATURES = {
     "vbnmf_trim_pool": (C.c_int, [C.c_int]),
     "vbnmf_init_random": (C.c_int, [C.c_void_p, C.c_int, c_dp, C.c_uint64, C.c_int64]),
     "vbnmf_init_svd2": (C.c_int, [C.c_void_p, C.c_int, c_dp, C.c_uint64, C.c_int64]),
+    "vbnmf_init_svd": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_int64]),
     "vbnmf_info": (C.c_int, [C.c_void_p, c_i64p]),
     "vbnmf_layout_info": (C.c_int, [C.c_void_p, c_i64p]),
 }

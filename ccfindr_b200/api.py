@@ -239,7 +239,14 @@ def vb_init(nrow, ncol, mat, rank, hyper, initializer, seed):
         h = np.abs(np.diag(d) @ v.T)
         scale = hyper["bh"] / h.mean()
         return w / scale, h * scale
-    w = np.zeros((nrow, rank))                                  # 'svd', :116-149
+    return svd_init_from(u, d, v)
+
+
+def svd_init_from(u, d, v):
+    """The 'svd' initializer (R/bayesian.R:116-149) from a truncated SVD: u n x r, d (r), v m x r.
+    Returns w (n x r), h (r x m).  Literal, including the typo of :136-137."""
+    nrow, ncol, rank = u.shape[0], v.shape[0], len(d)
+    w = np.zeros((nrow, rank))
     h = np.zeros((rank, ncol))
     d1 = np.sqrt(d[0])
     w[:, 0] = d1 * u[:, 0]
@@ -312,9 +319,10 @@ def vb_factorize(object, ranks=2, nrun=1, verbose=2, progress_bar=True, initiali
     `ncores` and `useC` are accepted and ignored: the update always runs on the GPU.
     `precision`: 0 = fp64 (reference arithmetic), 1 = fp32-storage / fp64-accumulate.
     `device_init=True`: the 'random' initializer is drawn on the GPU (Engine.init_random, a counter
-    RNG keyed by seed and matrix position) and the 'svd2' initializer is computed on the GPU
-    (Engine.init_svd2, randomized truncated SVD of the resident matrix) instead of on the host and
-    uploaded.
+    RNG keyed by seed and matrix position) and the 'svd2' and 'svd' initializers are computed on
+    the GPU (Engine.init_svd2, Engine.init_svd: randomized truncated SVD of the resident matrix)
+    instead of on the host and uploaded.  'svd' on the GPU orients each pair of singular vectors
+    k >= 1 before the reference formula (vbnmf_init_svd in include/vbnmf.h).
     `parallel=True` (inside an initialised torch.distributed job, one process per GPU): the
     nrun x len(ranks) independent factorizations are spread over the ranks (the role of
     Rmpi::mpi.applyLB, R/bayesian.R:263), every rank holds a full copy of the matrix, results are
@@ -339,8 +347,8 @@ def vb_factorize(object, ranks=2, nrun=1, verbose=2, progress_bar=True, initiali
     ga = np.atleast_1d(np.asarray(gamma_a, dtype=np.float64))
     gb = np.atleast_1d(np.asarray(gamma_b, dtype=np.float64))
 
-    if device_init and initializer not in ("random", "svd2"):
-        raise ValueError("device_init applies to the 'random' and 'svd2' initializers")
+    if device_init and initializer not in ("random", "svd", "svd2"):
+        raise ValueError("device_init applies to the 'random', 'svd' and 'svd2' initializers")
     if device_init:
         initializer += "_device"
     common = (ga, gb, initializer, Itmax, hyper_update, Tol, hyper_update_n0, hyper_update_dn,
@@ -544,6 +552,8 @@ def _vb_iterate(eng, irun, mat, ranks, ga, gb, initializer, Itmax, hyper_update,
             eng.init_random(rank, hyper, seed * 100003 + 1000 * rank + irun, cell_offset=c0)
         elif initializer == "svd2_device":                      # :150-159 where the matrix lives
             eng.init_svd2(rank, hyper, seed * 100003 + 1000 * rank + irun, cell_offset=c0)
+        elif initializer == "svd_device":                       # :116-149, pairs oriented
+            eng.init_svd(rank, seed * 100003 + 1000 * rank + irun, cell_offset=c0)
         else:
             w0, h0 = vb_init(nrow, ncol, mat, rank, hyper, initializer,
                              seed * 100003 + 1000 * rank + irun)

@@ -1,6 +1,8 @@
 // vb_init(initializer = 'svd2') on the device (R/bayesian.R:150-159):
 //   s <- irlba(mat, rank);  w <- abs(s$u);  h <- abs(diag(s$d) %*% t(s$v));
 //   scale <- bh / mean(h);  h <- h * scale;  w <- w / scale
+// and vb_init(initializer = 'svd') (R/bayesian.R:116-149), the NNDSVD of Boutsidis & Gallopoulos
+// (2008) on the same truncated SVD, every pair (u_k, v_k), k >= 1, oriented first (vbnmf.h).
 // The truncated SVD is a randomized range finder on the CSC matrix already resident on the GPU
 // (Halko, Martinsson & Tropp 2011, alg. 4.4 + 5.1): Y = X Omega with k = rank + oversampling
 // Gaussian columns, a few power iterations Y <- X (X^T Q) with Cholesky-QR re-orthonormalisation
@@ -153,6 +155,51 @@ svd_store_kernel(int64_t rows, int r, int rs, const int32_t *__restrict__ dev,
     const int64_t row = t / r;
     const int c = (int)(t - row * r);
     const double v = fabs(A[t]) * f;
+    const int64_t d = dev[row];
+    panel[panel_ofs(d, c, rs, tsplit)] = v;
+    mirror[d * rs + c] = v;
+}
+
+// part[b][2c] / part[b][2c + 1] = sum over the rows of CTA b of A[row][c]^2 where A[row][c] > 0 /
+// where A[row][c] < 0 (A rows x r, r <= kBlock); CTA b takes rows b*per .. b*per + per - 1, then
+// steps by gridDim.x*per; the per rows are added in order: the sums do not depend on timing
+__global__ void __launch_bounds__(kBlock)
+signed_sq_part_kernel(int64_t rows, int r, const double *__restrict__ A, double *__restrict__ part) {
+    __shared__ double sp[kBlock], sn[kBlock];
+    const int per = kBlock / r, lr = threadIdx.x / r, c = threadIdx.x - lr * r;
+    double p = 0.0, q = 0.0;
+    if (lr < per)
+        for (int64_t row = (int64_t)blockIdx.x * per + lr; row < rows; row += (int64_t)gridDim.x * per) {
+            const double a = A[row * r + c];
+            if (a > 0.0) p = fma(a, a, p);
+            else q = fma(a, a, q);
+        }
+    sp[threadIdx.x] = p;
+    sn[threadIdx.x] = q;
+    __syncthreads();
+    if (threadIdx.x < r) {
+        for (int t = 1; t < per; t++) {
+            p += sp[t * r + threadIdx.x];
+            q += sn[t * r + threadIdx.x];
+        }
+        part[(size_t)blockIdx.x * 2 * r + 2 * threadIdx.x] = p;
+        part[(size_t)blockIdx.x * 2 * r + 2 * threadIdx.x + 1] = q;
+    }
+}
+
+// panel[dev[row]][c] = f[c] * max(s[c] * A[row][c], 0) for 1 <= c < r and f[0] * s[0] * A[row][0],
+// into the l panel and its mirror as svd_store_kernel: the 'svd' factors (f, s: r values each)
+__global__ void __launch_bounds__(kBlock)
+svd_pos_store_kernel(int64_t rows, int r, int rs, const int32_t *__restrict__ dev,
+                     const double *__restrict__ A, const double *__restrict__ f,
+                     const double *__restrict__ s, double *__restrict__ panel,
+                     double *__restrict__ mirror, int tsplit) {
+    const int64_t t = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+    if (t >= rows * r) return;
+    const int64_t row = t / r;
+    const int c = (int)(t - row * r);
+    const double a = s[c] * A[t];
+    const double v = f[c] * (c == 0 ? a : fmax(a, 0.0));
     const int64_t d = dev[row];
     panel[panel_ofs(d, c, rs, tsplit)] = v;
     mirror[d * rs + c] = v;

@@ -1194,7 +1194,10 @@ int init_common(H *h, int device) {
 
 }  // namespace
 
-// ---- vb_init(initializer = 'svd2') on the device (svd_init.cuh) ------------------------------------
+// ---- vb_init(initializer = 'svd2' and 'svd') on the device (svd_init.cuh) ---------------------------
+extern "C" {
+static int initial_ehsum(H *h);
+}
 namespace {
 
 template <typename VT>
@@ -1254,27 +1257,28 @@ struct SvdCtx {
     }
 };
 
-template <typename VT>
-int init_svd2_t(H *h, int r, const double hyper[4], uint64_t seed, int64_t cell_offset, int k,
-                int power_iters, bool *ok) {
-    const Layout *L = h->L;
+// Rank-r truncated SVD of the resident matrix from a sketch of k columns, then
+// finish(U, T, ok) while the buffers live: U (n x r) and T = V diag(d) (m x r, the local cells),
+// both row-major on the device, components in decreasing order of d.  *ok = false when a Gram
+// matrix is not positive definite (the sketch is rank-deficient).
+template <typename VT, typename Finish>
+int truncated_svd_t(H *h, int r, uint64_t seed, int64_t cell_offset, int k, int power_iters,
+                    bool *ok, Finish &&finish) {
     const int64_t n = h->n, m = h->m, big = std::max(n, m);
     SvdCtx<VT> c;
     c.h = h; c.k = k;
     c.gblocks = h->num_sms * 2;
-    double *d_Y = nullptr, *d_Z = nullptr, *d_sum = nullptr, *d_spart = nullptr;
+    double *d_Y = nullptr, *d_Z = nullptr;
     CK(vmalloc(h, &d_Y, (size_t)n * k * 8));
     CK(vmalloc(h, &d_Z, (size_t)m * k * 8));
     CK(vmalloc(h, &c.d_tmp, (size_t)big * k * 8));
     CK(vmalloc(h, &c.d_part, (size_t)c.gblocks * k * k * 8));
     CK(vmalloc(h, &c.d_G, (size_t)k * k * 8));
     CK(vmalloc(h, &c.d_M, (size_t)k * k * 8));
-    CK(vmalloc(h, &d_sum, 8));
-    CK(vmalloc(h, &d_spart, (size_t)h->num_sms * 4 * 8));
     struct Free {
-        cudaStream_t s; double *p[8];
+        cudaStream_t s; double *p[6];
         ~Free() { for (double *q : p) vfree(s, q); }
-    } fr{h->stream, {d_Y, d_Z, c.d_tmp, c.d_part, c.d_G, c.d_M, d_sum, d_spart}};
+    } fr{h->stream, {d_Y, d_Z, c.d_tmp, c.d_part, c.d_G, c.d_M}};
     int rc;
     vb::gauss_fill_kernel<<<cdiv(m * k, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         m, k, (unsigned long long)seed, cell_offset, d_Z);
@@ -1308,12 +1312,25 @@ int init_svd2_t(H *h, int r, const double hyper[4], uint64_t seed, int64_t cell_
     // U = Q U_B (n x r), T = B^T U_B = (diag(d) V^T)^T (m x r)
     double *d_U = c.d_tmp;
     if ((rc = c.right_mult(d_Y, n, M1, r, d_U))) return rc;
-    double *d_T = d_Y;                                    // reuse: n*k >= ... not guaranteed, so:
-    double *d_T2 = nullptr;
-    CK(vmalloc(h, &d_T2, (size_t)m * r * 8));
-    d_T = d_T2;
-    struct Free2 { cudaStream_t s; double *p; ~Free2() { vfree(s, p); } } fr2{h->stream, d_T2};
+    double *d_T = nullptr;
+    CK(vmalloc(h, &d_T, (size_t)m * r * 8));
+    struct Free2 { cudaStream_t s; double *p; ~Free2() { vfree(s, p); } } fr2{h->stream, d_T};
     if ((rc = c.right_mult(d_Z, m, M1, r, d_T))) return rc;
+    return finish(d_U, d_T, ok);
+}
+
+// 'svd2' from U and T: w = |U| / scale, h = |T| * scale, scale = bh / mean(|T|) over all cells
+int svd2_finish(H *h, int r, double bh, const double *d_U, const double *d_T, bool *ok) {
+    const Layout *L = h->L;
+    const int64_t n = h->n, m = h->m;
+    double *d_sum = nullptr, *d_spart = nullptr;
+    CK(vmalloc(h, &d_sum, 8));
+    CK(vmalloc(h, &d_spart, (size_t)h->num_sms * 4 * 8));
+    struct Free {
+        cudaStream_t s; double *p[2];
+        ~Free() { for (double *q : p) vfree(s, q); }
+    } fr{h->stream, {d_sum, d_spart}};
+    int rc;
     // scale <- bh / mean(h), h = |T|^T over all cells
     vb::abs_sum_kernel<<<h->num_sms * 4, vb::kBlock, 0, h->stream>>>(m * r, d_T, d_spart, d_sum,
                                                                    h->d_counters + 5);
@@ -1324,20 +1341,101 @@ int init_svd2_t(H *h, int r, const double hyper[4], uint64_t seed, int64_t cell_
     CK(cudaStreamSynchronize(h->stream));
     const double mean_h = sum / ((double)r * (double)h->m_global);
     if (!(mean_h > 0.0) || !std::isfinite(mean_h)) { *ok = false; return 0; }
-    const double scale = hyper[3] / mean_h;              // :156
-    const int rs = h->rs;
-    const size_t gr = (size_t)L->NG * rs * 8, cr = (size_t)L->NC * rs * 8;
+    const double scale = bh / mean_h;                    // :156
+    vb::svd_store_kernel<<<cdiv(n * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
+        n, r, h->rs, L->d_gene_dev, d_U, 1.0 / scale, h->d_lw, h->d_alw, h->tsplit);   // w / scale
+    vb::svd_store_kernel<<<cdiv(m * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
+        m, r, h->rs, L->d_cell_dev, d_T, scale, h->d_lh, h->d_alh, h->tsplit);         // h * scale
+    h->launches += 2;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// 'svd' from U and T (the rule of vbnmf_init_svd in vbnmf.h).  With v_k = T_k / d_k:
+//   k = 0:  w = sgn' sqrt(d_0) u_0, h = sgn sqrt(d_0) v_0 = sgn T_0 / sqrt(d_0), sgn = sign(u_00),
+//           sgn' = -1 if sgn < 0 else 1 (:120-124, literally);
+//   k >= 1: P = |u+| |v+|, N = |u-| |v-|; s = -1 if N > P else 1; with the oriented pair
+//           w = sqrt(d P) u+ / |u+| = sqrt(|T+| / |u+|) u+, h = sqrt(d P) v+ / |v+| = sqrt(|u+| / |T+|) T+
+//           (d_k cancels: |v+| = |T+| / d_k).
+// Only the 4r sums of squares, u_00 and the 4r factors cross the bus.
+int svd_finish(H *h, int r, const double *d_U, const double *d_T, bool *ok) {
+    const Layout *L = h->L;
+    const int64_t n = h->n, m = h->m;
+    const int nb = h->num_sms * 2;
+    double *d_part = nullptr, *d_sq = nullptr, *d_fs = nullptr;
+    CK(vmalloc(h, &d_part, (size_t)nb * 2 * r * 8));
+    CK(vmalloc(h, &d_sq, (size_t)4 * r * 8));           // U: (pos, neg) x r, then T: (pos, neg) x r
+    CK(vmalloc(h, &d_fs, (size_t)4 * r * 8));           // f_w, s_w, f_h, s_h
+    struct Free {
+        cudaStream_t s; double *p[3];
+        ~Free() { for (double *q : p) vfree(s, q); }
+    } fr{h->stream, {d_part, d_sq, d_fs}};
+    int rc;
+    vb::signed_sq_part_kernel<<<nb, vb::kBlock, 0, h->stream>>>(n, r, d_U, d_part);
+    vb::gram_sum_kernel<<<1, vb::kBlock, 0, h->stream>>>(nb, 2 * r, d_part, d_sq);
+    vb::signed_sq_part_kernel<<<nb, vb::kBlock, 0, h->stream>>>(m, r, d_T, d_part);
+    vb::gram_sum_kernel<<<1, vb::kBlock, 0, h->stream>>>(nb, 2 * r, d_part, d_sq + 2 * r);
+    h->launches += 4;
+    if ((rc = allreduce(h, d_sq + 2 * r, 2 * r))) return rc;   // T: sums over all cells
+    std::vector<double> sq((size_t)4 * r), fs((size_t)4 * r);
+    double u00 = 0.0;
+    CK(cudaMemcpyAsync(sq.data(), d_sq, (size_t)4 * r * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&u00, d_U, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    double *fw = fs.data(), *sw = fw + r, *fh = sw + r, *sh = fh + r;
+    const double d0 = std::sqrt(sq[2 * r] + sq[2 * r + 1]);   // |T_0| = d_0
+    const double sgn = u00 > 0.0 ? 1.0 : (u00 < 0.0 ? -1.0 : 0.0);
+    fw[0] = std::sqrt(d0);
+    sw[0] = sgn < 0.0 ? -1.0 : 1.0;
+    fh[0] = 1.0 / std::sqrt(d0);
+    sh[0] = sgn;
+    if (!(d0 > 0.0) || !std::isfinite(d0)) { *ok = false; return 0; }
+    for (int q = 1; q < r; q++) {
+        const double up = std::sqrt(sq[2 * q]), un = std::sqrt(sq[2 * q + 1]);
+        const double tp = std::sqrt(sq[2 * r + 2 * q]), tn = std::sqrt(sq[2 * r + 2 * q + 1]);
+        const bool flip = un * tn > up * tp;
+        const double nu = flip ? un : up, nt = flip ? tn : tp;
+        // P = N = 0 cannot happen for a nonnegative matrix and d_k > 0 (u^T X v would be <= 0)
+        if (!(nu > 0.0 && nt > 0.0) || !std::isfinite(nu * nt)) { *ok = false; return 0; }
+        fw[q] = std::sqrt(nt / nu);
+        fh[q] = std::sqrt(nu / nt);
+        sw[q] = sh[q] = flip ? -1.0 : 1.0;
+    }
+    CK(cudaMemcpyAsync(d_fs, fs.data(), (size_t)4 * r * 8, cudaMemcpyHostToDevice, h->stream));
+    vb::svd_pos_store_kernel<<<cdiv(n * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
+        n, r, h->rs, L->d_gene_dev, d_U, d_fs, d_fs + r, h->d_lw, h->d_alw, h->tsplit);
+    vb::svd_pos_store_kernel<<<cdiv(m * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
+        m, r, h->rs, L->d_cell_dev, d_T, d_fs + 2 * r, d_fs + 3 * r, h->d_lh, h->d_alh, h->tsplit);
+    h->launches += 2;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// The two SVD initialisers: zeroed panels, the truncated SVD with oversampling 20 (a rank-deficient
+// sketch, where Cholesky fails, falls back to none) and at most 60 subspace iterations, then
+// finish(U, T, ok), the mirrors and rowSums(eh).
+template <typename Finish>
+int svd_init(H *h, int r, uint64_t seed, int64_t cell_offset, const char *name, Finish finish) {
+    int rc;
+    if ((rc = alloc_panels(h, r))) return rc;
+    const Layout *L = h->L;
+    const size_t gr = (size_t)L->NG * h->rs * 8, cr = (size_t)L->NC * h->rs * 8;
     CK(cudaMemsetAsync(h->d_lw, 0, gr, h->stream));
     CK(cudaMemsetAsync(h->d_alw, 0, gr, h->stream));
     CK(cudaMemsetAsync(h->d_lh, 0, cr, h->stream));
     CK(cudaMemsetAsync(h->d_alh, 0, cr, h->stream));
-    vb::svd_store_kernel<<<cdiv(n * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
-        n, r, rs, L->d_gene_dev, d_U, 1.0 / scale, h->d_lw, h->d_alw, h->tsplit);   // w / scale
-    vb::svd_store_kernel<<<cdiv(m * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
-        m, r, rs, L->d_cell_dev, d_T, scale, h->d_lh, h->d_alh, h->tsplit);         // h * scale
-    h->launches += 2;
-    CK(cudaGetLastError());
-    return 0;
+    const int kmax = (int)std::min<int64_t>(std::min(h->n, h->m_global), vb::kSvdMaxK);
+    for (int k : {std::min(r + 20, kmax), r}) {
+        bool ok = true;
+        rc = h->val_float ? truncated_svd_t<float>(h, r, seed, cell_offset, k, 60, &ok, finish)
+                          : truncated_svd_t<double>(h, r, seed, cell_offset, k, 60, &ok, finish);
+        if (rc) return rc;
+        if (ok) {
+            if ((rc = refresh_mirrors(h))) return rc;
+            return initial_ehsum(h);
+        }
+    }
+    return fail(h, VBNMF_ERR_ARG, std::string(name) + " initializer: the matrix has numerical rank below `rank`");
 }
 
 }  // namespace
@@ -2370,22 +2468,22 @@ int vbnmf_init_svd2(vbnmf_handle *h, int r, const double hyper[4], uint64_t seed
     if (r > std::min(h->n, h->m_global)) return fail(h, VBNMF_ERR_ARG, "rank exceeds min(n, m)");
     CK(cudaSetDevice(h->device));
     StageTimer tm("vbnmf_init_svd2(total)");
-    int rc;
-    if ((rc = alloc_panels(h, r))) return rc;
-    const int kmax = (int)std::min<int64_t>(std::min(h->n, h->m_global), vb::kSvdMaxK);
-    // oversampling 20, at most 60 subspace iterations; a rank-deficient sketch (Cholesky fails)
-    // falls back to no oversampling
-    for (int k : {std::min(r + 20, kmax), r}) {
-        bool ok = true;
-        rc = h->val_float ? init_svd2_t<float>(h, r, hyper, seed, cell_offset, k, 60, &ok)
-                          : init_svd2_t<double>(h, r, hyper, seed, cell_offset, k, 60, &ok);
-        if (rc) return rc;
-        if (ok) {
-            if ((rc = refresh_mirrors(h))) return rc;
-            return initial_ehsum(h);
-        }
-    }
-    return fail(h, VBNMF_ERR_ARG, "svd2 initializer: the matrix has numerical rank below `rank`");
+    const double bh = hyper[3];
+    return svd_init(h, r, seed, cell_offset, "svd2", [h, r, bh](const double *U, const double *T, bool *ok) {
+        return svd2_finish(h, r, bh, U, T, ok);
+    });
+}
+
+int vbnmf_init_svd(vbnmf_handle *h, int r, uint64_t seed, int64_t cell_offset) {
+    if (!h) return VBNMF_ERR_ARG;
+    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    if (cell_offset < 0) return fail(h, VBNMF_ERR_ARG, "cell_offset must be >= 0");
+    if (r > std::min(h->n, h->m_global)) return fail(h, VBNMF_ERR_ARG, "rank exceeds min(n, m)");
+    CK(cudaSetDevice(h->device));
+    StageTimer tm("vbnmf_init_svd(total)");
+    return svd_init(h, r, seed, cell_offset, "svd", [h, r](const double *U, const double *T, bool *ok) {
+        return svd_finish(h, r, U, T, ok);
+    });
 }
 
 int vbnmf_step(vbnmf_handle *h, const double hyper[4], double fudge, double *lkh) {

@@ -265,6 +265,13 @@ class Engine:
                                           int(cell_offset)))
         self.r = int(rank)
 
+    def init_svd(self, rank, seed=1, cell_offset=0):
+        """vb_init(initializer='svd') (R/bayesian.R:116-149) computed on the device from the same
+        truncated SVD as init_svd2, each pair of singular vectors k >= 1 oriented first (see
+        vbnmf_init_svd in include/vbnmf.h; synth.device_svd_init_reference restates it)."""
+        self._ck(self.lib.vbnmf_init_svd(self.handle, int(rank), int(seed), int(cell_offset)))
+        self.r = int(rank)
+
     def get_state(self, which=("lw", "lh", "ew", "eh", "dw", "dh")):
         r = self.r
         out = {}

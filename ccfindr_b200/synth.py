@@ -218,6 +218,27 @@ def device_random_init_reference(nrow, ncol, rank, hyper, seed, cell_offset=0):
     return w, h
 
 
+def orient_svd_pairs(u, v):
+    """The orientation Engine.init_svd applies before the 'svd' formula: for every k >= 1,
+    (u_k, v_k) -> (-u_k, -v_k) when |u_k-| |v_k-| > |u_k+| |v_k+| (norms of the negative and
+    positive parts); ties and component 0 are kept.  Returns new arrays."""
+    u, v = np.array(u, dtype=np.float64), np.array(v, dtype=np.float64)
+    for k in range(1, u.shape[1]):
+        P = np.linalg.norm(np.maximum(u[:, k], 0)) * np.linalg.norm(np.maximum(v[:, k], 0))
+        N = np.linalg.norm(np.minimum(u[:, k], 0)) * np.linalg.norm(np.minimum(v[:, k], 0))
+        if N > P:
+            u[:, k], v[:, k] = -u[:, k], -v[:, k]
+    return u, v
+
+
+def device_svd_init_reference(u, d, v):
+    """What Engine.init_svd puts on the device for the truncated SVD (u n x r, d, v m x r):
+    orient_svd_pairs, then the reference formula (api.svd_init_from).  Returns w, h."""
+    from .api import svd_init_from
+    u, v = orient_svd_pairs(u, v)
+    return svd_init_from(u, np.asarray(d, dtype=np.float64), v)
+
+
 # ---- CPU restatement of the on-device column shuffle (csrc/shuffle.cuh) ----------------------
 _GOLDEN = np.uint64(0x9E3779B97F4A7C15)
 

@@ -14,7 +14,8 @@
  *   uniform-column test, R/bayesian.R:368-369                          vbnmf_uniform_columns
  *   cluster_id(): apply(h,2,which.max), R/utils.R:903-909              vbnmf_cluster_id
  *   nmf_updateR() + likelihood() loop, R/factorize.R:189-212           mlnmf_run, mlnmf_run2 (both criteria)
- *   vb_init(): 'random', 'svd2', R/bayesian.R:111-115,150-159          vbnmf_init_random, vbnmf_init_svd2
+ *   vb_init(): 'random', 'svd', 'svd2', R/bayesian.R:111-149,150-159   vbnmf_init_random, vbnmf_init_svd,
+ *                                                                      vbnmf_init_svd2
  *   read_10x(): readMM + as(., 'dgCMatrix'), R/utils.R:34               vbnmf_create_from_mtx
  *   filter_cells(): colSums(counts), R/utils.R:78-95                   vbnmf_qc_stats +
  *                                                                      vbnmf_create_subset
@@ -213,6 +214,22 @@ VBNMF_API int vbnmf_init_random(vbnmf_handle *h, int r, const double hyper[4], u
  * depend on the sharding.  hyper = {aw, bw, ah, bh} (only bh is used, as in the reference). */
 VBNMF_API int vbnmf_init_svd2(vbnmf_handle *h, int r, const double hyper[4], uint64_t seed,
                               int64_t cell_offset);
+
+/* vb_init(initializer = 'svd') (R/bayesian.R:116-149) on the device, from the same truncated SVD
+ * as vbnmf_init_svd2 (same seed, same cell_offset rule), U = (u_k) n x r, d, V = (v_k) m x r:
+ *   component 0, as the reference: w_0 = sqrt(d_0) u_0, h_0 = sqrt(d_0) v_0, both multiplied by
+ *     sgn = sign(w_00) (gene 0), and w_0 kept unflipped with h_0 = 0 when w_00 is exactly 0;
+ *   components k >= 1, NNDSVD (Boutsidis & Gallopoulos 2008): P = |u_k+| |v_k+|, N = |u_k-| |v_k-|
+ *     (norms of the positive and negative parts over all genes and all cells); when N > P the
+ *     pair becomes (-u_k, -v_k) (ties keep it); then w_k = sqrt(d_k P) u_k+ / |u_k+|,
+ *     h_k = sqrt(d_k P) v_k+ / |v_k+|.
+ * The reference computes its negative-part norms from the positive parts (:136-137), so it always
+ * takes the positive parts of whatever signs irlba returned, and gives NaN when both are <= 0.
+ * Orienting each pair first makes the result independent of the SVD's sign choice, equal to the
+ * reference whenever irlba returned the dominant orientation, and finite: for a nonnegative matrix
+ * and d_k > 0, P = N = 0 would force u_k^T X v_k <= 0.  lw = ew = w, lh = eh = h; no hyper-
+ * parameter enters.  Numerical rank below r: VBNMF_ERR_ARG, as vbnmf_init_svd2. */
+VBNMF_API int vbnmf_init_svd(vbnmf_handle *h, int r, uint64_t seed, int64_t cell_offset);
 
 /* One call of vbnmf_update (src/vbnmf_update.cpp:16-102): state <- update(state); *lkh = bound. */
 VBNMF_API int vbnmf_step(vbnmf_handle *h, const double hyper[4], double fudge, double *lkh);

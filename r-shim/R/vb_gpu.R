@@ -50,10 +50,19 @@ vb_iterate_gpu <- function(irun, bundle) {
     if (rank > min(nrow, ncol)) stop('Rank exceeded min(nrow,ncol)')
     hyper <- list(aw = bundle$gamma.a[1], ah = bundle$gamma.a[length(bundle$gamma.a)],
                   bw = bundle$gamma.b[1], bh = bundle$gamma.b[length(bundle$gamma.b)])
-    if (identical(bundle$initializer, 'random') && isTRUE(bundle$device.init)) {
-      # vb_init 'random' drawn on the GPU: no nrow x rank / rank x ncol matrices cross the bus
-      .Call(C_vbnmf_init_random, h, as.integer(rank),
-            c(hyper$aw, hyper$bw, hyper$ah, hyper$bh), as.numeric(bundle$seed + irun))
+    device.init <- isTRUE(bundle$device.init) && bundle$initializer %in% c('random', 'svd2', 'svd')
+    if (device.init) {
+      # vb_init drawn / computed on the GPU: no nrow x rank / rank x ncol matrices cross the bus
+      # ('svd' orients each pair of singular vectors k >= 1 first, include/vbnmf.h)
+      seed <- as.numeric(bundle$seed + irun)
+      if (bundle$initializer == 'random')
+        .Call(C_vbnmf_init_random, h, as.integer(rank),
+              c(hyper$aw, hyper$bw, hyper$ah, hyper$bh), seed)
+      else if (bundle$initializer == 'svd2')
+        .Call(C_vbnmf_init_svd2, h, as.integer(rank),
+              c(hyper$aw, hyper$bw, hyper$ah, hyper$bh), seed)
+      else
+        .Call(C_vbnmf_init_svd, h, as.integer(rank), seed)
     } else {
       wh <- ccfindR:::vb_init(nrow, ncol, bundle$mat, rank, hyper = hyper,
                               initializer = bundle$initializer)

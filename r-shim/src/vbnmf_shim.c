@@ -67,6 +67,22 @@ SEXP C_vbnmf_init_random(SEXP ptr, SEXP rank, SEXP hyper, SEXP seed) {
     return R_NilValue;
 }
 
+/* vb_init(initializer = 'svd2') computed on the device from the resident matrix
+ * (R/bayesian.R:150-159): randomized truncated SVD keyed by seed.  hyper = c(aw, bw, ah, bh) */
+SEXP C_vbnmf_init_svd2(SEXP ptr, SEXP rank, SEXP hyper, SEXP seed) {
+    vbnmf_handle *h = get_handle(ptr);
+    chk(vbnmf_init_svd2(h, Rf_asInteger(rank), REAL(hyper), (uint64_t)Rf_asReal(seed), 0), h);
+    return R_NilValue;
+}
+
+/* vb_init(initializer = 'svd') computed on the device (R/bayesian.R:116-149), each pair of
+ * singular vectors k >= 1 oriented first (include/vbnmf.h) */
+SEXP C_vbnmf_init_svd(SEXP ptr, SEXP rank, SEXP seed) {
+    vbnmf_handle *h = get_handle(ptr);
+    chk(vbnmf_init_svd(h, Rf_asInteger(rank), (uint64_t)Rf_asReal(seed), 0), h);
+    return R_NilValue;
+}
+
 /* one vbnmf_update (src/vbnmf_update.cpp:16-102); hyper = c(aw, bw, ah, bh) */
 SEXP C_vbnmf_step(SEXP ptr, SEXP hyper, SEXP fudge) {
     vbnmf_handle *h = get_handle(ptr);
@@ -218,6 +234,8 @@ static const R_CallMethodDef CallEntries[] = {
     {"C_vbnmf_destroy", (DL_FUNC)&C_vbnmf_destroy, 1},
     {"C_vbnmf_set_state", (DL_FUNC)&C_vbnmf_set_state, 5},
     {"C_vbnmf_init_random", (DL_FUNC)&C_vbnmf_init_random, 4},
+    {"C_vbnmf_init_svd2", (DL_FUNC)&C_vbnmf_init_svd2, 4},
+    {"C_vbnmf_init_svd", (DL_FUNC)&C_vbnmf_init_svd, 3},
     {"C_vbnmf_step", (DL_FUNC)&C_vbnmf_step, 3},
     {"C_vbnmf_run", (DL_FUNC)&C_vbnmf_run, 8},
     {"C_vbnmf_get_state", (DL_FUNC)&C_vbnmf_get_state, 1},
