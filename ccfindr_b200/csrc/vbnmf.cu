@@ -29,6 +29,7 @@
 #include <atomic>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <numeric>
 #include <mutex>
 #include <string>
@@ -267,6 +268,12 @@ int fail(H *h, int code, const std::string &msg) {
     h->err = msg;
     return code;
 }
+int check_rank(H *h, int r) {
+    return r < 1 || r > kMaxRank ? fail(h, VBNMF_ERR_ARG, "rank must be in 1..64") : 0;
+}
+int check_state(H *h) {
+    return h->d_lw ? 0 : fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+}
 
 // Device memory comes from the stream-ordered pool (cudaMallocAsync) with a high release
 // threshold: the many GB-sized buffers of a handle are recycled instead of being mapped and
@@ -278,6 +285,52 @@ cudaError_t vmalloc(H *h, T **p, size_t bytes) {
 inline void vfree(cudaStream_t s, void *p) {
     if (p) cudaFreeAsync(p, s);
 }
+
+// Scratch device memory of one scope: every buffer taken with get() is freed (stream-ordered)
+// when the scope ends, on every return path.  free() returns one earlier, where keeping it until
+// the end would raise the peak; keep() hands one over to an owner that outlives the scope.
+struct ScopedBufs {
+    H *h;
+    cudaStream_t s;
+    std::vector<void *> p;
+    explicit ScopedBufs(H *h_) : h(h_), s(h_->stream) {}
+    ScopedBufs(const ScopedBufs &) = delete;
+    ScopedBufs &operator=(const ScopedBufs &) = delete;
+    ~ScopedBufs() { for (void *q : p) vfree(s, q); }
+    template <typename T>
+    cudaError_t get(T **x, size_t bytes) {
+        *x = nullptr;
+        const cudaError_t e = vmalloc(h, x, bytes);
+        if (e == cudaSuccess) p.push_back((void *)*x);
+        return e;
+    }
+    void hold(void *x) { p.push_back(x); }  // x (allocated elsewhere) is freed with the scope
+    template <typename T>
+    void free(T *&x) {
+        vfree(s, keep(x));
+        x = nullptr;
+    }
+    template <typename T>
+    T *keep(T *x) {
+        p.erase(std::remove(p.begin(), p.end(), (void *)x), p.end());
+        return x;
+    }
+};
+
+// A device-controlled loop: while this lives the kernels read the stop flag and the hypers from the
+// control block (h->d_ctl); the host-controlled mode is restored on every exit path.
+struct DeviceControl {
+    H *h;
+    explicit DeviceControl(H *h_) : h(h_) { h->ctl = h->d_ctl; }
+    ~DeviceControl() { h->ctl = nullptr; }
+};
+
+// f(float()) or f(double()): the stored type of the counts as a template argument
+template <typename F>
+auto with_val_type(bool as_float, F &&f) {
+    return as_float ? f(float()) : f(double());
+}
+
 inline cudaError_t copy_sync(H *h, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind) {
     cudaError_t e = cudaMemcpyAsync(dst, src, bytes, kind, h->stream);
     return e != cudaSuccess ? e : cudaStreamSynchronize(h->stream);
@@ -370,8 +423,9 @@ int setup_xchg(H *h) {
     }
     // all-gather the 64-byte handles (+ the per-rank failure flag in a 65th... kept separate below)
     const int hb = (int)sizeof(cudaIpcMemHandle_t);
+    ScopedBufs B(h);
     char *d_all = nullptr;
-    CK(vmalloc(h, &d_all, (size_t)hb * (h->nranks + 1)));
+    CK(B.get(&d_all, (size_t)hb * (h->nranks + 1)));
     CK(cudaMemcpyAsync(d_all + (size_t)hb * h->nranks, &mine, hb, cudaMemcpyHostToDevice, h->stream));
     if (g_nccl.AllGather) {
         CKN(g_nccl.AllGather(d_all + (size_t)hb * h->nranks, d_all, (size_t)hb, ncclInt8, h->comm,
@@ -380,7 +434,7 @@ int setup_xchg(H *h) {
     std::vector<cudaIpcMemHandle_t> all((size_t)h->nranks);
     CK(cudaMemcpyAsync(all.data(), d_all, (size_t)hb * h->nranks, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, d_all);
+    B.free(d_all);
     if (!bad) {
         h->xchg_peer[h->rank] = h->d_xchg;
         for (int p = 0; p < h->nranks && !bad; p++) {
@@ -397,13 +451,13 @@ int setup_xchg(H *h) {
     }
     // agree: the sum of the failure flags over the ranks must be zero
     double *d_flag = nullptr, flag = (double)bad;
-    CK(vmalloc(h, &d_flag, 8));
+    CK(B.get(&d_flag, 8));
     CK(cudaMemcpyAsync(d_flag, &flag, 8, cudaMemcpyHostToDevice, h->stream));
     int rc = allreduce(h, d_flag, 1);
     if (rc) return rc;
     CK(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, d_flag);
+    B.free(d_flag);
     if (flag != 0.0) { free_xchg(h); return 0; }
     h->peer_ok = true;
     h->xchg_seq = 0;
@@ -452,12 +506,12 @@ int deal_device(H *h, const unsigned long long *d_cnt, int64_t count, int T, int
     size_t tmp_bytes = 0;
     CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k_in, k_out, v_in, v_out, count, 0, 31,
                                        h->stream));
+    ScopedBufs B(h);
     void *d_tmp = nullptr;
-    CK(vmalloc(h, &d_tmp, tmp_bytes));
+    CK(B.get(&d_tmp, tmp_bytes));
     CK(cub::DeviceRadixSort::SortPairs(d_tmp, tmp_bytes, k_in, k_out, v_in, v_out, count, 0, 31,
                                        h->stream));
     vb::deal_kernel<<<g, vb::kBlock, 0, h->stream>>>(count, S, T, v_out, d_dev);
-    vfree(h->stream, d_tmp);
     return 0;
 }
 
@@ -487,26 +541,30 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
     size_t tmp_bytes = 0;
     CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k_in, k_out, p_in, p_out, nnz, 0, bits,
                                        h->stream));
+    // the segment pointers stay with the 8-byte layout; the packed-16 layout needs them only
+    // until its segments are built
+    ScopedBufs B(h);
     void *d_tmp = nullptr;
-    CK(vmalloc(h, &d_tmp, tmp_bytes));
+    int64_t *d_ptr = nullptr;
+    CK(B.get(&d_tmp, tmp_bytes));
     { StageTimer t1("  radix_sort");
     CK(cub::DeviceRadixSort::SortPairs(d_tmp, tmp_bytes, k_in, k_out, p_in, p_out, nnz, 0, bits,
                                        h->stream)); }
-    CK(vmalloc(h, &P.d_ptr, (size_t)(P.E + 1) * 8));
+    CK(B.get(&d_ptr, (size_t)(P.E + 1) * 8));
     { StageTimer t1("  segment_ptr");
-    vb::segment_ptr_kernel<<<g, vb::kBlock, 0, h->stream>>>(P.E, nnz, k_out, P.d_ptr); }
+    vb::segment_ptr_kernel<<<g, vb::kBlock, 0, h->stream>>>(P.E, nnz, k_out, d_ptr); }
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, d_tmp);
+    B.free(d_tmp);
     if (L->npg > 0) {
         // packed-16 layout: pad every segment to whole quads, scan the quad counts into ptr4
         uint32_t *d_len4 = nullptr;
         uint8_t *d_dead = nullptr;
-        CK(vmalloc(h, &d_len4, (size_t)(P.E + 1) * 4));
-        if (L->kmult == 1) CK(vmalloc(h, &d_dead, (size_t)P.E));
+        CK(B.get(&d_len4, (size_t)(P.E + 1) * 4));
+        if (L->kmult == 1) CK(B.get(&d_dead, (size_t)P.E));
         CK(vmalloc(h, &P.d_ptr4, (size_t)(P.E + 1) * 4));
         const uint32_t *d_words = p_out;  // the sorted payloads are the packed words
         { StageTimer t1("  plan(p16)");
-        vb::plan_p16_kernel<<<g, vb::kBlock, 0, h->stream>>>(P.E, P.d_ptr, d_words, L->npg,
+        vb::plan_p16_kernel<<<g, vb::kBlock, 0, h->stream>>>(P.E, d_ptr, d_words, L->npg,
                                                              L->kmult, L->mode, d_len4, d_dead); }
         // order the segments by decreasing number of steps inside windows of W owners
         // (seg_order_keys_kernel; VBNMF_SEG_WINDOW: experiments, 0 = owner order)
@@ -514,14 +572,14 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
         if (const char *wenv = getenv("VBNMF_SEG_WINDOW")) W = atoi(wenv);
         uint32_t *d_len4p = nullptr, *d_okey = nullptr, *d_oval = nullptr;
         uint8_t *d_deadp = nullptr;
-        CK(vmalloc(h, &d_len4p, (size_t)(P.E + 1) * 4));
-        if (d_dead) CK(vmalloc(h, &d_deadp, (size_t)P.E));
+        CK(B.get(&d_len4p, (size_t)(P.E + 1) * 4));
+        if (d_dead) CK(B.get(&d_deadp, (size_t)P.E));
         CK(vmalloc(h, &P.d_seg, (size_t)P.E * 4));
         { StageTimer t1("  order segments");
         const int ge = cdiv(P.E + 1, vb::kBlock);
         void *d_otmp = nullptr;
         if (W > 0) {
-            CK(vmalloc(h, &d_okey, (size_t)P.E * 4 * 4));  // keys in/out, values in/out
+            CK(B.get(&d_okey, (size_t)P.E * 4 * 4));  // keys in/out, values in/out
             d_oval = d_okey + 2 * P.E;
             vb::seg_order_keys_kernel<<<ge, vb::kBlock, 0, h->stream>>>(P.E, NO, W, d_len4, d_dead,
                                                                         L->npg, d_okey, d_oval);
@@ -533,30 +591,30 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
             size_t ob = 0;
             CK(cub::DeviceRadixSort::SortPairs(nullptr, ob, d_okey, d_okey + P.E, d_oval,
                                                d_oval + P.E, P.E, 0, obits, h->stream));
-            CK(vmalloc(h, &d_otmp, ob));
+            CK(B.get(&d_otmp, ob));
             CK(cub::DeviceRadixSort::SortPairs(d_otmp, ob, d_okey, d_okey + P.E, d_oval,
                                                d_oval + P.E, P.E, 0, obits, h->stream));
         }
         vb::seg_permute_kernel<<<ge, vb::kBlock, 0, h->stream>>>(
             P.E, NO, W > 0 ? d_oval + P.E : nullptr, d_len4, d_dead, d_len4p, d_deadp, P.d_seg);
-        vfree(h->stream, d_otmp); }
+        B.free(d_otmp); }
         size_t scan_bytes = 0;
         CK(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_len4p, P.d_ptr4, P.E + 1, h->stream));
         void *d_scan = nullptr;
-        CK(vmalloc(h, &d_scan, scan_bytes));
+        CK(B.get(&d_scan, scan_bytes));
         CK(cub::DeviceScan::ExclusiveSum(d_scan, scan_bytes, d_len4p, P.d_ptr4, P.E + 1, h->stream));
         if (2 * nnz + 32 * P.E >= ((int64_t)1 << 34))
             return fail(h, VBNMF_ERR_ARG, "matrix too large for 32-bit quad pointers on one GPU");
         uint32_t quads = 0;
         CK(cudaMemcpyAsync(&quads, P.d_ptr4 + P.E, 4, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
-        vfree(h->stream, d_len4); vfree(h->stream, d_scan);
-        vfree(h->stream, d_len4p); vfree(h->stream, d_okey);
+        B.free(d_len4); B.free(d_scan);
+        B.free(d_len4p); B.free(d_okey);
         CK(vmalloc(h, &P.d_ent, (size_t)quads * 16));
         P.nent = (int64_t)quads * 4;
         { StageTimer t1("  build_segments(p16)");
         vb::build_segments_p16_kernel<<<g, vb::kBlock, 0, h->stream>>>(
-            P.E, NO, P.d_ptr, P.d_ptr4, P.d_seg, d_words, L->npg, L->kmult, L->mode,
+            P.E, NO, d_ptr, P.d_ptr4, P.d_seg, d_words, L->npg, L->kmult, L->mode,
             cols_pass ? h->n : h->m, cols_pass ? L->Sg : L->Sc, (uint32_t *)P.d_ent); }
         CK(vmalloc(h, &P.d_split, (size_t)(L->grid + 1) * 8));
         // per-segment overhead in quads (VBNMF_SPLIT_KAPPA: tuning)
@@ -569,9 +627,6 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
                                                                                     P.d_ptr4);
         CK(cudaStreamSynchronize(h->stream));
         CK(cudaGetLastError());
-        vfree(h->stream, d_dead); vfree(h->stream, d_deadp);
-        vfree(h->stream, P.d_ptr);
-        P.d_ptr = nullptr;
         return 0;
     }
     P.nent = nnz;
@@ -583,13 +638,14 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
     }
     { StageTimer t1("  build_segments");
     vb::build_segments_kernel<VT><<<g, vb::kBlock, 0, h->stream>>>(
-        P.E, P.d_ptr, p_out, h->d_rowidx, d_colof, L->d_gene_dev, L->d_cell_dev,
+        P.E, d_ptr, p_out, h->d_rowidx, d_colof, L->d_gene_dev, L->d_cell_dev,
         (const VT *)h->d_val, L->T, cols_pass, P.d_idx, (VT *)P.d_val, (int2 *)P.d_ent); }
     CK(vmalloc(h, &P.d_split, (size_t)(L->grid + 1) * 8));
-    vb::split_kernel<<<cdiv(L->grid + 1, 128), 128, 0, h->stream>>>(L->grid, P.E, nnz, P.d_ptr,
+    vb::split_kernel<<<cdiv(L->grid + 1, 128), 128, 0, h->stream>>>(L->grid, P.E, nnz, d_ptr,
                                                                    P.d_split);
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
+    P.d_ptr = B.keep(d_ptr);
     return 0;
 }
 
@@ -623,11 +679,13 @@ int get_layout(H *h, int T, int npg, int kmult, int mode, Layout **out) {
         // one arena: [colof | 4 sort buffers], nnz 32-bit words each (also the scratch of the
         // two small sorts that renumber the genes and the cells)
         const int64_t words = std::max<int64_t>(h->nnz * 5, 4 * std::max(h->n, h->m));
+        ScopedBufs B(h);
         uint32_t *arena = h->d_arena;
         const bool have_colof = arena && h->colof_in_arena;
         h->d_arena = nullptr;
         h->colof_in_arena = false;
-        if (!arena) CK(vmalloc(h, &arena, (size_t)words * 4));
+        if (arena) B.hold(arena);
+        else CK(B.get(&arena, (size_t)words * 4));
         int32_t *d_colof = (int32_t *)arena;
         uint32_t *scratch = arena + h->nnz;
         int rc = 0;
@@ -636,26 +694,25 @@ int get_layout(H *h, int T, int npg, int kmult, int mode, Layout **out) {
         uint32_t *dscr = scratch;
         uint32_t *own = nullptr;
         if (4 * std::max(h->n, h->m) > 4 * h->nnz) {
-            CK(vmalloc(h, &own, (size_t)4 * std::max(h->n, h->m) * 4));
+            CK(B.get(&own, (size_t)4 * std::max(h->n, h->m) * 4));
             dscr = own;
         }
         rc = deal_device(h, h->d_cnt, h->n, T, L->Sg, L->d_gene_dev, dscr);
         if (!rc) rc = deal_device(h, h->d_cnt + h->n, h->m, T, L->Sc, L->d_cell_dev, dscr);
-        vfree(h->stream, own); }
-        if (!rc && !have_colof) {
-            StageTimer t1("  expand_cols");
-            if (h->val_float) launch_expand_cols<float>(h, d_colof, nullptr, nullptr);
-            else launch_expand_cols<double>(h, d_colof, nullptr, nullptr);
-        }
-        if (!rc)
-            rc = h->val_float ? build_pass<float>(h, L, true, d_colof, scratch)
-                              : build_pass<double>(h, L, true, d_colof, scratch);
-        if (!rc)
-            rc = h->val_float ? build_pass<float>(h, L, false, d_colof, scratch)
-                              : build_pass<double>(h, L, false, d_colof, scratch);
-        { StageTimer t1("  free(arena)");
-        vfree(h->stream, arena); }
-        return rc;
+        B.free(own); }
+        if (rc) return rc;
+        return with_val_type(h->val_float, [&](auto v) -> int {
+            using VT = decltype(v);
+            if (!have_colof) {
+                StageTimer t1("  expand_cols");
+                launch_expand_cols<VT>(h, d_colof, nullptr, nullptr);
+            }
+            int rc2 = build_pass<VT>(h, L, true, d_colof, scratch);
+            if (!rc2) rc2 = build_pass<VT>(h, L, false, d_colof, scratch);
+            StageTimer t1("  free(arena)");
+            B.free(arena);
+            return rc2;
+        });
     };
     int rc = body();
     if (rc) return bail(rc);
@@ -676,11 +733,12 @@ int scan_matrix_t(H *h) {
     StageTimer tm("scan_matrix");
     const int64_t n = h->n, m = h->m, nnz = h->nnz;
     const int gridK = h->num_sms * 8;
+    ScopedBufs B(h);
     double *d_part = nullptr, *d_out = nullptr;
     unsigned *d_flags = nullptr;  // [bad row index, empty rows, empty cols]
-    CK(vmalloc(h, &d_part, (size_t)gridK * 4 * 8));
-    CK(vmalloc(h, &d_out, 4 * 8));
-    CK(vmalloc(h, &d_flags, 4 * sizeof(unsigned)));
+    CK(B.get(&d_part, (size_t)gridK * 4 * 8));
+    CK(B.get(&d_out, 4 * 8));
+    CK(B.get(&d_flags, 4 * sizeof(unsigned)));
     CK(cudaMemsetAsync(d_flags, 0, 4 * sizeof(unsigned), h->stream));
     vb::count_constants_kernel<VT><<<gridK, vb::kBlock, 0, h->stream>>>(
         nnz, (const VT *)h->d_val, d_part, d_out, h->d_counters + 4);
@@ -690,14 +748,14 @@ int scan_matrix_t(H *h) {
     // the column of every entry goes into the arena the first layout build sorts in (so that it
     // is expanded once), or into a temporary when the handle has no arena
     int32_t *d_colof = (int32_t *)h->d_arena;
-    if (!d_colof) CK(vmalloc(h, &d_colof, (size_t)nnz * 4));
+    if (!d_colof) CK(B.get(&d_colof, (size_t)nnz * 4));
     CK(vmalloc(h, &h->d_cnt, (size_t)(n + m) * 8));
     CK(cudaMemsetAsync(h->d_cnt, 0, (size_t)(n + m) * 8, h->stream));
     launch_expand_cols<VT>(h, d_colof, h->d_cnt, d_flags);
     h->colof_in_arena = h->d_arena != nullptr;
     // empty genes / cells: counted by the kernel that makes the sort keys (scratch discarded)
     uint32_t *d_scr = nullptr;
-    CK(vmalloc(h, &d_scr, (size_t)2 * std::max(n, m) * 4));
+    CK(B.get(&d_scr, (size_t)2 * std::max(n, m) * 4));
     vb::order_keys_kernel<<<cdiv(n, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         n, h->d_cnt, d_scr, d_scr + std::max(n, m), d_flags + 1);
     vb::order_keys_kernel<<<cdiv(m, vb::kBlock), vb::kBlock, 0, h->stream>>>(
@@ -705,9 +763,6 @@ int scan_matrix_t(H *h) {
     CK(cudaMemcpyAsync(flags, d_flags, sizeof(flags), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
-    vfree(h->stream, d_part); vfree(h->stream, d_out); vfree(h->stream, d_flags);
-    vfree(h->stream, d_scr);
-    if (!h->d_arena) vfree(h->stream, d_colof);
     if (flags[0]) return fail(h, VBNMF_ERR_ARG, "row index out of range");
     if (consts[3] != 0.0)
         return fail(h, VBNMF_ERR_ARG, "counts must be finite and non-negative");
@@ -826,6 +881,18 @@ int alloc_panels(H *h, int r) {
     return setup_xchg(h);
 }
 
+// panels for rank r with all four zeroed (their padding rows and columns must read 0)
+int zeroed_panels(H *h, int r) {
+    int rc = alloc_panels(h, r);
+    if (rc) return rc;
+    const size_t gr = (size_t)h->L->NG * h->rs * 8, cr = (size_t)h->L->NC * h->rs * 8;
+    CK(cudaMemsetAsync(h->d_lw, 0, gr, h->stream));
+    CK(cudaMemsetAsync(h->d_alw, 0, gr, h->stream));
+    CK(cudaMemsetAsync(h->d_lh, 0, cr, h->stream));
+    CK(cudaMemsetAsync(h->d_alh, 0, cr, h->stream));
+    return 0;
+}
+
 // fp32-storage mode: refresh the mirrors from the fp64 panels (after an upload)
 int refresh_mirrors(H *h) {
     if (h->precision != VBNMF_FP32_STORAGE) return 0;
@@ -834,6 +901,38 @@ int refresh_mirrors(H *h) {
     h->launches += 2;
     CK(cudaGetLastError());
     return 0;
+}
+
+// rowSums(eh) of the state just loaded (alh holds eh before the first update), over all shards,
+// into the tail of the reduce buffer and the host vectors
+int initial_ehsum(H *h) {
+    const Layout *L = h->L;
+    const int rs = h->rs, r = h->r;
+    int rc;
+    double *tail = h->d_red + tail_off(h);
+    CK(cudaMemsetAsync(tail, 0, (size_t)(rs + 8) * 8, h->stream));
+    vb::ColsumArgs ca{L->NC, h->d_alh, h->d_partH, tail, h->d_counters + 1, 0};
+    h->tab->colsum(ca, h->stream);
+    h->launches += 1;
+    if ((rc = allreduce(h, tail, rs + 8))) return rc;
+    double s[kMaxRank + 16];  // rs + 8 <= 66 + 8
+    CK(cudaMemcpyAsync(s, tail, (size_t)(rs + 8) * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaGetLastError());
+    for (int k = 0; k < kMaxRank; k++) {
+        h->ehsum[k] = k < r ? s[k] : 0.0;
+        h->ewsum[k] = 0.0;
+        h->bew[k] = h->beh[k] = 1.0;
+    }
+    h->stats_valid = false;
+    h->has_posterior = false;
+    return 0;
+}
+
+// a state just written into the panels: the fp32 mirrors and rowSums(eh)
+int loaded_state(H *h) {
+    int rc = refresh_mirrors(h);
+    return rc ? rc : initial_ehsum(h);
 }
 
 // caller's matrix (n x r column-major for the W side, r x m for the H side) -> device panel(s) in
@@ -921,6 +1020,20 @@ int sweep(H *h) {
     if ((rc = allreduce(h, h->d_red, red_len(h)))) return rc;
     CK(cudaGetLastError());
     h->stats_valid = true;
+    return 0;
+}
+
+// the statistics at the loaded state when they are stale; the H-side sums already in the reduce
+// buffer must survive the pass
+int ensure_stats(H *h) {
+    if (h->stats_valid) return 0;
+    std::vector<double> keep((size_t)h->rs + 8, 0.0);
+    for (int k = 0; k < h->r; k++) keep[k] = h->ehsum[k];
+    int rc = sweep(h);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(h->d_red + tail_off(h), keep.data(), (size_t)h->rs * 8,
+                       cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
@@ -1147,15 +1260,15 @@ int staged_download(H *h, double *dst, const double *d_src, int64_t count) {
 int upload_panel(H *h, double *dst1, double *dst2, const double *src, bool wside, int r) {
     const Layout *L = h->L;
     const int64_t cnt = wside ? h->n : h->m;
+    ScopedBufs B(h);
     double *d_raw = nullptr;
-    CK(vmalloc(h, &d_raw, (size_t)cnt * r * 8));
+    CK(B.get(&d_raw, (size_t)cnt * r * 8));
     bool ok = true;
     int rc = staged_upload(h, d_raw, src, cnt * r, [](double v, double &o) { o = v; return true; },
                            &ok);
-    if (rc) { vfree(h->stream, d_raw); return rc; }
+    if (rc) return rc;
     vb::scatter_panel_kernel<<<cdiv(cnt * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         cnt, r, h->rs, wside ? L->d_gene_dev : L->d_cell_dev, d_raw, wside, dst1, dst2, h->tsplit);
-    vfree(h->stream, d_raw);
     return 0;
 }
 
@@ -1192,13 +1305,72 @@ int init_common(H *h, int device) {
     return 0;
 }
 
-}  // namespace
+// ---- handle creation ---------------------------------------------------------------------------
+// the matrix one GPU holds: int32 row / column indices, fewer than 2^32-1 entries
+int set_dims(H *h, int64_t n, int64_t m, int64_t nnz) {
+    if (n > INT32_MAX || m > INT32_MAX)
+        return fail(h, VBNMF_ERR_ARG, "n and m must be below 2^31 (int32 row/column indices)");
+    if (nnz >= (int64_t)UINT32_MAX) return fail(h, VBNMF_ERR_ARG, "nnz per GPU must be < 2^32-1");
+    h->n = n; h->m = m; h->nnz = nnz;
+    return 0;
+}
+
+// the CSC arrays of h->nnz entries, after the scratch arena of the first layout build (the
+// allocation order vbnmf_handle::d_arena explains); the values follow (store_values)
+int alloc_csc(H *h) {
+    CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(h->nnz * 5, 4 * std::max(h->n, h->m)) * 4));
+    CK(vmalloc(h, &h->d_colptr, (size_t)(h->m + 1) * 8));
+    CK(vmalloc(h, &h->d_rowidx, (size_t)h->nnz * 4));
+    return 0;
+}
+
+// The counts into h->d_val: fp32 when fill(float *dst, bool *exact) finds every one exactly
+// representable, else fp64 through fill(double *dst, bool *exact).  The fp32 buffer is returned
+// before the fp64 one is taken.
+template <typename Fill>
+int store_values(H *h, Fill &&fill) {
+    ScopedBufs B(h);
+    float *dv = nullptr;
+    CK(B.get(&dv, (size_t)h->nnz * 4));
+    bool exact = true;
+    int rc = fill(dv, &exact);
+    if (rc) return rc;
+    h->val_float = exact;
+    if (exact) {
+        h->d_val = B.keep(dv);
+        return 0;
+    }
+    B.free(dv);
+    double *dd = nullptr;
+    CK(B.get(&dd, (size_t)h->nnz * 8));
+    if ((rc = fill(dd, &exact))) return rc;
+    h->d_val = B.keep(dd);
+    return 0;
+}
+
+// Every handle is made here.  check(h) validates the arguments and sets n, m, nnz without touching
+// the device, so that a bad argument is reported as one on a machine without a GPU; fill(h) puts
+// the count matrix on the device, which is then scanned.  On failure the error text is kept for
+// vbnmf_last_error(NULL) and the handle is destroyed.  out = NULL: a temporary handle for a
+// handle-free entry point (no matrix, no scan), destroyed when fill returns.
+template <typename Check, typename Fill>
+int create_handle(vbnmf_handle **out, int device, Check &&check, Fill &&fill) {
+    H *h = new H();
+    int rc = check(h);
+    if (!rc) rc = init_common(h, device);
+    if (!rc) rc = fill(h);
+    if (!rc && out)
+        rc = with_val_type(h->val_float, [h](auto v) { return scan_matrix_t<decltype(v)>(h); });
+    if (rc || !out) {
+        g_create_error = h->err;
+        vbnmf_destroy(h);
+        return rc;
+    }
+    *out = h;
+    return 0;
+}
 
 // ---- vb_init(initializer = 'svd2' and 'svd') on the device (svd_init.cuh) ---------------------------
-extern "C" {
-static int initial_ehsum(H *h);
-}
-namespace {
 
 template <typename VT>
 struct SvdCtx {
@@ -1268,17 +1440,14 @@ int truncated_svd_t(H *h, int r, uint64_t seed, int64_t cell_offset, int k, int 
     SvdCtx<VT> c;
     c.h = h; c.k = k;
     c.gblocks = h->num_sms * 2;
+    ScopedBufs B(h);
     double *d_Y = nullptr, *d_Z = nullptr;
-    CK(vmalloc(h, &d_Y, (size_t)n * k * 8));
-    CK(vmalloc(h, &d_Z, (size_t)m * k * 8));
-    CK(vmalloc(h, &c.d_tmp, (size_t)big * k * 8));
-    CK(vmalloc(h, &c.d_part, (size_t)c.gblocks * k * k * 8));
-    CK(vmalloc(h, &c.d_G, (size_t)k * k * 8));
-    CK(vmalloc(h, &c.d_M, (size_t)k * k * 8));
-    struct Free {
-        cudaStream_t s; double *p[6];
-        ~Free() { for (double *q : p) vfree(s, q); }
-    } fr{h->stream, {d_Y, d_Z, c.d_tmp, c.d_part, c.d_G, c.d_M}};
+    CK(B.get(&d_Y, (size_t)n * k * 8));
+    CK(B.get(&d_Z, (size_t)m * k * 8));
+    CK(B.get(&c.d_tmp, (size_t)big * k * 8));
+    CK(B.get(&c.d_part, (size_t)c.gblocks * k * k * 8));
+    CK(B.get(&c.d_G, (size_t)k * k * 8));
+    CK(B.get(&c.d_M, (size_t)k * k * 8));
     int rc;
     vb::gauss_fill_kernel<<<cdiv(m * k, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         m, k, (unsigned long long)seed, cell_offset, d_Z);
@@ -1313,8 +1482,7 @@ int truncated_svd_t(H *h, int r, uint64_t seed, int64_t cell_offset, int k, int 
     double *d_U = c.d_tmp;
     if ((rc = c.right_mult(d_Y, n, M1, r, d_U))) return rc;
     double *d_T = nullptr;
-    CK(vmalloc(h, &d_T, (size_t)m * r * 8));
-    struct Free2 { cudaStream_t s; double *p; ~Free2() { vfree(s, p); } } fr2{h->stream, d_T};
+    CK(B.get(&d_T, (size_t)m * r * 8));
     if ((rc = c.right_mult(d_Z, m, M1, r, d_T))) return rc;
     return finish(d_U, d_T, ok);
 }
@@ -1323,13 +1491,10 @@ int truncated_svd_t(H *h, int r, uint64_t seed, int64_t cell_offset, int k, int 
 int svd2_finish(H *h, int r, double bh, const double *d_U, const double *d_T, bool *ok) {
     const Layout *L = h->L;
     const int64_t n = h->n, m = h->m;
+    ScopedBufs B(h);
     double *d_sum = nullptr, *d_spart = nullptr;
-    CK(vmalloc(h, &d_sum, 8));
-    CK(vmalloc(h, &d_spart, (size_t)h->num_sms * 4 * 8));
-    struct Free {
-        cudaStream_t s; double *p[2];
-        ~Free() { for (double *q : p) vfree(s, q); }
-    } fr{h->stream, {d_sum, d_spart}};
+    CK(B.get(&d_sum, 8));
+    CK(B.get(&d_spart, (size_t)h->num_sms * 4 * 8));
     int rc;
     // scale <- bh / mean(h), h = |T|^T over all cells
     vb::abs_sum_kernel<<<h->num_sms * 4, vb::kBlock, 0, h->stream>>>(m * r, d_T, d_spart, d_sum,
@@ -1362,14 +1527,11 @@ int svd_finish(H *h, int r, const double *d_U, const double *d_T, bool *ok) {
     const Layout *L = h->L;
     const int64_t n = h->n, m = h->m;
     const int nb = h->num_sms * 2;
+    ScopedBufs B(h);
     double *d_part = nullptr, *d_sq = nullptr, *d_fs = nullptr;
-    CK(vmalloc(h, &d_part, (size_t)nb * 2 * r * 8));
-    CK(vmalloc(h, &d_sq, (size_t)4 * r * 8));           // U: (pos, neg) x r, then T: (pos, neg) x r
-    CK(vmalloc(h, &d_fs, (size_t)4 * r * 8));           // f_w, s_w, f_h, s_h
-    struct Free {
-        cudaStream_t s; double *p[3];
-        ~Free() { for (double *q : p) vfree(s, q); }
-    } fr{h->stream, {d_part, d_sq, d_fs}};
+    CK(B.get(&d_part, (size_t)nb * 2 * r * 8));
+    CK(B.get(&d_sq, (size_t)4 * r * 8));           // U: (pos, neg) x r, then T: (pos, neg) x r
+    CK(B.get(&d_fs, (size_t)4 * r * 8));           // f_w, s_w, f_h, s_h
     int rc;
     vb::signed_sq_part_kernel<<<nb, vb::kBlock, 0, h->stream>>>(n, r, d_U, d_part);
     vb::gram_sum_kernel<<<1, vb::kBlock, 0, h->stream>>>(nb, 2 * r, d_part, d_sq);
@@ -1417,23 +1579,15 @@ int svd_finish(H *h, int r, const double *d_U, const double *d_T, bool *ok) {
 template <typename Finish>
 int svd_init(H *h, int r, uint64_t seed, int64_t cell_offset, const char *name, Finish finish) {
     int rc;
-    if ((rc = alloc_panels(h, r))) return rc;
-    const Layout *L = h->L;
-    const size_t gr = (size_t)L->NG * h->rs * 8, cr = (size_t)L->NC * h->rs * 8;
-    CK(cudaMemsetAsync(h->d_lw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_alw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_lh, 0, cr, h->stream));
-    CK(cudaMemsetAsync(h->d_alh, 0, cr, h->stream));
+    if ((rc = zeroed_panels(h, r))) return rc;
     const int kmax = (int)std::min<int64_t>(std::min(h->n, h->m_global), vb::kSvdMaxK);
     for (int k : {std::min(r + 20, kmax), r}) {
         bool ok = true;
-        rc = h->val_float ? truncated_svd_t<float>(h, r, seed, cell_offset, k, 60, &ok, finish)
-                          : truncated_svd_t<double>(h, r, seed, cell_offset, k, 60, &ok, finish);
+        rc = with_val_type(h->val_float, [&](auto v) {
+            return truncated_svd_t<decltype(v)>(h, r, seed, cell_offset, k, 60, &ok, finish);
+        });
         if (rc) return rc;
-        if (ok) {
-            if ((rc = refresh_mirrors(h))) return rc;
-            return initial_ehsum(h);
-        }
+        if (ok) return loaded_state(h);
     }
     return fail(h, VBNMF_ERR_ARG, std::string(name) + " initializer: the matrix has numerical rank below `rank`");
 }
@@ -1447,15 +1601,12 @@ namespace {
 template <typename OT>
 void launch_subset_compact(H *h, const H *src, const int32_t *d_cols, const int32_t *d_rowmap,
                            const double *d_scale, OT *out_val, unsigned *d_bad) {
-    const int grid = h->num_sms * 8;
-    if (src->val_float)
-        vb::qc_subset_compact_kernel<float, OT><<<grid, vb::kBlock, 0, h->stream>>>(
-            h->m, d_cols, src->d_colptr, src->d_rowidx, (const float *)src->d_val, d_rowmap,
+    with_val_type(src->val_float, [&](auto v) {
+        using VT = decltype(v);
+        vb::qc_subset_compact_kernel<VT, OT><<<h->num_sms * 8, vb::kBlock, 0, h->stream>>>(
+            h->m, d_cols, src->d_colptr, src->d_rowidx, (const VT *)src->d_val, d_rowmap,
             d_scale, h->d_colptr, h->d_rowidx, out_val, d_bad);
-    else
-        vb::qc_subset_compact_kernel<double, OT><<<grid, vb::kBlock, 0, h->stream>>>(
-            h->m, d_cols, src->d_colptr, src->d_rowidx, (const double *)src->d_val, d_rowmap,
-            d_scale, h->d_colptr, h->d_rowidx, out_val, d_bad);
+    });
 }
 
 }  // namespace
@@ -1488,20 +1639,6 @@ int launch_shuffle(H *h, const H *src, uint64_t seed, unsigned *d_bad) {
 // ---- consensus measures (consensus.cuh) ---------------------------------------------------------
 namespace {
 
-// device buffers freed (stream-ordered) when the scope ends
-struct ScopedBufs {
-    cudaStream_t s;
-    std::vector<void *> p;
-    ~ScopedBufs() { for (void *q : p) vfree(s, q); }
-    template <typename T>
-    cudaError_t get(H *h, T **x, size_t bytes) {
-        *x = nullptr;
-        const cudaError_t e = vmalloc(h, x, bytes);
-        if (e == cudaSuccess) p.push_back((void *)*x);
-        return e;
-    }
-};
-
 inline int64_t choose2(unsigned long long x) { return (int64_t)(x * (x - 1) / 2); }
 
 // S1 = sum over runs t of sum_c C(n^t_c, 2) (the tables of the pairs (t, t) are diagonal);
@@ -1514,12 +1651,12 @@ int consensus_moments(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, in
         for (int u = t; u < nrun; u++) { pt.push_back(t); pu.push_back(u); }
     const int64_t batch = std::max<int64_t>(1, std::min<int64_t>({npairs, 65535,
                                                                  (256ll << 20) / ((int64_t)KK * 8)}));
-    ScopedBufs B{h->stream, {}};
+    ScopedBufs B(h);
     int32_t *d_pt = nullptr, *d_pu = nullptr;
     unsigned long long *d_tab = nullptr;
-    CK(B.get(h, &d_pt, (size_t)npairs * 4));
-    CK(B.get(h, &d_pu, (size_t)npairs * 4));
-    CK(B.get(h, &d_tab, (size_t)batch * KK * 8));
+    CK(B.get(&d_pt, (size_t)npairs * 4));
+    CK(B.get(&d_pu, (size_t)npairs * 4));
+    CK(B.get(&d_tab, (size_t)batch * KK * 8));
     CK(cudaMemcpyAsync(d_pt, pt.data(), (size_t)npairs * 4, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(d_pu, pu.data(), (size_t)npairs * 4, cudaMemcpyHostToDevice, h->stream));
     const int smem = KK * 4;
@@ -1550,17 +1687,17 @@ int consensus_moments(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, in
 
 // Groups of cells with equal label tuples, in lexicographic order of (L[0], L[1], ...): their
 // count G, sizes (G) and tuples (G x W words, 4 labels per word).  d_size / d_tup are allocated
-// here and owned by the caller.
-int consensus_groups(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, int W, int64_t *G_out,
-                     int64_t **d_size, uint32_t **d_tup) {
+// in the caller's scope `out`.
+int consensus_groups(H *h, ScopedBufs &out, int64_t m, int nrun, int K, const int32_t *d_lab, int W,
+                     int64_t *G_out, int64_t **d_size, uint32_t **d_tup) {
     cudaStream_t s = h->stream;
-    ScopedBufs B{s, {}};
+    ScopedBufs B(h);
     uint32_t *d_k0, *d_k1;
     int32_t *d_p0, *d_p1, *d_flag, *d_gid;
-    CK(B.get(h, &d_k0, (size_t)m * 4));
-    CK(B.get(h, &d_k1, (size_t)m * 4));
-    CK(B.get(h, &d_p0, (size_t)m * 4));
-    CK(B.get(h, &d_p1, (size_t)m * 4));
+    CK(B.get(&d_k0, (size_t)m * 4));
+    CK(B.get(&d_k1, (size_t)m * 4));
+    CK(B.get(&d_p0, (size_t)m * 4));
+    CK(B.get(&d_p1, (size_t)m * 4));
     int bits = 1;
     while ((1 << bits) < K) bits++;
     cub::DoubleBuffer<uint32_t> keys(d_k0, d_k1);
@@ -1569,7 +1706,7 @@ int consensus_groups(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, int
     CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)m, 0, bits, s));
     CK(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, d_p0, d_p1, (int)m, s));
     void *d_tmp = nullptr;
-    CK(B.get(h, &d_tmp, std::max(sort_bytes, scan_bytes)));
+    CK(B.get(&d_tmp, std::max(sort_bytes, scan_bytes)));
     std::vector<int32_t> iota((size_t)m);
     std::iota(iota.begin(), iota.end(), 0);
     CK(cudaMemcpyAsync(vals.Current(), iota.data(), (size_t)m * 4, cudaMemcpyHostToDevice, s));
@@ -1589,9 +1726,9 @@ int consensus_groups(H *h, int64_t m, int nrun, int K, const int32_t *d_lab, int
     CK(copy_sync(h, &G32, d_gid + m - 1, 4, cudaMemcpyDeviceToHost));
     const int64_t G = G32;
     int64_t *d_start;
-    CK(B.get(h, &d_start, (size_t)G * 8));
-    CK(vmalloc(h, d_size, (size_t)G * 8));
-    CK(vmalloc(h, d_tup, (size_t)G * W * 4));
+    CK(B.get(&d_start, (size_t)G * 8));
+    CK(out.get(d_size, (size_t)G * 8));
+    CK(out.get(d_tup, (size_t)G * W * 4));
     vb::group_start_kernel<<<gm, vb::kBlock, 0, s>>>(m, nrun, W, d_lab, d_perm, d_flag, d_gid,
                                                      d_start, *d_tup);
     vb::group_size_kernel<<<cdiv(G, vb::kBlock), vb::kBlock, 0, s>>>(G, m, d_start, *d_size);
@@ -1620,7 +1757,7 @@ size_t device_bytes_available(H *h) {
 int consensus_tree(H *h, int64_t G, int nrun, int W, const int64_t *d_size0, const uint32_t *d_tup,
                    int64_t *merges, int64_t *rescans) {
     cudaStream_t s = h->stream;
-    ScopedBufs B{s, {}};
+    ScopedBufs B(h);
     vb::MergeArgs A;
     A.G = G;
     A.nrun = nrun;
@@ -1628,16 +1765,16 @@ int consensus_tree(H *h, int64_t G, int nrun, int W, const int64_t *d_size0, con
     int per_sm = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, vb::merge_loop_kernel, vb::kMergeBlock, 0));
     const int grid = h->num_sms * std::max(per_sm, 1);
-    CK(B.get(h, &A.ip, (size_t)ntri * 8));
-    CK(B.get(h, &A.size, (size_t)G * 8));
-    CK(B.get(h, &A.bq, (size_t)G * 8));
-    CK(B.get(h, &A.bb, (size_t)G * 4));
-    CK(B.get(h, &A.merges, (size_t)(G - 1) * 5 * 8));
-    CK(B.get(h, &A.resc, (size_t)G * 4));
-    CK(B.get(h, &A.nresc, 16));
-    CK(B.get(h, &A.part_q, (size_t)grid * 8));
-    CK(B.get(h, &A.part_a, (size_t)grid * 8));
-    CK(B.get(h, &A.rescans, 8));
+    CK(B.get(&A.ip, (size_t)ntri * 8));
+    CK(B.get(&A.size, (size_t)G * 8));
+    CK(B.get(&A.bq, (size_t)G * 8));
+    CK(B.get(&A.bb, (size_t)G * 4));
+    CK(B.get(&A.merges, (size_t)(G - 1) * 5 * 8));
+    CK(B.get(&A.resc, (size_t)G * 4));
+    CK(B.get(&A.nresc, 16));
+    CK(B.get(&A.part_q, (size_t)grid * 8));
+    CK(B.get(&A.part_a, (size_t)grid * 8));
+    CK(B.get(&A.rescans, 8));
     CK(cudaMemcpyAsync(A.size, d_size0, (size_t)G * 8, cudaMemcpyDeviceToDevice, s));
     CK(cudaMemsetAsync(A.rescans, 0, 8, s));
     const int pad = 4 * W - nrun;
@@ -1702,86 +1839,47 @@ int vbnmf_create(vbnmf_handle **out, int64_t n, int64_t m, int64_t nnz, const in
                  const int64_t *colptr64, const int32_t *rowidx, const double *values, int device) {
     if (!out) return VBNMF_ERR_ARG;
     *out = nullptr;
-    H *h = new H();
-    auto bail = [&](int rc) {
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
-    };
     StageTimer tm("vbnmf_create(total)");
-    if (n <= 0 || m <= 0 || nnz <= 0 || (!colptr32 == !colptr64) || !rowidx || !values)
-        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create: bad arguments"));
-    if (n > INT32_MAX || m > INT32_MAX)
-        return bail(fail(h, VBNMF_ERR_ARG, "n and m must be below 2^31 (int32 row/column indices)"));
-    if (nnz >= (int64_t)UINT32_MAX)
-        return bail(fail(h, VBNMF_ERR_ARG, "nnz per GPU must be < 2^32-1"));
-    h->n = n; h->m = m; h->nnz = nnz;
-    int rc = init_common(h, device);
-    if (rc) return bail(rc);
-    bool as_float = true;
-    auto up = [&]() -> int {
+    auto check = [&](H *h) -> int {
+        if (n <= 0 || m <= 0 || nnz <= 0 || (!colptr32 == !colptr64) || !rowidx || !values)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create: bad arguments");
+        return set_dims(h, n, m, nnz);
+    };
+    return create_handle(out, device, check, [&](H *h) -> int {
         StageTimer tu("  upload (staged, pinned)");
-        bool ok = true;
-        std::atomic<int> unsorted{0};
-        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
-        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
-        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
+        int rc = alloc_csc(h);
+        if (rc) return rc;
         // column pointers: widened to 64 bits and checked on the way (first = 0, last = nnz,
         // non-decreasing: element j is compared with element j + 1, which the caller's array holds)
-        int rc2;
-        if (colptr64) {
-            if (colptr64[0] != 0 || colptr64[m] != nnz) return fail(h, VBNMF_ERR_ARG, "colptr does not span nnz");
-            rc2 = staged_upload(h, h->d_colptr, colptr64, m + 1,
-                                [](const int64_t &v, int64_t &o) { o = v; return true; }, &ok);
+        auto colptr_up = [&](const auto *cp) -> int {
+            if (cp[0] != 0 || (int64_t)cp[m] != nnz) return fail(h, VBNMF_ERR_ARG, "colptr does not span nnz");
+            bool ok = true;
+            int rc2 = staged_upload(h, h->d_colptr, cp, m + 1,
+                                    [](const auto &v, int64_t &o) { o = v; return true; }, &ok);
             if (rc2) return rc2;
+            std::atomic<int> unsorted{0};
             pool().run([&](int t, int nt) {
                 bool g = true;
-                for (int64_t j = m * t / nt; j < m * (t + 1) / nt; j++) g &= colptr64[j] <= colptr64[j + 1];
+                for (int64_t j = m * t / nt; j < m * (t + 1) / nt; j++) g &= cp[j] <= cp[j + 1];
                 if (!g) unsorted.store(1);
             });
-        } else {
-            if (colptr32[0] != 0 || (int64_t)colptr32[m] != nnz) return fail(h, VBNMF_ERR_ARG, "colptr does not span nnz");
-            rc2 = staged_upload(h, h->d_colptr, colptr32, m + 1,
-                                [](const int32_t &v, int64_t &o) { o = v; return true; }, &ok);
-            if (rc2) return rc2;
-            pool().run([&](int t, int nt) {
-                bool g = true;
-                for (int64_t j = m * t / nt; j < m * (t + 1) / nt; j++) g &= colptr32[j] <= colptr32[j + 1];
-                if (!g) unsorted.store(1);
-            });
-        }
-        if (unsorted.load()) return fail(h, VBNMF_ERR_ARG, "colptr is not non-decreasing");
+            return unsorted.load() ? fail(h, VBNMF_ERR_ARG, "colptr is not non-decreasing") : 0;
+        };
+        if ((rc = colptr64 ? colptr_up(colptr64) : colptr_up(colptr32))) return rc;
         // row indices: plain copy, range-checked on the device (scan_matrix)
-        rc2 = staged_upload(h, h->d_rowidx, rowidx, nnz,
-                            [](int32_t v, int32_t &o) { o = v; return true; }, &ok);
-        if (rc2) return rc2;
-        // counts go to the device as fp32 when every one of them is exactly representable
-        // (NaN compares unequal: it takes the fp64 path and is refused by scan_matrix)
-        float *dv = nullptr;
-        CK(vmalloc(h, &dv, (size_t)nnz * 4));
-        rc2 = staged_upload(h, dv, values, nnz,
-                            [](double v, float &o) { o = (float)v; return (double)o == v; }, &ok);
-        if (rc2) return rc2;
-        if (ok) {
-            h->d_val = dv;
-        } else {
-            as_float = false;
-            vfree(h->stream, dv);
-            double *dd = nullptr;
-            CK(vmalloc(h, &dd, (size_t)nnz * 8));
-            rc2 = staged_upload(h, dd, values, nnz, [](double v, double &o) { o = v; return true; },
-                                &ok);
-            if (rc2) return rc2;
-            h->d_val = dd;
-        }
-        return 0;
-    };
-    if ((rc = up())) return bail(rc);
-    h->val_float = as_float;
-    rc = as_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
-    if (rc) return bail(rc);
-    *out = h;
-    return 0;
+        bool ok = true;
+        rc = staged_upload(h, h->d_rowidx, rowidx, nnz,
+                           [](int32_t v, int32_t &o) { o = v; return true; }, &ok);
+        if (rc) return rc;
+        // NaN compares unequal: it takes the fp64 path and is refused by scan_matrix
+        return store_values(h, [&](auto *dv, bool *exact) {
+            using VT = std::remove_pointer_t<decltype(dv)>;
+            return staged_upload(h, dv, values, nnz, [](double v, VT &o) {
+                o = (VT)v;
+                return sizeof(VT) == 8 || (double)o == v;
+            }, exact);
+        });
+    });
 }
 
 int vbnmf_create_from_device(vbnmf_handle **out, int64_t n, int64_t m, int64_t nnz,
@@ -1789,77 +1887,63 @@ int vbnmf_create_from_device(vbnmf_handle **out, int64_t n, int64_t m, int64_t n
                              int device) {
     if (!out) return VBNMF_ERR_ARG;
     *out = nullptr;
-    H *h = new H();
-    auto bail = [&](int rc) {
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
+    auto check = [&](H *h) -> int {
+        if (n <= 0 || m <= 0 || nnz <= 0 || !d_colptr || !d_rowidx || !d_values)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create_from_device: bad arguments");
+        return set_dims(h, n, m, nnz);
     };
-    if (n <= 0 || m <= 0 || nnz <= 0 || !d_colptr || !d_rowidx || !d_values)
-        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_from_device: bad arguments"));
-    if (n > INT32_MAX || m > INT32_MAX)
-        return bail(fail(h, VBNMF_ERR_ARG, "n and m must be below 2^31 (int32 row/column indices)"));
-    if (nnz >= (int64_t)UINT32_MAX)
-        return bail(fail(h, VBNMF_ERR_ARG, "nnz per GPU must be < 2^32-1"));
-    h->n = n; h->m = m; h->nnz = nnz;
-    int rc = init_common(h, device);
-    if (rc) return bail(rc);
-    h->borrowed = true;
-    h->val_float = true;
-    h->d_colptr = const_cast<int64_t *>(d_colptr);
-    h->d_rowidx = const_cast<int32_t *>(d_rowidx);
-    h->d_val = const_cast<float *>(d_values);
-    if ((rc = scan_matrix_t<float>(h))) return bail(rc);
-    *out = h;
-    return 0;
+    return create_handle(out, device, check, [&](H *h) -> int {
+        h->borrowed = true;
+        h->val_float = true;
+        h->d_colptr = const_cast<int64_t *>(d_colptr);
+        h->d_rowidx = const_cast<int32_t *>(d_rowidx);
+        h->d_val = const_cast<float *>(d_values);
+        return 0;
+    });
 }
 
 int vbnmf_create_from_mtx(vbnmf_handle **out, const char *path, int device, int64_t dims[3]) {
     if (!out || !path) return VBNMF_ERR_ARG;
     *out = nullptr;
-    H *h = new H();
-    FILE *fp = nullptr;
-    auto bail = [&](int rc) {
-        if (fp) fclose(fp);
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
-    };
     StageTimer tm("vbnmf_create_from_mtx(total)");
-    fp = fopen(path, "rb");
-    if (!fp) return bail(fail(h, VBNMF_ERR_ARG, std::string("cannot open ") + path));
+    std::unique_ptr<FILE, int (*)(FILE *)> file(nullptr, fclose);
+    int64_t nbytes = 0;
     // header (host): banner, comments, the size line
-    char line[1024];
-    if (!fgets(line, sizeof(line), fp) || strncmp(line, "%%MatrixMarket", 14) != 0)
-        return bail(fail(h, VBNMF_ERR_ARG, "not a MatrixMarket file"));
-    std::string banner(line);
-    for (auto &ch : banner) ch = (char)tolower((unsigned char)ch);
-    if (banner.find("matrix") == std::string::npos || banner.find("coordinate") == std::string::npos ||
-        banner.find("general") == std::string::npos ||
-        (banner.find("real") == std::string::npos && banner.find("integer") == std::string::npos))
-        return bail(fail(h, VBNMF_ERR_ARG,
-                         "MatrixMarket: only 'matrix coordinate real|integer general' is supported"));
-    long long n = 0, m = 0, nnz = 0;
-    for (;;) {
-        if (!fgets(line, sizeof(line), fp))
-            return bail(fail(h, VBNMF_ERR_ARG, "MatrixMarket: missing size line"));
-        if (line[0] == '%' || line[0] == '\n' || line[0] == '\r') continue;
-        if (sscanf(line, "%lld %lld %lld", &n, &m, &nnz) != 3)
-            return bail(fail(h, VBNMF_ERR_ARG, "MatrixMarket: malformed size line"));
-        break;
-    }
-    if (n <= 0 || m <= 0 || nnz <= 0 || n > INT32_MAX || m > INT32_MAX || nnz >= (long long)UINT32_MAX)
-        return bail(fail(h, VBNMF_ERR_ARG, "MatrixMarket: dimensions out of range"));
-    const long off = ftell(fp);
-    fseek(fp, 0, SEEK_END);
-    const int64_t nbytes = (int64_t)ftell(fp) - off;
-    fseek(fp, off, SEEK_SET);
-    if (nbytes <= 0) return bail(fail(h, VBNMF_ERR_ARG, "MatrixMarket: no entries"));
-    h->n = n; h->m = m; h->nnz = nnz;
-    int rc = init_common(h, device);
-    if (rc) return bail(rc);
-    bool as_float = true;
-    auto body = [&]() -> int {
+    auto check = [&](H *h) -> int {
+        FILE *fp = fopen(path, "rb");
+        if (!fp) return fail(h, VBNMF_ERR_ARG, std::string("cannot open ") + path);
+        file.reset(fp);
+        char line[1024];
+        if (!fgets(line, sizeof(line), fp) || strncmp(line, "%%MatrixMarket", 14) != 0)
+            return fail(h, VBNMF_ERR_ARG, "not a MatrixMarket file");
+        std::string banner(line);
+        for (auto &ch : banner) ch = (char)tolower((unsigned char)ch);
+        if (banner.find("matrix") == std::string::npos || banner.find("coordinate") == std::string::npos ||
+            banner.find("general") == std::string::npos ||
+            (banner.find("real") == std::string::npos && banner.find("integer") == std::string::npos))
+            return fail(h, VBNMF_ERR_ARG,
+                        "MatrixMarket: only 'matrix coordinate real|integer general' is supported");
+        long long n = 0, m = 0, nnz = 0;
+        for (;;) {
+            if (!fgets(line, sizeof(line), fp))
+                return fail(h, VBNMF_ERR_ARG, "MatrixMarket: missing size line");
+            if (line[0] == '%' || line[0] == '\n' || line[0] == '\r') continue;
+            if (sscanf(line, "%lld %lld %lld", &n, &m, &nnz) != 3)
+                return fail(h, VBNMF_ERR_ARG, "MatrixMarket: malformed size line");
+            break;
+        }
+        if (n <= 0 || m <= 0 || nnz <= 0 || set_dims(h, n, m, nnz))
+            return fail(h, VBNMF_ERR_ARG, "MatrixMarket: dimensions out of range");
+        const long off = ftell(fp);
+        fseek(fp, 0, SEEK_END);
+        nbytes = (int64_t)ftell(fp) - off;
+        fseek(fp, off, SEEK_SET);
+        if (nbytes <= 0) return fail(h, VBNMF_ERR_ARG, "MatrixMarket: no entries");
+        return 0;
+    };
+    const int rc = create_handle(out, device, check, [&](H *h) -> int {
+        const int64_t n = h->n, m = h->m, nnz = h->nnz;
+        ScopedBufs B(h);
         char *d_buf = nullptr;
         uint8_t *d_flag = nullptr;
         int64_t *d_start = nullptr, *d_num = nullptr;
@@ -1867,13 +1951,7 @@ int vbnmf_create_from_mtx(vbnmf_handle **out, const char *path, int device, int6
         double *d_v = nullptr, *d_v2 = nullptr;
         unsigned *d_bad = nullptr;
         void *d_tmp = nullptr;
-        struct Free {
-            cudaStream_t s; void **p[10];
-            ~Free() { for (void **q : p) if (q) vfree(s, *q); }
-        } fr{h->stream, {(void **)&d_buf, (void **)&d_flag, (void **)&d_start, (void **)&d_num,
-                         (void **)&d_key, (void **)&d_key2, (void **)&d_v, (void **)&d_v2,
-                         (void **)&d_bad, &d_tmp}};
-        CK(vmalloc(h, &d_buf, (size_t)nbytes));
+        CK(B.get(&d_buf, (size_t)nbytes));
         {   // file bytes -> device through the pinned staging buffers
             std::lock_guard<std::mutex> lock(g_staging_mu);
             if (!g_staging.init()) return fail(h, VBNMF_ERR_CUDA, "cannot allocate pinned staging buffers");
@@ -1881,18 +1959,19 @@ int vbnmf_create_from_mtx(vbnmf_handle **out, const char *path, int device, int6
             for (int64_t lo = 0; lo < nbytes; lo += (int64_t)Staging::kBytes, slot = (slot + 1) % Staging::kSlots) {
                 const size_t len = (size_t)std::min<int64_t>((int64_t)Staging::kBytes, nbytes - lo);
                 CK(cudaEventSynchronize(g_staging.ev[slot]));
-                if (fread(g_staging.buf[slot], 1, len, fp) != len)
+                if (fread(g_staging.buf[slot], 1, len, file.get()) != len)
                     return fail(h, VBNMF_ERR_ARG, "MatrixMarket: short read");
                 CK(cudaMemcpyAsync(d_buf + lo, g_staging.buf[slot], len, cudaMemcpyHostToDevice, h->stream));
                 CK(cudaEventRecord(g_staging.ev[slot], h->stream));
             }
             CK(cudaStreamSynchronize(h->stream));
         }
+        file.reset();
         // line starts
-        CK(vmalloc(h, &d_flag, (size_t)nbytes));
-        CK(vmalloc(h, &d_start, (size_t)(nnz + 1) * 8));
-        CK(vmalloc(h, &d_num, 8));
-        CK(vmalloc(h, &d_bad, 4 * sizeof(unsigned)));
+        CK(B.get(&d_flag, (size_t)nbytes));
+        CK(B.get(&d_start, (size_t)(nnz + 1) * 8));
+        CK(B.get(&d_num, 8));
+        CK(B.get(&d_bad, 4 * sizeof(unsigned)));
         CK(cudaMemsetAsync(d_bad, 0, 4 * sizeof(unsigned), h->stream));
         vb::mtx_line_flags_kernel<<<h->num_sms * 8, vb::kBlock, 0, h->stream>>>(nbytes, d_buf, d_flag);
         // count first (the output must not overflow when the file has more lines than declared)
@@ -1900,69 +1979,52 @@ int vbnmf_create_from_mtx(vbnmf_handle **out, const char *path, int device, int6
         cub::CountingInputIterator<int64_t> iota(0);
         int64_t *d_cnt = d_num;
         CK(cub::DeviceReduce::Sum(nullptr, tb, d_flag, d_cnt, nbytes, h->stream));
-        CK(vmalloc(h, &d_tmp, tb));
+        CK(B.get(&d_tmp, tb));
         CK(cub::DeviceReduce::Sum(d_tmp, tb, d_flag, d_cnt, nbytes, h->stream));
         int64_t nlines = 0;
         CK(cudaMemcpyAsync(&nlines, d_cnt, 8, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
-        vfree(h->stream, d_tmp); d_tmp = nullptr;
+        B.free(d_tmp);
         if (nlines != nnz)
             return fail(h, VBNMF_ERR_ARG, "MatrixMarket: number of entry lines differs from the size line");
         CK(cub::DeviceSelect::Flagged(nullptr, tb, iota, d_flag, d_start, d_num, nbytes, h->stream));
-        CK(vmalloc(h, &d_tmp, tb));
+        CK(B.get(&d_tmp, tb));
         CK(cub::DeviceSelect::Flagged(d_tmp, tb, iota, d_flag, d_start, d_num, nbytes, h->stream));
-        vfree(h->stream, d_tmp); d_tmp = nullptr;
+        B.free(d_tmp);
         // parse, sort by (column, row)
-        CK(vmalloc(h, &d_key, (size_t)nnz * 8));
-        CK(vmalloc(h, &d_key2, (size_t)nnz * 8));
-        CK(vmalloc(h, &d_v, (size_t)nnz * 8));
-        CK(vmalloc(h, &d_v2, (size_t)nnz * 8));
+        CK(B.get(&d_key, (size_t)nnz * 8));
+        CK(B.get(&d_key2, (size_t)nnz * 8));
+        CK(B.get(&d_v, (size_t)nnz * 8));
+        CK(B.get(&d_v2, (size_t)nnz * 8));
         vb::mtx_parse_kernel<<<cdiv(nnz, vb::kBlock), vb::kBlock, 0, h->stream>>>(
             nnz, nbytes, d_buf, d_start, n, m, d_key, d_v, d_bad);
         int cbits = 1;
         while ((1ll << cbits) < m) cbits++;
         CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, d_key, d_key2, d_v, d_v2, nnz, 0, 32 + cbits, h->stream));
-        CK(vmalloc(h, &d_tmp, tb));
+        CK(B.get(&d_tmp, tb));
         CK(cub::DeviceRadixSort::SortPairs(d_tmp, tb, d_key, d_key2, d_v, d_v2, nnz, 0, 32 + cbits, h->stream));
-        // CSC arrays owned by the handle
-        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
-        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
-        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
-        float *dv = nullptr;
-        CK(vmalloc(h, &dv, (size_t)nnz * 4));
-        vb::mtx_unpack_kernel<float><<<cdiv(nnz, vb::kBlock), vb::kBlock, 0, h->stream>>>(
-            nnz, d_key2, d_v2, h->d_rowidx, dv, d_bad);
+        int rc = alloc_csc(h);
+        if (rc) return rc;
         vb::mtx_colptr_kernel<<<cdiv(m + 1, vb::kBlock), vb::kBlock, 0, h->stream>>>(m, nnz, d_key2,
                                                                                    h->d_colptr);
-        unsigned bad[4];
-        CK(cudaMemcpyAsync(bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        CK(cudaGetLastError());
-        if (bad[0]) { vfree(h->stream, dv); return fail(h, VBNMF_ERR_ARG, "MatrixMarket: malformed entry line or index out of range"); }
-        if (bad[1]) { vfree(h->stream, dv); return fail(h, VBNMF_ERR_ARG, "MatrixMarket: duplicate entries"); }
-        if (bad[2]) {  // counts not exact in fp32: keep them in fp64
-            vfree(h->stream, dv);
-            double *dd = nullptr;
-            CK(vmalloc(h, &dd, (size_t)nnz * 8));
-            vb::mtx_unpack_kernel<double><<<cdiv(nnz, vb::kBlock), vb::kBlock, 0, h->stream>>>(
-                nnz, d_key2, d_v2, h->d_rowidx, dd, d_bad + 3);
-            h->d_val = dd;
-            as_float = false;
-        } else {
-            h->d_val = dv;
-        }
-        CK(cudaStreamSynchronize(h->stream));
-        return 0;
-    };
-    if ((rc = body())) return bail(rc);
-    fclose(fp);
-    fp = nullptr;
-    h->val_float = as_float;
-    rc = as_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
-    if (rc) return bail(rc);
-    if (dims) { dims[0] = n; dims[1] = m; dims[2] = nnz; }
-    *out = h;
-    return 0;
+        // the fp32 pass also flags malformed lines and duplicates; the fp64 pass writes its flags
+        // apart, from d_bad + 3
+        return store_values(h, [&](auto *dv, bool *exact) -> int {
+            using VT = std::remove_pointer_t<decltype(dv)>;
+            vb::mtx_unpack_kernel<VT><<<cdiv(nnz, vb::kBlock), vb::kBlock, 0, h->stream>>>(
+                nnz, d_key2, d_v2, h->d_rowidx, dv, sizeof(VT) == 4 ? d_bad : d_bad + 3);
+            unsigned bad[4];
+            CK(cudaMemcpyAsync(bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            CK(cudaGetLastError());
+            if (bad[0]) return fail(h, VBNMF_ERR_ARG, "MatrixMarket: malformed entry line or index out of range");
+            if (bad[1]) return fail(h, VBNMF_ERR_ARG, "MatrixMarket: duplicate entries");
+            *exact = !bad[2];
+            return 0;
+        });
+    });
+    if (!rc && dims) { dims[0] = (*out)->n; dims[1] = (*out)->m; dims[2] = (*out)->nnz; }
+    return rc;
 }
 
 /* the CSC arrays a handle holds, back on the host (colptr m+1 int64, rowidx nnz int32, values nnz
@@ -1994,28 +2056,21 @@ int vbnmf_qc_stats(vbnmf_handle *h, double *cell_sum, double *gene_sum, double *
     CK(cudaSetDevice(h->device));
     const int64_t n = h->n, m = h->m;
     if (cell_sum || gene_sum || gene_sumsq) {
+        ScopedBufs B(h);
         double *d = nullptr;  // [cell_sum m | gene_sum n | gene_sumsq n]
-        CK(vmalloc(h, &d, (size_t)(m + 2 * n) * 8));
-        auto body = [&]() -> int {
-            CK(cudaMemsetAsync(d + m, 0, (size_t)2 * n * 8, h->stream));
-            const int grid = h->num_sms * 8;
-            if (h->val_float)
-                vb::qc_stats_kernel<float><<<grid, vb::kBlock, 0, h->stream>>>(
-                    m, h->d_colptr, h->d_rowidx, (const float *)h->d_val, d, d + m, d + m + n);
-            else
-                vb::qc_stats_kernel<double><<<grid, vb::kBlock, 0, h->stream>>>(
-                    m, h->d_colptr, h->d_rowidx, (const double *)h->d_val, d, d + m, d + m + n);
-            CK(cudaGetLastError());
-            if (cell_sum) CK(cudaMemcpyAsync(cell_sum, d, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
-            if (gene_sum) CK(cudaMemcpyAsync(gene_sum, d + m, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
-            if (gene_sumsq)
-                CK(cudaMemcpyAsync(gene_sumsq, d + m + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
-            CK(cudaStreamSynchronize(h->stream));
-            return 0;
-        };
-        const int rc = body();
-        vfree(h->stream, d);
-        if (rc) return rc;
+        CK(B.get(&d, (size_t)(m + 2 * n) * 8));
+        CK(cudaMemsetAsync(d + m, 0, (size_t)2 * n * 8, h->stream));
+        with_val_type(h->val_float, [&](auto v) {
+            using VT = decltype(v);
+            vb::qc_stats_kernel<VT><<<h->num_sms * 8, vb::kBlock, 0, h->stream>>>(
+                m, h->d_colptr, h->d_rowidx, (const VT *)h->d_val, d, d + m, d + m + n);
+        });
+        CK(cudaGetLastError());
+        if (cell_sum) CK(cudaMemcpyAsync(cell_sum, d, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (gene_sum) CK(cudaMemcpyAsync(gene_sum, d + m, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (gene_sumsq)
+            CK(cudaMemcpyAsync(gene_sumsq, d + m + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
     }
     // entries with a non-zero value: the counts scan_matrix keeps on the device
     static_assert(sizeof(unsigned long long) == sizeof(int64_t), "d_cnt is copied as int64");
@@ -2029,61 +2084,51 @@ int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *ke
                         const uint8_t *keep_cols, const double *col_scale) {
     if (!out) return VBNMF_ERR_ARG;
     *out = nullptr;
-    H *h = new H();
-    auto bail = [&](int rc) {
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
-    };
     StageTimer tm("vbnmf_create_subset(total)");
-    if (!src || !keep_rows || !keep_cols)
-        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: bad arguments"));
-    // the gene statistics and the empty-gene test of one shard are partial: refused, not guessed
-    if (src->nranks > 1)
-        return bail(fail(h, VBNMF_ERR_STATE, "vbnmf_create_subset: the source holds one shard of "
-                                             "the cells (vbnmf_attach_comm)"));
-    const int64_t n0 = src->n, m0 = src->m;
-    int64_t n = 0, m = 0;
-    for (int64_t i = 0; i < n0; i++) n += keep_rows[i] != 0;
-    for (int64_t j = 0; j < m0; j++) m += keep_cols[j] != 0;
-    if (n == 0 || m == 0)
-        return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: no rows or no columns selected"));
-    h->n = n; h->m = m;
-    int rc = init_common(h, src->device);
-    if (rc) return bail(rc);
-    bool as_float = true;
-    auto body = [&]() -> int {
+    auto check = [&](H *h) -> int {
+        if (!src || !keep_rows || !keep_cols)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: bad arguments");
+        // the gene statistics and the empty-gene test of one shard are partial: refused, not guessed
+        if (src->nranks > 1)
+            return fail(h, VBNMF_ERR_STATE, "vbnmf_create_subset: the source holds one shard of "
+                                            "the cells (vbnmf_attach_comm)");
+        int64_t n = 0, m = 0;
+        for (int64_t i = 0; i < src->n; i++) n += keep_rows[i] != 0;
+        for (int64_t j = 0; j < src->m; j++) m += keep_cols[j] != 0;
+        if (n == 0 || m == 0)
+            return fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: no rows or no columns selected");
+        h->n = n; h->m = m;
+        return 0;
+    };
+    return create_handle(out, src ? src->device : 0, check, [&](H *h) -> int {
+        const int64_t n0 = src->n, m0 = src->m, m = h->m;
+        ScopedBufs B(h);
         uint8_t *d_mask = nullptr;  // [rows n0 | columns m0]
         double *d_scale = nullptr;
         int32_t *d_rowmap = nullptr, *d_cols = nullptr, *d_nsel = nullptr;
         int64_t *d_ptr = nullptr;
         unsigned *d_bad = nullptr;
         void *d_tmp = nullptr;
-        struct Free {
-            cudaStream_t s; void **p[8];
-            ~Free() { for (void **q : p) if (q) vfree(s, *q); }
-        } fr{h->stream, {(void **)&d_mask, (void **)&d_scale, (void **)&d_rowmap, (void **)&d_cols,
-                         (void **)&d_nsel, (void **)&d_ptr, (void **)&d_bad, &d_tmp}};
         // src's arrays are read on this handle's stream: src's own work on them must be complete
         CK(cudaStreamSynchronize(src->stream));
         cudaStream_t s = h->stream;
-        CK(vmalloc(h, &d_mask, (size_t)(n0 + m0)));
+        CK(B.get(&d_mask, (size_t)(n0 + m0)));
         CK(cudaMemcpyAsync(d_mask, keep_rows, (size_t)n0, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(d_mask + n0, keep_cols, (size_t)m0, cudaMemcpyHostToDevice, s));
         if (col_scale) {
-            CK(vmalloc(h, &d_scale, (size_t)m0 * 8));
+            CK(B.get(&d_scale, (size_t)m0 * 8));
             CK(cudaMemcpyAsync(d_scale, col_scale, (size_t)m0 * 8, cudaMemcpyHostToDevice, s));
         }
-        CK(vmalloc(h, &d_rowmap, (size_t)n0 * 4));
-        CK(vmalloc(h, &d_cols, (size_t)m * 4));
-        CK(vmalloc(h, &d_nsel, 4));
-        CK(vmalloc(h, &d_ptr, (size_t)(m + 1) * 8));
+        CK(B.get(&d_rowmap, (size_t)n0 * 4));
+        CK(B.get(&d_cols, (size_t)m * 4));
+        CK(B.get(&d_nsel, 4));
+        CK(B.get(&d_ptr, (size_t)(m + 1) * 8));
         cub::CountingInputIterator<int32_t> iota(0);
         size_t tb1 = 0, tb2 = 0, tb3 = 0;
         CK(cub::DeviceScan::ExclusiveSum(nullptr, tb1, d_rowmap, d_rowmap, n0, s));
         CK(cub::DeviceSelect::Flagged(nullptr, tb2, iota, d_mask + n0, d_cols, d_nsel, m0, s));
         CK(cub::DeviceScan::ExclusiveSum(nullptr, tb3, d_ptr, d_ptr, m + 1, s));
-        CK(vmalloc(h, &d_tmp, std::max(tb1, std::max(tb2, tb3))));
+        CK(B.get(&d_tmp, std::max(tb1, std::max(tb2, tb3))));
         // kept rows renumbered in order (exclusive scan of the row mask), dropped rows -> -1
         vb::qc_mask_kernel<<<cdiv(n0, vb::kBlock), vb::kBlock, 0, s>>>(n0, d_mask, d_rowmap);
         CK(cub::DeviceScan::ExclusiveSum(d_tmp, tb1, d_rowmap, d_rowmap, n0, s));
@@ -2100,178 +2145,127 @@ int vbnmf_create_subset(vbnmf_handle **out, vbnmf_handle *src, const uint8_t *ke
         CK(cudaGetLastError());
         if (nnz == 0) return fail(h, VBNMF_ERR_ARG, "vbnmf_create_subset: the selection holds no entries");
         h->nnz = h->nnz_global = nnz;
-        // allocation order of the other create paths: the arena first, then the CSC arrays
-        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
-        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
+        int rc = alloc_csc(h);
+        if (rc) return rc;
         CK(cudaMemcpyAsync(h->d_colptr, d_ptr, (size_t)(m + 1) * 8, cudaMemcpyDeviceToDevice, s));
-        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
-        CK(vmalloc(h, &d_bad, 4));
+        CK(B.get(&d_bad, 4));
         CK(cudaMemsetAsync(d_bad, 0, 4, s));
-        // values as fp32 when every kept (scaled) value is exact in fp32, else fp64 (vbnmf_create)
-        float *dv = nullptr;
-        CK(vmalloc(h, &dv, (size_t)nnz * 4));
-        h->d_val = dv;
-        launch_subset_compact<float>(h, src, d_cols, d_rowmap, d_scale, dv, d_bad);
-        unsigned bad = 0;
-        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-        if (bad) {
-            vfree(s, dv);
-            h->d_val = nullptr;
-            double *dd = nullptr;
-            CK(vmalloc(h, &dd, (size_t)nnz * 8));
-            h->d_val = dd;
-            launch_subset_compact<double>(h, src, d_cols, d_rowmap, d_scale, dd, d_bad);
-            as_float = false;
-        }
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-        return 0;
-    };
-    if ((rc = body())) return bail(rc);
-    h->val_float = as_float;
-    rc = as_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
-    if (rc) return bail(rc);
-    *out = h;
-    return 0;
+        // the kept (scaled) values
+        return store_values(h, [&](auto *dv, bool *exact) -> int {
+            launch_subset_compact(h, src, d_cols, d_rowmap, d_scale, dv, d_bad);
+            unsigned bad = 0;
+            CK(copy_sync(h, &bad, d_bad, 4, cudaMemcpyDeviceToHost));
+            CK(cudaGetLastError());
+            *exact = !bad;
+            return 0;
+        });
+    });
 }
 
 int vbnmf_create_shuffled(vbnmf_handle **out, vbnmf_handle *src, uint64_t seed) {
     if (!out) return VBNMF_ERR_ARG;
     *out = nullptr;
-    H *h = new H();
-    auto bail = [&](int rc) {
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
-    };
     StageTimer tm("vbnmf_create_shuffled(total)");
-    if (!src) return bail(fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: bad arguments"));
-    // the draw is keyed by the column index: a shard would need its global column offset
-    if (src->nranks > 1)
-        return bail(fail(h, VBNMF_ERR_STATE, "vbnmf_create_shuffled: the source holds one shard of "
-                                             "the cells (vbnmf_attach_comm)"));
-    if (src->n > vb::kShuffleMaxRows)
-        return bail(fail(h, VBNMF_ERR_ARG,
-                         "vbnmf_create_shuffled: n = " + std::to_string(src->n) + " rows; at most " +
-                             std::to_string(vb::kShuffleMaxRows) +
-                             " (a column's row bitmap must fit one CTA's shared memory)"));
-    const int64_t n = src->n, m = src->m, nnz = src->nnz;
-    h->n = n; h->m = m; h->nnz = nnz;
-    int rc = init_common(h, src->device);
-    if (rc) return bail(rc);
-    h->val_float = src->val_float;
-    auto body = [&]() -> int {
-        unsigned *d_bad = nullptr;
-        struct Free {
-            cudaStream_t s; unsigned **p;
-            ~Free() { vfree(s, *p); }
-        } fr{h->stream, &d_bad};
+    auto check = [&](H *h) -> int {
+        if (!src) return fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: bad arguments");
+        // the draw is keyed by the column index: a shard would need its global column offset
+        if (src->nranks > 1)
+            return fail(h, VBNMF_ERR_STATE, "vbnmf_create_shuffled: the source holds one shard of "
+                                            "the cells (vbnmf_attach_comm)");
+        if (src->n > vb::kShuffleMaxRows)
+            return fail(h, VBNMF_ERR_ARG,
+                        "vbnmf_create_shuffled: n = " + std::to_string(src->n) + " rows; at most " +
+                            std::to_string(vb::kShuffleMaxRows) +
+                            " (a column's row bitmap must fit one CTA's shared memory)");
+        h->n = src->n; h->m = src->m; h->nnz = src->nnz;
+        h->val_float = src->val_float;
+        return 0;
+    };
+    return create_handle(out, src ? src->device : 0, check, [&](H *h) -> int {
         int optin = 0;
         CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-        if (optin < vb::shuffle_words(n) * 2 * 4)
+        if (optin < vb::shuffle_words(h->n) * 2 * 4)
             return fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: the row bitmap of a column does "
                                           "not fit this device's shared memory");
         // src's arrays are read on this handle's stream: src's own work on them must be complete
         CK(cudaStreamSynchronize(src->stream));
         cudaStream_t s = h->stream;
-        // allocation order of the other create paths: the arena first, then the CSC arrays
-        CK(vmalloc(h, &h->d_arena, (size_t)std::max<int64_t>(nnz * 5, 4 * std::max(n, m)) * 4));
-        CK(vmalloc(h, &h->d_colptr, (size_t)(m + 1) * 8));
-        CK(cudaMemcpyAsync(h->d_colptr, src->d_colptr, (size_t)(m + 1) * 8,
+        int rc = alloc_csc(h);
+        if (rc) return rc;
+        CK(cudaMemcpyAsync(h->d_colptr, src->d_colptr, (size_t)(h->m + 1) * 8,
                            cudaMemcpyDeviceToDevice, s));
-        CK(vmalloc(h, &h->d_rowidx, (size_t)nnz * 4));
-        CK(vmalloc(h, &h->d_val, (size_t)nnz * (h->val_float ? 4 : 8)));
-        CK(vmalloc(h, &d_bad, 4));
+        CK(vmalloc(h, &h->d_val, (size_t)h->nnz * (h->val_float ? 4 : 8)));
+        ScopedBufs B(h);
+        unsigned *d_bad = nullptr;
+        CK(B.get(&d_bad, 4));
         CK(cudaMemsetAsync(d_bad, 0, 4, s));
-        const int lrc = h->val_float ? launch_shuffle<float>(h, src, seed, d_bad)
-                                     : launch_shuffle<double>(h, src, seed, d_bad);
-        if (lrc) return lrc;
+        rc = with_val_type(h->val_float, [&](auto v) {
+            return launch_shuffle<decltype(v)>(h, src, seed, d_bad);
+        });
+        if (rc) return rc;
         unsigned bad = 0;
-        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
+        CK(copy_sync(h, &bad, d_bad, 4, cudaMemcpyDeviceToHost));
         CK(cudaGetLastError());
         if (bad)
             return fail(h, VBNMF_ERR_ARG, "vbnmf_create_shuffled: a column holds more entries than "
                                           "there are rows (repeated entries)");
         return 0;
-    };
-    if ((rc = body())) return bail(rc);
-    rc = h->val_float ? scan_matrix_t<float>(h) : scan_matrix_t<double>(h);
-    if (rc) return bail(rc);
-    *out = h;
-    return 0;
+    });
 }
 
 int vbnmf_consensus(int device, int64_t m, int nrun, int nlabels, const int32_t *labels,
                     int64_t max_groups, int64_t moments[2], int64_t *ngroups, int64_t *merges,
                     int64_t merge_cap, int64_t *rescans) {
-    H *h = new H();
-    auto done = [&](int rc) {
-        g_create_error = h->err;
-        vbnmf_destroy(h);
-        return rc;
+    auto arg = [](H *h, const std::string &msg) {
+        return fail(h, VBNMF_ERR_ARG, "vbnmf_consensus: " + msg);
     };
-    auto arg = [&](const std::string &msg) { return done(fail(h, VBNMF_ERR_ARG, "vbnmf_consensus: " + msg)); };
     if (ngroups) *ngroups = 0;
     if (rescans) *rescans = 0;
-    if (!labels || !moments || (merges && (!ngroups || !rescans)))
-        return arg("labels and moments are required, ngroups and rescans with merges");
-    if (nrun < 1 || m < 1 || m > INT32_MAX) return arg("needs nrun >= 1 and 1 <= m < 2^31");
-    if (nlabels < 1 || nlabels > vb::kConsensusMaxLabels)
-        return arg("nlabels = " + std::to_string(nlabels) + "; 1 ... " +
-                   std::to_string(vb::kConsensusMaxLabels) +
-                   " (a K x K table of counters must fit one CTA's shared memory)");
-    const unsigned __int128 half = (unsigned __int128)((m + 1) / 2);
-    if ((unsigned __int128)nrun * half * half >= ((unsigned __int128)1 << 53))
-        return arg("nrun * ceil(m / 2)^2 must be below 2^53 (exact IP values and their fp64 ratios)");
-    for (int64_t i = 0; i < (int64_t)nrun * m; i++)
-        if (labels[i] < 0 || labels[i] >= nlabels)
-            return arg("label " + std::to_string(labels[i]) + " outside 0 ... nlabels - 1");
-    int rc = init_common(h, device);
-    if (rc) return done(rc);
-    StageTimer tm("vbnmf_consensus(total)");
-    const int W = (nrun + 3) / 4;
-    int64_t *d_size = nullptr;
-    uint32_t *d_tup = nullptr;
-    auto body = [&]() -> int {
+    auto check = [&](H *h) -> int {
+        if (!labels || !moments || (merges && (!ngroups || !rescans)))
+            return arg(h, "labels and moments are required, ngroups and rescans with merges");
+        if (nrun < 1 || m < 1 || m > INT32_MAX) return arg(h, "needs nrun >= 1 and 1 <= m < 2^31");
+        if (nlabels < 1 || nlabels > vb::kConsensusMaxLabels)
+            return arg(h, "nlabels = " + std::to_string(nlabels) + "; 1 ... " +
+                              std::to_string(vb::kConsensusMaxLabels) +
+                              " (a K x K table of counters must fit one CTA's shared memory)");
+        const unsigned __int128 half = (unsigned __int128)((m + 1) / 2);
+        if ((unsigned __int128)nrun * half * half >= ((unsigned __int128)1 << 53))
+            return arg(h, "nrun * ceil(m / 2)^2 must be below 2^53 (exact IP values and their fp64 ratios)");
+        for (int64_t i = 0; i < (int64_t)nrun * m; i++)
+            if (labels[i] < 0 || labels[i] >= nlabels)
+                return arg(h, "label " + std::to_string(labels[i]) + " outside 0 ... nlabels - 1");
+        return 0;
+    };
+    return create_handle(nullptr, device, check, [&](H *h) -> int {
+        StageTimer tm("vbnmf_consensus(total)");
+        const int W = (nrun + 3) / 4;
+        ScopedBufs B(h);
         int32_t *d_lab = nullptr;
-        CK(vmalloc(h, &d_lab, (size_t)nrun * m * 4));
-        struct Free {
-            cudaStream_t s; int32_t *p;
-            ~Free() { vfree(s, p); }
-        } fr{h->stream, d_lab};
+        CK(B.get(&d_lab, (size_t)nrun * m * 4));
         CK(cudaMemcpyAsync(d_lab, labels, (size_t)nrun * m * 4, cudaMemcpyHostToDevice, h->stream));
-        int r = consensus_moments(h, m, nrun, nlabels, d_lab, moments);
-        if (r || !merges) return r;
-        int64_t G = 0;
-        if ((r = consensus_groups(h, m, nrun, nlabels, d_lab, W, &G, &d_size, &d_tup))) return r;
+        int rc = consensus_moments(h, m, nrun, nlabels, d_lab, moments);
+        if (rc || !merges) return rc;
+        int64_t G = 0, *d_size = nullptr;
+        uint32_t *d_tup = nullptr;
+        if ((rc = consensus_groups(h, B, m, nrun, nlabels, d_lab, W, &G, &d_size, &d_tup))) return rc;
+        B.free(d_lab);
         *ngroups = G;
         if (merge_cap < G - 1)
             return fail(h, VBNMF_ERR_ARG, "vbnmf_consensus: merge_cap = " + std::to_string(merge_cap) +
                                               " below G - 1 = " + std::to_string(G - 1));
-        return 0;
-    };
-    rc = body();
-    if (!rc && merges && *ngroups > 1) {
-        const int64_t G = *ngroups;
+        if (G <= 1) return 0;
         // the triangle, the row cache, the merge list and the sizes; 256 MB left for the rest
         const double need = 8.0 * G * (G - 1) / 2 + 64.0 * G + (256 << 20);
         if (max_groups > 0 && G > max_groups)
-            rc = fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) +
-                                               " groups above max_groups = " + std::to_string(max_groups));
-        else if (cudaStreamSynchronize(h->stream) != cudaSuccess ||
-                 need > (double)device_bytes_available(h))
-            rc = fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) + " groups need " +
-                                               std::to_string((int64_t)(need / 1e9)) +
-                                               " GB of device memory for the IP triangle");
-        else
-            rc = consensus_tree(h, G, nrun, W, d_size, d_tup, merges, rescans);
-    }
-    vfree(h->stream, d_size);
-    vfree(h->stream, d_tup);
-    return done(rc);
+            return fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) +
+                                                 " groups above max_groups = " + std::to_string(max_groups));
+        if (cudaStreamSynchronize(h->stream) != cudaSuccess || need > (double)device_bytes_available(h))
+            return fail(h, VBNMF_ERR_MEMORY, "vbnmf_consensus: G = " + std::to_string(G) + " groups need " +
+                                                 std::to_string((int64_t)(need / 1e9)) +
+                                                 " GB of device memory for the IP triangle");
+        return consensus_tree(h, G, nrun, W, d_size, d_tup, merges, rescans);
+    });
 }
 
 int vbnmf_set_precision(vbnmf_handle *h, int precision) {
@@ -2350,12 +2344,13 @@ int vbnmf_attach_comm(vbnmf_handle *h, vbnmf_comm *c) {
     // tile height (split layout, staging slots), which all ranks must share -- the gene panels
     // are all-reduced in device order
     double hv[5] = {(double)h->m, h->lgx, h->mlconst, (double)h->nnz, h->p16 ? 0.0 : 1.0};
+    ScopedBufs B(h);
     double *dv = nullptr;
     unsigned *d_flag = nullptr;
     uint32_t *d_scr = nullptr;
-    CK(vmalloc(h, &dv, 5 * 8));
-    CK(vmalloc(h, &d_flag, 4));
-    CK(vmalloc(h, &d_scr, (size_t)2 * h->n * 4));
+    CK(B.get(&dv, 5 * 8));
+    CK(B.get(&d_flag, 4));
+    CK(B.get(&d_scr, (size_t)2 * h->n * 4));
     CK(cudaMemsetAsync(d_flag, 0, 4, h->stream));
     CK(cudaMemcpyAsync(dv, hv, 5 * 8, cudaMemcpyHostToDevice, h->stream));
     int rc = allreduce(h, dv, 5);
@@ -2367,7 +2362,7 @@ int vbnmf_attach_comm(vbnmf_handle *h, vbnmf_comm *c) {
     CK(cudaMemcpyAsync(hv, dv, 5 * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(&nzero, d_flag, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, dv); vfree(h->stream, d_flag); vfree(h->stream, d_scr);
+    B.free(dv); B.free(d_flag); B.free(d_scr);
     h->m_global = (int64_t)llround(hv[0]);
     h->lgx = hv[1];
     h->mlconst = hv[2];
@@ -2380,46 +2375,14 @@ int vbnmf_attach_comm(vbnmf_handle *h, vbnmf_comm *c) {
     return 0;
 }
 
-// rowSums(eh) of the state just loaded (alh holds eh before the first update), over all shards,
-// into the tail of the reduce buffer and the host vectors
-static int initial_ehsum(H *h) {
-    const Layout *L = h->L;
-    const int rs = h->rs, r = h->r;
-    int rc;
-    double *tail = h->d_red + tail_off(h);
-    CK(cudaMemsetAsync(tail, 0, (size_t)(rs + 8) * 8, h->stream));
-    vb::ColsumArgs ca{L->NC, h->d_alh, h->d_partH, tail, h->d_counters + 1, 0};
-    h->tab->colsum(ca, h->stream);
-    h->launches += 1;
-    if ((rc = allreduce(h, tail, rs + 8))) return rc;
-    double s[kMaxRank + 16];  // rs + 8 <= 66 + 8
-    CK(cudaMemcpyAsync(s, tail, (size_t)(rs + 8) * 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaGetLastError());
-    for (int k = 0; k < kMaxRank; k++) {
-        h->ehsum[k] = k < r ? s[k] : 0.0;
-        h->ewsum[k] = 0.0;
-        h->bew[k] = h->beh[k] = 1.0;
-    }
-    h->stats_valid = false;
-    h->has_posterior = false;
-    return 0;
-}
-
 int vbnmf_set_state(vbnmf_handle *h, int r, const double *lw, const double *lh, const double *ew,
                     const double *eh) {
     if (!h || !lw || !lh) return VBNMF_ERR_ARG;
-    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    int rc;
+    if ((rc = check_rank(h, r))) return rc;
     CK(cudaSetDevice(h->device));
     StageTimer tm("vbnmf_set_state(total)");
-    int rc;
-    if ((rc = alloc_panels(h, r))) return rc;
-    const Layout *L = h->L;
-    const size_t gr = (size_t)L->NG * h->rs * 8, cr = (size_t)L->NC * h->rs * 8;
-    CK(cudaMemsetAsync(h->d_lw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_alw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_lh, 0, cr, h->stream));
-    CK(cudaMemsetAsync(h->d_alh, 0, cr, h->stream));
+    if ((rc = zeroed_panels(h, r))) return rc;
     // before the first update ew/eh are whatever the caller holds (vb_init: ew = w, eh = h); a
     // matrix passed twice goes up once
     const bool ew_same = !ew || ew == lw, eh_same = !eh || eh == lh;
@@ -2427,27 +2390,21 @@ int vbnmf_set_state(vbnmf_handle *h, int r, const double *lw, const double *lh, 
     if (!ew_same && (rc = upload_panel(h, h->d_alw, nullptr, ew, true, r))) return rc;
     if ((rc = upload_panel(h, h->d_lh, eh_same ? h->d_alh : nullptr, lh, false, r))) return rc;
     if (!eh_same && (rc = upload_panel(h, h->d_alh, nullptr, eh, false, r))) return rc;
-    if ((rc = refresh_mirrors(h))) return rc;
-    return initial_ehsum(h);
+    return loaded_state(h);
 }
 
 int vbnmf_init_random(vbnmf_handle *h, int r, const double hyper[4], uint64_t seed,
                       int64_t cell_offset) {
     if (!h || !hyper) return VBNMF_ERR_ARG;
-    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    int rc;
+    if ((rc = check_rank(h, r))) return rc;
     if (!(hyper[0] > 0 && hyper[1] > 0 && hyper[2] > 0 && hyper[3] > 0) || cell_offset < 0)
         return fail(h, VBNMF_ERR_ARG, "hyper-parameters must be positive");
     CK(cudaSetDevice(h->device));
     StageTimer tm("vbnmf_init_random(total)");
-    int rc;
-    if ((rc = alloc_panels(h, r))) return rc;
+    if ((rc = zeroed_panels(h, r))) return rc;
     const Layout *L = h->L;
     const int rs = h->rs;
-    const size_t gr = (size_t)L->NG * rs * 8, cr = (size_t)L->NC * rs * 8;
-    CK(cudaMemsetAsync(h->d_lw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_alw, 0, gr, h->stream));
-    CK(cudaMemsetAsync(h->d_lh, 0, cr, h->stream));
-    CK(cudaMemsetAsync(h->d_alh, 0, cr, h->stream));
     // w ~ Gamma(aw, scale bw/aw), h ~ Gamma(ah, scale bh/ah); lw = ew = w, lh = eh = h (:111-115,170)
     vb::init_random_kernel<<<cdiv(h->n * r, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         h->n, r, rs, L->d_gene_dev, 0, 0, (unsigned long long)seed, hyper[0], hyper[1] / hyper[0],
@@ -2456,14 +2413,13 @@ int vbnmf_init_random(vbnmf_handle *h, int r, const double hyper[4], uint64_t se
         h->m, r, rs, L->d_cell_dev, 1, cell_offset, (unsigned long long)seed, hyper[2],
         hyper[3] / hyper[2], h->d_lh, h->d_alh, h->tsplit);
     h->launches += 2;
-    if ((rc = refresh_mirrors(h))) return rc;
-    return initial_ehsum(h);
+    return loaded_state(h);
 }
 
 int vbnmf_init_svd2(vbnmf_handle *h, int r, const double hyper[4], uint64_t seed,
                     int64_t cell_offset) {
     if (!h || !hyper) return VBNMF_ERR_ARG;
-    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    if (int rc = check_rank(h, r)) return rc;
     if (!(hyper[3] > 0) || cell_offset < 0) return fail(h, VBNMF_ERR_ARG, "bh must be positive");
     if (r > std::min(h->n, h->m_global)) return fail(h, VBNMF_ERR_ARG, "rank exceeds min(n, m)");
     CK(cudaSetDevice(h->device));
@@ -2476,7 +2432,7 @@ int vbnmf_init_svd2(vbnmf_handle *h, int r, const double hyper[4], uint64_t seed
 
 int vbnmf_init_svd(vbnmf_handle *h, int r, uint64_t seed, int64_t cell_offset) {
     if (!h) return VBNMF_ERR_ARG;
-    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    if (int rc = check_rank(h, r)) return rc;
     if (cell_offset < 0) return fail(h, VBNMF_ERR_ARG, "cell_offset must be >= 0");
     if (r > std::min(h->n, h->m_global)) return fail(h, VBNMF_ERR_ARG, "rank exceeds min(n, m)");
     CK(cudaSetDevice(h->device));
@@ -2488,18 +2444,10 @@ int vbnmf_init_svd(vbnmf_handle *h, int r, uint64_t seed, int64_t cell_offset) {
 
 int vbnmf_step(vbnmf_handle *h, const double hyper[4], double fudge, double *lkh) {
     if (!h || !hyper || !lkh) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
-    CK(cudaSetDevice(h->device));
     int rc;
-    if (!h->stats_valid) {
-        // the statistics pass must not disturb the H-side sums already in the reduce buffer
-        std::vector<double> keep((size_t)h->rs + 8, 0.0);
-        for (int k = 0; k < h->r; k++) keep[k] = h->ehsum[k];
-        if ((rc = sweep(h))) return rc;
-        CK(cudaMemcpyAsync(h->d_red + tail_off(h), keep.data(), (size_t)h->rs * 8,
-                           cudaMemcpyHostToDevice, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
+    if ((rc = check_state(h))) return rc;
+    CK(cudaSetDevice(h->device));
+    if ((rc = ensure_stats(h))) return rc;
     return iterate(h, hyper, fudge, lkh);
 }
 
@@ -2513,23 +2461,17 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
     CK(cudaSetDevice(h->device));
     int rc;
     const int rs = h->rs, r = h->r, itmax = cfg->itmax;
-    if (!h->stats_valid) {
-        std::vector<double> keep((size_t)rs + 8, 0.0);
-        for (int k = 0; k < r; k++) keep[k] = h->ehsum[k];
-        if ((rc = sweep(h))) return rc;
-        CK(cudaMemcpyAsync(h->d_red + tail_off(h), keep.data(), (size_t)rs * 8,
-                           cudaMemcpyHostToDevice, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
+    if ((rc = ensure_stats(h))) return rc;
     // control block: hypers, lk0 = 0 (R/bayesian.R:336), rowSums(eh) of the loaded state
     double *c = h->h_ctl;
     for (int i = 0; i < vb::kCtlLen; i++) c[i] = 0.0;
     for (int q = 0; q < 4; q++) c[vb::kCtlHyper + q] = hyper[q];
     for (int k = 0; k < r; k++) c[vb::kCtlEhsum + k] = h->ehsum[k];
     CK(cudaMemcpyAsync(h->d_ctl, c, vb::kCtlLen * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    ScopedBufs B(h);
     double *d_trace = nullptr, *d_htrace = nullptr;
-    CK(vmalloc(h, &d_trace, (size_t)itmax * 8));
-    CK(vmalloc(h, &d_htrace, (size_t)itmax * 32));
+    CK(B.get(&d_trace, (size_t)itmax * 8));
+    CK(B.get(&d_htrace, (size_t)itmax * 32));
     vb::ControlArgs ca;
     ca.ctl = h->d_ctl;
     ca.scal = h->d_scal;
@@ -2539,18 +2481,8 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
     ca.n = (double)h->n; ca.m_global = (double)h->m_global; ca.lgx = h->lgx; ca.tol = cfg->tol;
     ca.r = r; ca.rs = rs; ca.itmax = itmax; ca.n0 = cfg->n0; ca.dn = cfg->dn;
     for (int q = 0; q < 4; q++) ca.flags[q] = cfg->hyper_update[q];
-    // from here on the kernels read the stop flag and the hypers from the control block; the
-    // guard restores the host-controlled mode on every exit path
-    struct CtlGuard {
-        H *h;
-        double *t0, *t1;
-        ~CtlGuard() {
-            h->ctl = nullptr;
-            vfree(h->stream, t0);
-            vfree(h->stream, t1);
-        }
-    } guard{h, d_trace, d_htrace};
-    h->ctl = h->d_ctl;
+    // from here on the kernels read the stop flag and the hypers from the control block
+    DeviceControl dc(h);
     const int batch = 8;
     int launched = 0, it = 0;
     bool done = false;
@@ -2568,7 +2500,6 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
     } gg;
     const bool use_graph = !ev && h->nranks == 1 && itmax >= 4 * batch && h->nnz <= kGraphMaxNnz &&
                            !getenv("VBNMF_NO_GRAPH");
-    auto finish = [&](int code) { return code; };
     auto enqueue = [&](int gi) -> int {
         if ((rc = launch_posterior(h, true, 0, 0, cfg->fudge))) return rc;
         if ((rc = launch_posterior(h, false, 0, 0, cfg->fudge))) return rc;
@@ -2592,7 +2523,7 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
         cudaError_t ce = cudaStreamEndCapture(h->stream, &gg.g);
         launches_per_batch = h->launches - l0;
         h->launches = l0;
-        if (rc) return finish(rc);
+        if (rc) return rc;
         CK(ce);
         CK(cudaGraphInstantiate(&gg.x, gg.g, 0));
     }
@@ -2603,7 +2534,7 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
             h->launches += launches_per_batch;
         } else {
             for (int b = 0; b < nb; b++)
-                if ((rc = enqueue(launched + b))) return finish(rc);
+                if ((rc = enqueue(launched + b))) return rc;
         }
         launched += nb;
         CK(cudaMemcpyAsync(c, h->d_ctl, vb::kCtlLen * sizeof(double), cudaMemcpyDeviceToHost,
@@ -2620,7 +2551,7 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
         CK(cudaMemcpyAsync(hyper_trace, d_htrace, (size_t)it * 32, cudaMemcpyDeviceToHost,
                            h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    if ((rc = peer_exit_barrier(h))) return finish(rc);
+    if ((rc = peer_exit_barrier(h))) return rc;
     for (int k = 0; k < r; k++) {
         h->bew[k] = c[vb::kCtlBew + k];
         h->beh[k] = c[vb::kCtlBeh + k];
@@ -2635,14 +2566,14 @@ static int run_device_loop(H *h, const vbnmf_cfg *cfg, double hyper[4], double *
     *lml = c[vb::kCtlLk0];                                                  // R/bayesian.R:379
     *stop_reason = (int)c[vb::kCtlReason];
     if (c[vb::kCtlHyperErr] != 0.0)
-        return finish(fail(h, VBNMF_ERR_HYPER, "Hyper-parameter update failed to converge"));
-    return finish(0);
+        return fail(h, VBNMF_ERR_HYPER, "Hyper-parameter update failed to converge");
+    return 0;
 }
 
 int vbnmf_run(vbnmf_handle *h, const vbnmf_cfg *cfg, double hyper[4], double *lkh_trace,
               double *hyper_trace, int *niter, double *lml, int *stop_reason) {
     if (!h || !cfg || !hyper || !niter || !lml || !stop_reason) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+    if (int rc = check_state(h)) return rc;
     if (cfg->itmax < 1 || cfg->dn < 1) return fail(h, VBNMF_ERR_ARG, "itmax and dn must be >= 1");
     if (!getenv("VBNMF_HOST_LOOP"))
         return run_device_loop(h, cfg, hyper, lkh_trace, hyper_trace, niter, lml, stop_reason,
@@ -2683,7 +2614,7 @@ int vbnmf_get_means(vbnmf_handle *h, double means[4]) {
 int vbnmf_get_state(vbnmf_handle *h, double *lw, double *lh, double *ew, double *eh, double *dw,
                     double *dh) {
     if (!h) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+    if (int rc = check_state(h)) return rc;
     CK(cudaSetDevice(h->device));
     CK(cudaStreamSynchronize(h->stream));
     StageTimer tm("vbnmf_get_state(total)");
@@ -2692,9 +2623,10 @@ int vbnmf_get_state(vbnmf_handle *h, double *lw, double *lh, double *ew, double 
     const int r = h->r;
     const int64_t n = h->n, m = h->m;
     const Layout *L = h->L;
+    ScopedBufs B(h);
     double *d_be = nullptr, *d_tmp = nullptr;
-    CK(vmalloc(h, &d_be, 2 * kMaxRank * 8));
-    CK(vmalloc(h, &d_tmp, (size_t)std::max(n, m) * r * 8));
+    CK(B.get(&d_be, 2 * kMaxRank * 8));
+    CK(B.get(&d_tmp, (size_t)std::max(n, m) * r * 8));
     CK(cudaMemcpyAsync(d_be, h->bew, kMaxRank * 8, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(d_be + kMaxRank, h->beh, kMaxRank * 8, cudaMemcpyHostToDevice, h->stream));
     auto one = [&](const double *panel, bool wside, int mode, double *out) -> int {
@@ -2712,29 +2644,26 @@ int vbnmf_get_state(vbnmf_handle *h, double *lw, double *lh, double *ew, double 
         CK(cudaStreamSynchronize(h->stream));
         return 0;
     };
-    int rc = 0;
-    if (!rc) rc = one(h->d_lw, true, 0, lw);
-    if (!rc) rc = one(h->d_alw, true, 1, ew);
-    if (!rc) rc = one(h->d_alw, true, 2, dw);
-    if (!rc) rc = one(h->d_lh, false, 0, lh);
-    if (!rc) rc = one(h->d_alh, false, 1, eh);
-    if (!rc) rc = one(h->d_alh, false, 2, dh);
-    vfree(h->stream, d_be);
-    vfree(h->stream, d_tmp);
-    if (!rc) CK(cudaGetLastError());
-    return rc;
+    int rc;
+    if ((rc = one(h->d_lw, true, 0, lw)) || (rc = one(h->d_alw, true, 1, ew)) ||
+        (rc = one(h->d_alw, true, 2, dw)) || (rc = one(h->d_lh, false, 0, lh)) ||
+        (rc = one(h->d_alh, false, 1, eh)) || (rc = one(h->d_alh, false, 2, dh)))
+        return rc;
+    CK(cudaGetLastError());
+    return 0;
 }
 
 int vbnmf_cluster_id(vbnmf_handle *h, int32_t *cid) {
     if (!h || !cid) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+    if (int rc = check_state(h)) return rc;
     CK(cudaSetDevice(h->device));
     const Layout *L = h->L;
+    ScopedBufs B(h);
     double *d_beh = nullptr;
     int32_t *d_cid = nullptr, *d_out = nullptr;
-    CK(vmalloc(h, &d_beh, kMaxRank * 8));
-    CK(vmalloc(h, &d_cid, (size_t)L->NC * 4));
-    CK(vmalloc(h, &d_out, (size_t)h->m * 4));
+    CK(B.get(&d_beh, kMaxRank * 8));
+    CK(B.get(&d_cid, (size_t)L->NC * 4));
+    CK(B.get(&d_out, (size_t)h->m * 4));
     CK(cudaMemcpyAsync(d_beh, h->beh, kMaxRank * 8, cudaMemcpyHostToDevice, h->stream));
     vb::cluster_id_kernel<<<cdiv(L->NC, vb::kBlock), vb::kBlock, 0, h->stream>>>(
         L->NC, h->rs, h->r, h->d_alh, d_beh, d_cid);
@@ -2742,29 +2671,25 @@ int vbnmf_cluster_id(vbnmf_handle *h, int32_t *cid) {
         h->m, L->d_cell_dev, d_cid, d_out);
     CK(cudaMemcpyAsync(cid, d_out, (size_t)h->m * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, d_beh);
-    vfree(h->stream, d_cid);
-    vfree(h->stream, d_out);
     CK(cudaGetLastError());
     return 0;
 }
 
 int vbnmf_uniform_columns(vbnmf_handle *h, double tol, int32_t *flags) {
     if (!h || !flags) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+    if (int rc = check_state(h)) return rc;
     CK(cudaSetDevice(h->device));
     const Layout *L = h->L;
+    ScopedBufs B(h);
     double *d_bew = nullptr;
     int32_t *d_fl = nullptr;
-    CK(vmalloc(h, &d_bew, kMaxRank * 8));
-    CK(vmalloc(h, &d_fl, kMaxRank * 4));
+    CK(B.get(&d_bew, kMaxRank * 8));
+    CK(B.get(&d_fl, kMaxRank * 4));
     CK(cudaMemcpyAsync(d_bew, h->bew, kMaxRank * 8, cudaMemcpyHostToDevice, h->stream));
     vb::uniform_columns_kernel<<<h->r, vb::kBlock, 0, h->stream>>>(
         L->NG, L->T, L->Sg, h->n, h->rs, h->d_alw, d_bew, tol, d_fl);
     CK(cudaMemcpyAsync(flags, d_fl, (size_t)h->r * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    vfree(h->stream, d_bew);
-    vfree(h->stream, d_fl);
     CK(cudaGetLastError());
     return 0;
 }
@@ -2772,7 +2697,7 @@ int vbnmf_uniform_columns(vbnmf_handle *h, double tol, int32_t *flags) {
 int vbnmf_bench_iterations(vbnmf_handle *h, double hyper[4], double fudge, int iters,
                            int hyper_on, double ms[4], int64_t *launches, double *lkh_last) {
     if (!h || !hyper || !ms || iters < 1) return VBNMF_ERR_ARG;
-    if (!h->d_lw) return fail(h, VBNMF_ERR_STATE, "vbnmf_set_state has not been called");
+    if (int rc = check_state(h)) return rc;
     CK(cudaSetDevice(h->device));
     int rc;
     double lkh = 0.0;
@@ -2781,7 +2706,11 @@ int vbnmf_bench_iterations(vbnmf_handle *h, double hyper[4], double fudge, int i
     // triggers, CUDA events around the two sweep passes.  hyper_on = 1: hyper_update after every
     // iteration, i.e. the steady state of the reference loop past hyper.update.n0
     // (R/bayesian.R:342), hyper[] is updated; 0: hyper-parameters held fixed.
-    std::vector<cudaEvent_t> ev((size_t)iters * 4 + 2);
+    std::vector<cudaEvent_t> ev((size_t)iters * 4 + 2, nullptr);
+    struct DestroyEvents {  // on every return
+        std::vector<cudaEvent_t> &e;
+        ~DestroyEvents() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+    } destroy_events{ev};
     for (auto &e : ev) CK(cudaEventCreate(&e));
     vbnmf_cfg cfg;
     cfg.itmax = iters; cfg.tol = -1.0; cfg.n0 = hyper_on ? 0 : 1 << 30; cfg.dn = 1;
@@ -2808,7 +2737,6 @@ int vbnmf_bench_iterations(vbnmf_handle *h, double hyper[4], double fudge, int i
         ms[2] += t;
     }
     ms[3] = ms[0] - ms[1] - ms[2];
-    for (auto &e : ev) cudaEventDestroy(e);
     for (int q = 0; q < 4; q++) hyper[q] = hy[q];
     if (launches) *launches = h->launches - l0;
     if (lkh_last) *lkh_last = h->h_ctl[vb::kCtlLkh];
@@ -2847,14 +2775,14 @@ int mlnmf_run2(vbnmf_handle *h, int r, const double *w0, const double *h0, int i
                int criterion, int ncnn_step, double *w, double *h_out, double *lik_trace,
                double *nchange_trace, int *niter) {
     if (!h || !w0 || !h0 || !niter || itmax < 1) return VBNMF_ERR_ARG;
-    if (r < 1 || r > kMaxRank) return fail(h, VBNMF_ERR_ARG, "rank must be in 1..64");
+    if (int rc = check_rank(h, r)) return rc;
     if (criterion != VBNMF_ML_LIKELIHOOD && criterion != VBNMF_ML_CONNECTIVITY)
         return fail(h, VBNMF_ERR_ARG, "Unknown stopping criterion.");   // R/factorize.R:212
     if (criterion == VBNMF_ML_CONNECTIVITY && ncnn_step < 1)
         return fail(h, VBNMF_ERR_ARG, "ncnn_step must be >= 1");
     CK(cudaSetDevice(h->device));
     int rc;
-    if ((rc = alloc_panels(h, r))) return rc;
+    if ((rc = alloc_panels(h, r))) return rc;  // (lw and lh only: the ML path has no alw, alh)
     CK(cudaMemsetAsync(h->d_lw, 0, (size_t)h->L->NG * h->rs * 8, h->stream));
     CK(cudaMemsetAsync(h->d_lh, 0, (size_t)h->L->NC * h->rs * 8, h->stream));
     if ((rc = upload_panel(h, h->d_lw, nullptr, w0, true, r))) return rc;
@@ -2867,17 +2795,14 @@ int mlnmf_run2(vbnmf_handle *h, int r, const double *w0, const double *h0, int i
     const int rs = h->rs, wd = rs + 8;
     double *tail = h->d_red + tail_off(h);
     // connectivity criterion: labels of the previous and the current h, their contingency table
+    ScopedBufs B(h);
     int32_t *d_lab[2] = {nullptr, nullptr};
     double *d_cont = nullptr;
     std::vector<double> cont;
-    struct Guard {
-        cudaStream_t s; int32_t **l; double **c;
-        ~Guard() { vfree(s, l[0]); vfree(s, l[1]); vfree(s, *c); }
-    } guard{h->stream, d_lab, &d_cont};
     if (criterion == VBNMF_ML_CONNECTIVITY) {
-        CK(vmalloc(h, &d_lab[0], (size_t)L->NC * 4));
-        CK(vmalloc(h, &d_lab[1], (size_t)L->NC * 4));
-        CK(vmalloc(h, &d_cont, (size_t)r * r * 8));
+        CK(B.get(&d_lab[0], (size_t)L->NC * 4));
+        CK(B.get(&d_lab[1], (size_t)L->NC * 4));
+        CK(B.get(&d_cont, (size_t)r * r * 8));
         cont.resize((size_t)r * r);
     }
     auto colsum = [&](bool wside) -> int {
@@ -2944,13 +2869,10 @@ int mlnmf_run2(vbnmf_handle *h, int r, const double *w0, const double *h0, int i
         for (int i = 0; i < vb::kCtlLen; i++) c[i] = 0.0;
         c[vb::kCtlLk0] = -INFINITY;                                        // lkold, :190
         CK(cudaMemcpyAsync(h->d_ctl, c, vb::kCtlLen * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        ScopedBufs Bt(h);
         double *d_trace = nullptr;
-        CK(vmalloc(h, &d_trace, (size_t)itmax * 8));
-        struct CtlGuard {
-            H *h; double *t;
-            ~CtlGuard() { h->ctl = nullptr; vfree(h->stream, t); }
-        } cg{h, d_trace};
-        h->ctl = h->d_ctl;
+        CK(Bt.get(&d_trace, (size_t)itmax * 8));
+        DeviceControl dc(h);
         vb::MlControlArgs ca{h->d_ctl, h->d_scal, tail, d_trace, (double)h->n, (double)h->m_global,
                              h->mlconst, tol, r, rs, itmax};
         int turns = 0;

@@ -31,42 +31,44 @@ class Engine:
     `counts(object)` of an scNMFSet (R/bayesian.R:239).
     """
 
-    def __init__(self, counts=None, device=0, _device_csc=None):
+    def __init__(self, counts=None, device=0):
+        import scipy.sparse as sp
+        csc = counts if sp.isspmatrix_csc(counts) else sp.csc_matrix(counts)
+        if not csc.has_sorted_indices:
+            csc = csc.copy()
+            csc.sort_indices()
+        n, m = csc.shape
+        rowidx = np.ascontiguousarray(csc.indices, dtype=np.int32)
+        values = np.ascontiguousarray(csc.data, dtype=np.float64)
+        p32 = p64 = None
+        if csc.indptr.dtype == np.int32:  # dgCMatrix @p is int32
+            ptr = np.ascontiguousarray(csc.indptr)
+            p32 = ptr.ctypes.data_as(_lib.c_i32p)
+        else:
+            ptr = np.ascontiguousarray(csc.indptr, dtype=np.int64)
+            p64 = ptr.ctypes.data_as(_lib.c_i64p)
+        self._open(lambda out: self.lib.vbnmf_create(out, n, m, csc.nnz, p32, p64,
+                                                     rowidx.ctypes.data_as(_lib.c_i32p),
+                                                     _dp(values), int(device)), device)
+
+    def _open(self, create, device, keep=None):
+        """Make this Engine the owner of the handle create(out) makes (out: where the library
+        stores it); keep: objects that must outlive the handle."""
         self.lib = _lib.load()
         self.handle = C.c_void_p()
-        self._keep = None
+        self._keep = keep
         self.device = int(device)
-        if _device_csc is not None:
-            n, m, nnz, d_colptr, d_rowidx, d_val, keep = _device_csc
-            self._keep = keep  # borrowed device arrays must outlive the handle
-            rc = self.lib.vbnmf_create_from_device(C.byref(self.handle), n, m, nnz,
-                                                   C.c_void_p(d_colptr), C.c_void_p(d_rowidx),
-                                                   C.c_void_p(d_val), int(device))
-        else:
-            import scipy.sparse as sp
-            csc = counts if sp.isspmatrix_csc(counts) else sp.csc_matrix(counts)
-            if not csc.has_sorted_indices:
-                csc = csc.copy()
-                csc.sort_indices()
-            n, m = csc.shape
-            nnz = csc.nnz
-            rowidx = np.ascontiguousarray(csc.indices, dtype=np.int32)
-            values = np.ascontiguousarray(csc.data, dtype=np.float64)
-            p32 = p64 = None
-            if csc.indptr.dtype == np.int32:  # dgCMatrix @p is int32
-                ptr = np.ascontiguousarray(csc.indptr)
-                p32 = ptr.ctypes.data_as(_lib.c_i32p)
-            else:
-                ptr = np.ascontiguousarray(csc.indptr, dtype=np.int64)
-                p64 = ptr.ctypes.data_as(_lib.c_i64p)
-            rc = self.lib.vbnmf_create(C.byref(self.handle), n, m, nnz, p32, p64,
-                                       rowidx.ctypes.data_as(_lib.c_i32p), _dp(values), int(device))
-        if rc != 0:
-            msg = self.lib.vbnmf_last_error(None)
-            self.handle = C.c_void_p()
-            raise _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
-        self.n, self.m, self.nnz = int(n), int(m), int(nnz)
+        _lib.check(create(C.byref(self.handle)))
+        info = self.info()
+        self.n, self.m, self.nnz = int(info["n"]), int(info["m"]), int(info["nnz"])
         self.r = 0
+
+    @classmethod
+    def _create(cls, create, device, keep=None):
+        """An Engine around the handle create(out) makes."""
+        self = cls.__new__(cls)
+        self._open(create, device, keep)
+        return self
 
     @classmethod
     def from_device_csc(cls, n, m, nnz, colptr_i64, rowidx_i32, values_f32, device=0):
@@ -77,28 +79,20 @@ class Engine:
         bound: the sum of lgamma(x + 1) came out short while the factors were right)."""
         import torch
         torch.cuda.current_stream(torch.device("cuda", int(device))).synchronize()
-        keep = (colptr_i64, rowidx_i32, values_f32)
-        return cls(device=device, _device_csc=(int(n), int(m), int(nnz), colptr_i64.data_ptr(),
-                                               rowidx_i32.data_ptr(), values_f32.data_ptr(), keep))
+        lib = _lib.load()
+        # the borrowed device arrays must outlive the handle
+        return cls._create(lambda out: lib.vbnmf_create_from_device(
+            out, int(n), int(m), int(nnz), C.c_void_p(colptr_i64.data_ptr()),
+            C.c_void_p(rowidx_i32.data_ptr()), C.c_void_p(values_f32.data_ptr()), int(device)),
+            device, keep=(colptr_i64, rowidx_i32, values_f32))
 
     @classmethod
     def from_mtx(cls, path, device=0):
         """MatrixMarket coordinate file (10x `matrix.mtx`) parsed and sorted into CSC on the GPU
         (readMM + as(., 'dgCMatrix') of read_10x, R/utils.R:34)."""
-        self = cls.__new__(cls)
-        self.lib = _lib.load()
-        self.handle = C.c_void_p()
-        self._keep = None
-        self.device = int(device)
-        dims = (C.c_int64 * 3)()
-        rc = self.lib.vbnmf_create_from_mtx(C.byref(self.handle), str(path).encode(), int(device), dims)
-        if rc != 0:
-            msg = self.lib.vbnmf_last_error(None)
-            self.handle = C.c_void_p()
-            raise _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
-        self.n, self.m, self.nnz = int(dims[0]), int(dims[1]), int(dims[2])
-        self.r = 0
-        return self
+        lib = _lib.load()
+        return cls._create(lambda out: lib.vbnmf_create_from_mtx(out, str(path).encode(), int(device),
+                                                                 None), device)
 
     def csc(self):
         """The count matrix the handle holds, as a scipy CSC matrix."""
@@ -147,9 +141,9 @@ class Engine:
                 raise ValueError("col_scale must be finite")
         rows = np.ascontiguousarray(keep_rows, dtype=np.uint8)
         cols = np.ascontiguousarray(keep_cols, dtype=np.uint8)
-        return self._derived(lambda out: self.lib.vbnmf_create_subset(
+        return Engine._create(lambda out: self.lib.vbnmf_create_subset(
             out, self.handle, rows.ctypes.data_as(_lib.c_u8p), cols.ctypes.data_as(_lib.c_u8p),
-            _dp(scale)))
+            _dp(scale)), self.device)
 
     def shuffle(self, seed):
         """A new Engine on the same device holding this engine's matrix with every column shuffled
@@ -158,25 +152,8 @@ class Engine:
         keyed by (seed, column); synth.shuffle_columns_reference is the CPU restatement.  Built
         from this engine's device arrays: nothing crosses the bus.  This engine is left as it
         was."""
-        return self._derived(lambda out: self.lib.vbnmf_create_shuffled(
-            out, self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF))
-
-    def _derived(self, create):
-        """An Engine around the handle create(out) makes from this engine's handle."""
-        out = Engine.__new__(Engine)
-        out.lib = self.lib
-        out.handle = C.c_void_p()
-        out._keep = None
-        out.device = self.device
-        rc = create(C.byref(out.handle))
-        if rc != 0:
-            msg = self.lib.vbnmf_last_error(None)
-            out.handle = C.c_void_p()
-            raise _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
-        info = out.info()
-        out.n, out.m, out.nnz = int(info["n"]), int(info["m"]), int(info["nnz"])
-        out.r = 0
-        return out
+        return Engine._create(lambda out: self.lib.vbnmf_create_shuffled(
+            out, self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF), self.device)
 
     # -- lifetime ------------------------------------------------------------------------------
     def close(self):
@@ -394,11 +371,11 @@ def consensus(labels, device=0, tree=True, max_groups=0):
                              mom.ctypes.data_as(_lib.c_i64p), C.byref(ng),
                              None if merges is None else merges.ctypes.data_as(_lib.c_i64p), cap,
                              C.byref(resc))
-    if rc != 0:
-        msg = lib.vbnmf_last_error(None)
-        err = _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
+    try:
+        _lib.check(rc)
+    except _lib.VbnmfError as err:
         err.ngroups = ng.value
-        raise err
+        raise
     out = dict(s1=int(mom[0]), s2=int(mom[1]))
     if tree:
         G = ng.value
@@ -413,10 +390,8 @@ class Comm:
         self.lib = _lib.load()
         self.ptr = C.c_void_p()
         buf = (C.c_char * 128).from_buffer_copy(uid)
-        rc = self.lib.vbnmf_comm_create(C.byref(self.ptr), int(nranks), int(rank), buf, int(device))
-        if rc != 0:
-            msg = self.lib.vbnmf_last_error(None)
-            raise _lib.VbnmfError(rc, msg.decode() if msg else "unknown")
+        _lib.check(self.lib.vbnmf_comm_create(C.byref(self.ptr), int(nranks), int(rank), buf,
+                                              int(device)))
         self.nranks, self.rank = int(nranks), int(rank)
 
     def close(self):
