@@ -40,8 +40,6 @@ if os.environ.get("VBNMF_SPLIT_PRED"):
     NVCC_FLAGS.append("-DVB_SPLIT_PRED=" + os.environ["VBNMF_SPLIT_PRED"])
 if os.environ.get("VBNMF_SKIP_DEAD"):
     NVCC_FLAGS.append("-DVB_SKIP_DEAD=" + os.environ["VBNMF_SKIP_DEAD"])
-if os.environ.get("VBNMF_LP_IMMEDIATE"):
-    NVCC_FLAGS.append("-DVB_LP_IMMEDIATE=" + os.environ["VBNMF_LP_IMMEDIATE"])
 if os.environ.get("VBNMF_DOT_CHAINS"):
     NVCC_FLAGS.append("-DVB_DOT_CHAINS=" + os.environ["VBNMF_DOT_CHAINS"])
 for _d in os.environ.get("VBNMF_DEFS", "").split():   # experiments: "VB_X=1 VB_Y=0" -> -DVB_X=1 ...

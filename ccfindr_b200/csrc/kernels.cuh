@@ -16,12 +16,6 @@
 #define VB_SKIP_DEAD 1    // split kernels: skip the all-hole steps at the end of a segment (their
                           // number rides in the low 2 bits of the segment's quad pointer)
 #endif
-#ifndef VB_LP_IMMEDIATE
-#define VB_LP_IMMEDIATE 0 // 1: large counts of the log-product bound term take their log at once
-                          // (group vote per nonzero) instead of per chunk from kept p values.
-                          // Measured SLOWER at r = 20 (cell-owner pass 3.06 -> 4.15 ms): the vote
-                          // serialises the four nonzeros of a chunk, and the spills stay
-#endif
 #ifndef VB_DOT_CHAINS
 #define VB_DOT_CHAINS 2   // independent FMA chains of the rank-r dot product (fp64)
 #endif
@@ -171,6 +165,9 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, unsigned bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
                  "r"(bytes)
                  : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, unsigned parity) {
     unsigned ok;
@@ -733,56 +730,50 @@ __device__ __forceinline__ void halve_reduce_store(const double (&v0)[N], int gl
     }
 }
 
-// x log p of the fp64 cell-owner pass through products (integer counts): with p = 2^e m,
-//   sum x log p = ln2 * sum x e + sum_b 2^b log( prod_{bit b of x set} m ),   b < kLpBits,
-// so a nonzero costs kLpBits predicated multiplies and a few integer operations instead of a
-// log (~35 instructions).  The mantissa products stay below 2^(T/8) <= 2^512 within a segment and
-// are renormalised at its end.  Counts >= 2^kLpBits take the log in an out-of-line slow path.
+// x log p of the fp64 cell-owner pass through products (integer counts): with p = 2^e m and
+// x' = x mod 2^kLpBits,
+//   sum x' log p = ln2 * sum x' e + log prod m^x',   m^x' = prod_{bit b of x' set} m^(2^b),
+// so a nonzero costs kLpBits - 1 squarings, kLpBits selected multiplies and a few integer
+// operations instead of a log (~35 instructions), and the state is one product, one exponent sum
+// and one accumulator.  The product grows by less than 2^(4 (2^kLpBits - 1)) per chunk of four
+// nonzeros and is renormalised after each.  The rest of a count >= 2^kLpBits, (x - x') log p,
+// takes the log in an out-of-line slow path.
 #ifndef VB_LP_BITS
-#define VB_LP_BITS 3   // 4 keeps counts up to 15 in the fast path (data with heavier tails) at no
-                       // cost at r = 10 and +3 % on the cell-owner pass at r = 20 (register spills)
+#define VB_LP_BITS 3   // 4 keeps counts up to 15 in the fast path (data with heavier tails)
 #endif
 constexpr int kLpBits = VB_LP_BITS;
 struct LogProd {
-    double P[kLpBits];
-    int E;          // sum x e of the current segment
-    double Es;      // ... of the finished ones (exact integer), and the slow-path terms
-    double slow;
-    __device__ __forceinline__ void init() {
-#pragma unroll
-        for (int b = 0; b < kLpBits; b++) P[b] = 1.0;
-        E = 0; Es = 0.0; slow = 0.0;
-    }
-    __device__ __forceinline__ void add(int xi, double p) {
+    double P;       // prod m^(x mod 2^kLpBits), renormalised to [1, 2) after every chunk
+    int E;          // sum x e and the exponents taken out of P, of the current segment
+    double sum;     // ln2 E of the finished segments and the slow-path terms
+    __device__ __forceinline__ void init() { P = 1.0; E = 0; sum = 0.0; }
+    // v: packed entry, count in the high 16 bits
+    __device__ __forceinline__ void add(uint32_t v, double p) {
         const int hi = __double2hiint(p);
-        const int e = ((hi >> 20) & 0x7ff) - 1023;
-        const double m = __hiloint2double((hi & 0x000fffff) | 0x3ff00000, __double2loint(p));
-        const int xm = xi < (1 << kLpBits) ? xi : 0;
-        E += xm * e;
-#pragma unroll
-        for (int b = 0; b < kLpBits; b++)
-            if ((xm >> b) & 1) P[b] *= m;
-    }
-    // counts >= 2^kLpBits (rare): called once per chunk, inside a branch taken only if one occurred
-    __device__ __forceinline__ void add_slow(int xi, double p) {
-        if (xi >= (1 << kLpBits)) slow = fma((double)xi, fast_log_pos(p), slow);
-    }
-    __device__ __forceinline__ void end_segment() {
+        const int e = (hi >> 20) - 1023;  // p > 0: the sign bit is clear
+        double m = __hiloint2double(hi - (e << 20), __double2loint(p));
+        E += (int)((v >> 16) & ((1u << kLpBits) - 1u)) * e;
 #pragma unroll
         for (int b = 0; b < kLpBits; b++) {
-            const int hi = __double2hiint(P[b]);
-            E += (((hi >> 20) & 0x7ff) - 1023) << b;
-            P[b] = __hiloint2double((hi & 0x000fffff) | 0x3ff00000, __double2loint(P[b]));
+            if (b) m *= m;
+            if ((v >> (16 + b)) & 1u) P *= m;
         }
-        Es += (double)E;
+    }
+    __device__ __forceinline__ void renorm() {
+        const int hi = __double2hiint(P);
+        const int e = (hi >> 20) - 1023;
+        E += e;
+        P = __hiloint2double(hi - (e << 20), __double2loint(P));
+    }
+    // counts >= 2^kLpBits (rare): the bits above the low kLpBits
+    __device__ __forceinline__ void add_slow(uint32_t v, double p) {
+        sum = fma((double)(int)((v >> (16 + kLpBits)) << kLpBits), fast_log_pos(p), sum);
+    }
+    __device__ __forceinline__ void end_segment() {
+        sum = fma((double)E, 0.6931471805599453094, sum);
         E = 0;
     }
-    __device__ __forceinline__ double total() const {
-        double t = slow + Es * 0.6931471805599453094;
-#pragma unroll
-        for (int b = 0; b < kLpBits; b++) t += (double)(1 << b) * log(P[b]);
-        return t;
-    }
+    __device__ __forceinline__ double total() const { return sum + log(P); }
 };
 
 // SPLIT (fp64 panels, one lane per nonzero, rows of >= 8 units; see split_rank / panel_ofs): the
@@ -834,25 +825,38 @@ sweep_p16_kernel(const SweepTiledArgs a) {
     const uint32_t tile_s = smem_u32(tile);
     __shared__ __align__(8) uint64_t mbar;
     __shared__ double red[NT / 32];
+    __shared__ uint32_t range_end;  // e1 below, read once per slab instead of held in a register
     const int gid = threadIdx.x / G, gl = threadIdx.x % G;
     const int l8 = threadIdx.x & 7;  // lane in the quarter-warp (bank phase): rotation of the gathers
     const int slot = gl / LPN, hf = gl % LPN;
     const unsigned gmask = ((1u << G) - 1u) << ((threadIdx.x & 31) & ~(G - 1));
-    const int64_t e0 = a.split[blockIdx.x], e1 = a.split[blockIdx.x + 1];
+    const unsigned pmask = 3u << ((threadIdx.x & 31) & ~1);  // the two lanes of a nonzero (LPN == 2)
+    // segment positions fit in 32 bits with a group stride to spare (build_pass checks it)
+    const uint32_t e0 = (uint32_t)a.split[blockIdx.x], e1 = (uint32_t)a.split[blockIdx.x + 1];
+    const uint32_t NO = (uint32_t)a.NO;
     const unsigned tile_bytes = (unsigned)a.T * PSS * (unsigned)sizeof(PT);
     const uint4 *ent4 = reinterpret_cast<const uint4 *>(a.ent);
     if (a.ctl && a.ctl[kCtlDone] != 0.0) return;
-    if (threadIdx.x == 0) mbar_init(&mbar, 1);
+    // the tile barrier completes one phase per slab; its phase parity is kept equal to the parity
+    // of the slab index (one empty phase first when the CTA starts at an odd slab), so that no
+    // register has to count the phases
+    if (threadIdx.x == 0) {
+        range_end = e1;
+        mbar_init(&mbar, 1);
+        if ((e0 / NO) & 1u) mbar_arrive(&mbar);
+    }
     __syncthreads();
-    unsigned parity = 0;
     double xl = 0.0;
     constexpr bool kLogProd = COLS && sizeof(PT) == 8;  // fp64 cell-owner pass: log-product
     LogProd lp;
     if (kLogProd) lp.init();
 
-    const uint32_t tileB_s = tile_s + (uint32_t)a.T * (uint32_t)(SA * 16);
-    const uint32_t rot = (uint32_t)(l8 & (SA - 1)) << 4;
-    const uint32_t rotb = kRotB ? (uint32_t)((l8 >> 2) & 1) << 4 : 0u;
+    // tile bases of the split layout plus this lane's rotation: a row of block A starts at a
+    // multiple of SA * 16 bytes, one of block B with kRotB at a multiple of 32, so that adding the
+    // rotation to the base is XORing it into the row address
+    const uint32_t tileA_r = tile_s + ((uint32_t)(l8 & (SA - 1)) << 4);
+    const uint32_t tileB_r = tile_s + (uint32_t)a.T * (uint32_t)(SA * 16) +
+                             (kRotB ? (uint32_t)((l8 >> 2) & 1) << 4 : 0u);
     if (SPLIT && (tile_s & 127u)) __trap();  // block A rows must start on SA * 16-byte boundaries
 
     // Owner rows.  A lane holds units hf, hf + LPN, ... of the row (SPLIT: in the rotated order of
@@ -921,17 +925,42 @@ sweep_p16_kernel(const SweepTiledArgs a) {
         }
         __syncwarp(gmask);
     };
+    // gather the tile row of packed entry v: this lane's units, in the order of its owner row
+    auto gather = [&](uint32_t v, PT(&dst)[KL]) {
+        if constexpr (SPLIT) {
+            const uint32_t row = v & 0xffffu;
+            const uint32_t ra = tileA_r + row * (uint32_t)(SA * 16);
+            const uint32_t rb = tileB_r + row * (uint32_t)BSB;
+#pragma unroll
+            for (int c = 0; c < SA; c++) lds_unit(ra ^ (uint32_t)(c << 4), dst + c * UE);
+#pragma unroll
+            for (int c = 0; c < NUB; c++)
+                lds_unit(kRotB ? (rb ^ (uint32_t)(c << 4)) : (rb + c * 16), dst + (SA + c) * UE);
+        } else {
+            const uint32_t raddr = tile_s + (v & 0xffffu) * (uint32_t)(PS * sizeof(PT));
+#pragma unroll
+            for (int c = 0; c < NUL; c++) {
+                const int uu = LPN * c + hf;
+                if (LPN == 1 || uu < NU) {
+                    lds_unit(raddr + uu * 16, dst + c * UE);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < UE; j++) dst[c * UE + j] = 0;
+                }
+            }
+        }
+    };
     PT tr[KL];  // the gathered row; SPLIT: kept by hole entries (overwritten in full otherwise)
 #pragma unroll
     for (int k = 0; k < KL; k++) tr[k] = 1;
 
-    for (int64_t ebase = e0; ebase < e1;) {
-        const int64_t slab = ebase / a.NO;
-        const int64_t eend = min(e1, (slab + 1) * a.NO);
+    for (uint32_t ebase = e0; ebase < range_end;) {
+        const uint32_t slab = ebase / NO;
+        const uint32_t eend = min(range_end, (slab + 1) * NO);
         __syncthreads();
         if (threadIdx.x == 0) {
             mbar_expect_tx(&mbar, tile_bytes);
-            bulk_g2s(tile, reinterpret_cast<const PT *>(a.tiles) + slab * (int64_t)a.T * PSS,
+            bulk_g2s(tile, reinterpret_cast<const PT *>(a.tiles) + (int64_t)slab * a.T * PSS,
                      tile_bytes, &mbar);
         }
         // prime the group's pipeline while the tile lands: pointers and owners of its first two
@@ -940,10 +969,11 @@ sweep_p16_kernel(const SweepTiledArgs a) {
         // of consecutive owners the segments are ordered by decreasing length, so that the four
         // groups of a warp, which run their chunk loops in lock step, get segments of (nearly
         // always) the same number of steps.
-        int64_t e = ebase + gid;
+        uint32_t e = ebase + gid;
+        // quad pointers of the current and the next segment; SPLIT: the start pointers carry the
+        // number of all-hole steps at the end of their segment in the low 2 bits until it starts
         uint32_t beg = 0, end = 0, nb = 0, ne = 0;
         uint32_t og = 0, nog = 0;   // owner rows of the current and the next segment
-        uint32_t dead = 0, ndead = 0, nndead = 0;  // all-hole steps at the end of the segment (SPLIT)
         constexpr uint32_t kTag = SPLIT ? 3u : 0u;
         uint4 f0 = make_uint4(0u, 0u, 0u, 0u);
         PT ownn[KL];
@@ -953,21 +983,22 @@ sweep_p16_kernel(const SweepTiledArgs a) {
             beg = __ldg(a.ptr4 + e);
             end = __ldg(a.ptr4 + e + 1) & ~kTag;
             og = __ldg(a.seg + e);
-            dead = beg & kTag; beg &= ~kTag;
             if (e + kGroups < eend) {
                 nb = __ldg(a.ptr4 + e + kGroups);
                 ne = __ldg(a.ptr4 + e + kGroups + 1) & ~kTag;
                 nog = __ldg(a.seg + e + kGroups);
-                ndead = nb & kTag; nb &= ~kTag;
             }
-            if (beg + slot < end) f0 = ldcs_quad(ent4 + beg + slot);
-            if (kOwnMode == 1 || kOwnMode == 2) load_owner(og, beg < end, ownn);
-            if (kOwnMode == 3) stage_owner(og, beg < end);
+            const uint32_t b0 = beg & ~kTag;
+            if (b0 + slot < end) f0 = ldcs_quad(ent4 + b0 + slot);
+            if (kOwnMode == 1 || kOwnMode == 2) load_owner(og, b0 < end, ownn);
+            if (kOwnMode == 3) stage_owner(og, b0 < end);
         }
-        mbar_wait(&mbar, parity);
-        parity ^= 1;
+        mbar_wait(&mbar, slab & 1u);
         while (e < eend) {
-            const int64_t en = e + kGroups;
+            const uint32_t en = e + kGroups;
+            const uint32_t dead = beg & kTag;
+            beg &= ~kTag;
+            const uint32_t nbu = nb & ~kTag;
             const int nq = (int)(end - beg);
             const uint4 *eb = ent4 + beg;
             uint4 cur = f0;
@@ -977,25 +1008,31 @@ sweep_p16_kernel(const SweepTiledArgs a) {
             if (kOwnMode == 0) load_owner(og, nq > 0, own);
             if (kOwnMode == 3) {
                 take_owner(own);   // (a segment without entries reads the previous row: unused)
-                stage_owner(nog, en < eend && nb < ne);
+                stage_owner(nog, en < eend && nbu < ne);
             }
             uint4 n1 = make_uint4(0u, 0u, 0u, 0u);
             if (NPG + slot < nq) n1 = ldcs_quad(eb + NPG + slot);
             // requests for the NEXT segment (pointers arrived during the previous one) and the
-            // pointers of the one after it
+            // pointers of the one after it.  Mode 2: the next segment's first quad and the
+            // pointers of the one after it are requested with its owner row, at the end of this
+            // segment, instead of being held in registers through it (the first quad comes from
+            // L2: the bulk prefetch includes it)
+            constexpr uint32_t kPf = kOwnMode == 2 ? 0u : (uint32_t)NPG;  // first prefetched quad
             uint32_t nnb = 0, nne = 0, nnog = 0;
-            f0 = make_uint4(0u, 0u, 0u, 0u);
-            if (en < eend) {
+            auto load_ptrs = [&]() {
                 if (en + kGroups < eend) {
                     nnb = __ldg(a.ptr4 + en + kGroups);
                     nne = __ldg(a.ptr4 + en + kGroups + 1) & ~kTag;
                     nnog = __ldg(a.seg + en + kGroups);
-                    nndead = nnb & kTag; nnb &= ~kTag;
                 }
-                if (nb + slot < ne) f0 = ldcs_quad(ent4 + nb + slot);
-                if (kOwnMode == 1) load_owner(nog, nb < ne, ownn);
-                if (gl == 0 && nb + NPG < ne)
-                    bulk_prefetch_l2(ent4 + nb + NPG, (ne - nb - NPG) * 16u);
+            };
+            if (kOwnMode != 2) f0 = make_uint4(0u, 0u, 0u, 0u);
+            if (en < eend) {
+                if (kOwnMode != 2) load_ptrs();
+                if (kOwnMode != 2 && nbu + slot < ne) f0 = ldcs_quad(ent4 + nbu + slot);
+                if (kOwnMode == 1) load_owner(nog, nbu < ne, ownn);
+                if (gl == 0 && nbu + kPf < ne)
+                    bulk_prefetch_l2(ent4 + nbu + kPf, (ne - nbu - kPf) * 16u);
             }
             PT acc[KL];
             PT xls = 0;
@@ -1004,69 +1041,48 @@ sweep_p16_kernel(const SweepTiledArgs a) {
             for (int c0 = 0; c0 < nq; c0 += NPG) {
                 uint4 n2 = make_uint4(0u, 0u, 0u, 0u);
                 if (c0 + 2 * NPG + slot < nq) n2 = ldcs_quad(eb + c0 + 2 * NPG + slot);
-                PT pu[4], xu[4];
-                uint32_t big = 0;  // kLogProd: OR of this lane's counts of the chunk
+                PT pu[4], xu[4];   // fp32 cell-owner pass, LPN == 2
                 // steps of this chunk that hold nonzeros (the last chunk of a segment may end in
                 // all-hole steps)
                 const int ulive = (SPLIT && VB_SKIP_DEAD && c0 + NPG >= nq) ? 4 - (int)dead : 4;
+                // kLogProd: a count of the chunk has bits above the low kLpBits
+                const bool big = ((cur.x | cur.y | cur.z | cur.w) >> (16 + kLpBits)) != 0u;
 #pragma unroll
                 for (int u = 0; u < 4; u++) {
                     if (SPLIT && VB_SKIP_DEAD && u > 0 && u >= ulive) break;
                     const uint32_t v = u == 0 ? cur.x : u == 1 ? cur.y : u == 2 ? cur.z : cur.w;
                     const PT x = (PT)(int)(v >> 16);
-                    if constexpr (SPLIT) {
-                        if (!VB_SPLIT_PRED || (v >> 16)) {  // a hole keeps the previous row: no shared-memory traffic
-                            const uint32_t row = v & 0xffffu;
-                            const uint32_t ra = (tile_s + row * (uint32_t)(SA * 16)) ^ rot;
-                            const uint32_t rb = (tileB_s + row * (uint32_t)BSB) ^ rotb;
-#pragma unroll
-                            for (int c = 0; c < SA; c++) lds_unit(ra ^ (uint32_t)(c << 4), tr + c * UE);
-#pragma unroll
-                            for (int c = 0; c < NUB; c++)
-                                lds_unit(kRotB ? (rb ^ (uint32_t)(c << 4)) : (rb + c * 16),
-                                         tr + (SA + c) * UE);
-                        }
-                    } else {
-                        const uint32_t raddr = tile_s + (v & 0xffffu) * (uint32_t)(PS * sizeof(PT));
-#pragma unroll
-                        for (int c = 0; c < NUL; c++) {
-                            const int uu = LPN * c + hf;
-                            if (LPN == 1 || uu < NU) {
-                                lds_unit(raddr + uu * 16, tr + c * UE);
-                            } else {
-#pragma unroll
-                                for (int j = 0; j < UE; j++) tr[c * UE + j] = 0;
-                            }
-                        }
-                    }
+                    // SPLIT: a hole keeps the previous row (no shared-memory traffic)
+                    if (!SPLIT || !VB_SPLIT_PRED || (v >> 16)) gather(v, tr);
                     PT p = dot_rows<KL>(own, tr);
                     if (LPN == 2) p += __shfl_xor_sync(gmask, p, 1);
                     const PT q = x * rcp_t(p);
                     axpy_row<KL>(acc, tr, q);
                     if (kLogProd) {
                         // LPN == 2: both lanes of a pair hold p, each takes every other nonzero
-                        const bool mine = LPN == 1 || (u & 1) == hf;
-                        if (mine) lp.add((int)(v >> 16), (double)p);
-                        if (VB_LP_IMMEDIATE) {
-                            // counts >= 2^kLpBits: the log right here, inside a branch the whole
-                            // group takes together (no p kept for a per-chunk slow path)
-                            if (__any_sync(gmask, mine && (v >> (16 + kLpBits)) != 0u)) {
-                                if (mine) lp.add_slow((int)(v >> 16), (double)p);
-                            }
-                        } else if (mine) {
-                            big |= v;
-                            pu[u] = p;
-                        }
+                        if (LPN == 1 || (u & 1) == hf) lp.add(v, (double)p);
                     } else if (COLS) {
                         if (LPN == 1) xls = fma(x, log_t(p), xls);
                         else { pu[u] = p; xu[u] = x; }
                     }
                 }
-                if (kLogProd && !VB_LP_IMMEDIATE && big >= (1u << (16 + kLpBits))) {
-                    const uint32_t cv[4] = {cur.x, cur.y, cur.z, cur.w};
-#pragma unroll 1
-                    for (int u = 0; u < 4; u++)
-                        if (LPN == 1 || (u & 1) == hf) lp.add_slow((int)(cv[u] >> 16), (double)pu[u]);
+                if (kLogProd) lp.renorm();
+                if (kLogProd && big) {
+                    // (rare) the p of such a count is formed again from the tile row and the owner
+                    // row, so that the steps keep nothing for it (both lanes of a pair hold the
+                    // same entries and take this branch together)
+                    const uint4 w = ldcs_quad(eb + c0 + slot);
+#pragma unroll
+                    for (int u = 0; u < 4; u++) {
+                        const uint32_t v = u == 0 ? w.x : u == 1 ? w.y : u == 2 ? w.z : w.w;
+                        if (v >> (16 + kLpBits)) {
+                            PT t[KL];
+                            gather(v, t);
+                            PT p = dot_rows<KL>(own, t);
+                            if (LPN == 2) p += __shfl_xor_sync(pmask, p, 1);
+                            if (LPN == 1 || (u & 1) == hf) lp.add_slow(v, (double)p);
+                        }
+                    }
                 }
                 if (COLS && !kLogProd && LPN == 2) {
 #pragma unroll
@@ -1081,9 +1097,16 @@ sweep_p16_kernel(const SweepTiledArgs a) {
             }
             if (kLogProd) lp.end_segment();
             else if (COLS) xl += (double)xls;
-            if (kOwnMode == 2 && en < eend) load_owner(nog, nb < ne, ownn);
+            if (kOwnMode == 2) {
+                f0 = make_uint4(0u, 0u, 0u, 0u);
+                if (en < eend) {
+                    load_ptrs();
+                    load_owner(nog, nbu < ne, ownn);
+                    if (nbu + slot < ne) f0 = ldcs_quad(ent4 + nbu + slot);
+                }
+            }
             // sum over the lanes that hold the same rank entries (fp64), recursive halving
-            double *out = a.Part + (slab * a.NO + (int64_t)og) * RS;
+            double *out = a.Part + (int64_t)(slab * NO + og) * RS;
             double v0[KL];
 #pragma unroll
             for (int k = 0; k < KL; k++) v0[k] = (double)acc[k];
@@ -1200,8 +1223,8 @@ sweep_p16_kernel(const SweepTiledArgs a) {
             }
             }
             e = en;
-            beg = nb; end = ne; dead = ndead; og = nog;
-            nb = nnb; ne = nne; ndead = nndead; nog = nnog;
+            beg = nb; end = ne; og = nog;
+            nb = nnb; ne = nne; nog = nnog;
         }
         ebase = eend;
     }

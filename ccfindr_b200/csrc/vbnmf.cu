@@ -527,7 +527,8 @@ int build_pass(H *h, Layout *L, bool cols_pass, const int32_t *d_colof, uint32_t
     const int64_t NO = cols_pass ? L->NC : L->NG;
     const int nslabs = cols_pass ? L->Sg : L->Sc;
     P.E = (int64_t)nslabs * NO;
-    if (P.E >= (int64_t)UINT32_MAX)
+    // (the sweep kernels also step 32-bit segment positions by up to two group strides past E)
+    if (P.E >= (int64_t)UINT32_MAX - 1024)
         return fail(h, VBNMF_ERR_ARG, "matrix too large for 32-bit segment keys on one GPU");
     const int g = h->num_sms * 8;
     uint32_t *k_in = scratch, *k_out = scratch + nnz, *p_in = scratch + 2 * nnz,

@@ -6,7 +6,8 @@
 Reads the objects the in-tree build leaves in ccfindr_b200/csrc/_obj (cuobjdump -sass,
 cuobjdump --dump-resource-usage).  The mnemonics that show the Blackwell path: UBLKCP (bulk
 asynchronous copy global -> shared, the TMA engine), UBLKPF (bulk L2 prefetch), SYNCS (mbarrier),
-LDS.128 (the gathers), DFMA (fp64 FMA), LDG.E.128 (the packed entries)."""
+LDS.128 (the gathers), DFMA (fp64 FMA), LDG.E.128 (the packed entries).  For each kernel also the
+size of its chunk loop and the local-memory instructions (LDL/STL) inside it."""
 import collections
 import os
 import re
@@ -21,6 +22,20 @@ WATCH = ["UBLKCP", "UBLKPF", "SYNCS", "LDS.128", "LDS.64", "LDG.E.128", "DFMA", 
 
 def demangle(name):
     return subprocess.run(["c++filt", name], capture_output=True, text=True).stdout.strip()
+
+
+def chunk_loop(code):
+    """(instructions, LDS.128, LDL/STL) of the chunk loop: the innermost backward branch whose
+    body holds the gathers of at least one whole chunk (4 steps)"""
+    best = None
+    for a, ins in code:
+        m = re.search(r"BRA\S*\s+(?:\S+,\s*)?(0x[0-9a-f]+)\s*$", ins)
+        if m and int(m.group(1), 16) < a:
+            body = [i for x, i in code if int(m.group(1), 16) <= x <= a]
+            lds = sum("LDS.128" in i for i in body)
+            if lds >= 16 and (best is None or len(body) < best[0]):
+                best = (len(body), lds, sum(bool(re.search(r"\b(LDL|STL)", i)) for i in body))
+    return best
 
 
 def main():
@@ -52,6 +67,9 @@ def main():
                 print("  %-62s regs %3d  static smem %4d B  local (spill) %4d B  SASS %5d" % (
                     d, u[0], u[1], u[2], tot))
                 print("     " + "  ".join("%s %d" % (k, counts[k]) for k in WATCH if counts[k]))
+                loop = chunk_loop(code)
+                if loop:
+                    print("     chunk loop: %d instructions, %d LDS.128, %d LDL/STL" % loop)
 
         for ln in sass.splitlines():
             m = re.search(r"Function : (\S+)", ln)
@@ -59,7 +77,11 @@ def main():
                 flush()
                 fn = m.group(1)
                 counts = collections.Counter()
+                code = []
                 continue
+            m = re.search(r"/\*([0-9a-f]{4,5})\*/\s+(.*?);", ln)
+            if m:
+                code.append((int(m.group(1), 16), m.group(2)))
             m = re.search(r"/\*[0-9a-f]{4}\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_.]+)", ln)
             if m:
                 op = m.group(1)
